@@ -15,7 +15,11 @@ torch.distributed is used only for the NCCL-id hand-off, the barrier and the max
 D2H + host SHA-256 are timed).  `e2e`: the full mpvss_verify_distribution call from pinned host
 buffers, host->device copies and position planning inside the timed region.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n N] [--t T]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n N] [--t T] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the last timed step returned (verdict, transcript digest and, on one GPU, the
+X_i / a1 / a2 rows) as DIR/<name>.npy; the box is synthesised from --seed, so two builds run with the same
+arguments can be compared output for output.
 
 `--impl reference` times the reference's CPU schedule (oracle/cpu_baseline.c, an OpenSSL
 proxy for num-bigint since the Rust reference cannot be built here) on all host cores; it never
@@ -59,6 +63,7 @@ RFC3526_2048 = int(
     "e39e772c180e86039b2783a2ec07a28fb5c55df06f4c52c9de2bcbf6955817183995497cea956ae515d2261898fa0510"
     "15728e5a8aacaa68ffffffffffffffff", 16)
 SECP_N = 0xFFFFFFFFFFFFFFFFFFFFFFFFFFFFFFFEBAAEDCE6AF48A03BBFD25E8CD0364141
+DUMP_BYTES = 64_000_000                  # --dump-outputs: all .npy files together stay below this
 
 
 def env_int(k, d):
@@ -366,6 +371,7 @@ class Runner:
         self.flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
         self.modp = box["group"] == "modp"
         self.check = True
+        self.outputs = None     # see keep_outputs()
 
     def P(self, key):
         return ctypes.cast(self.host[key].data_ptr(), ctypes.POINTER(ctypes.c_uint8))
@@ -376,9 +382,25 @@ class Runner:
             self.h, b["n"], b["t"], self.P("commitments"), None, self.P("publickeys"), self.P("shares"),
             self.P("responses"), self.P("challenge")))
 
-    def run(self, x_out=None, digest=None):
-        self.g.ctx.check(self.lib.mpvss_verify_distribution_run(self.h, ctypes.byref(self.ok), x_out, None, None, digest))
+    def run(self, x_out=None, digest=None, a1_out=None, a2_out=None):
+        self.g.ctx.check(self.lib.mpvss_verify_distribution_run(self.h, ctypes.byref(self.ok), x_out, a1_out, a2_out,
+                                                                digest))
         return self.ok.value, self.g.ctx.last_kernel_ms, self.g.ctx.last_phase_ms(2 if self.modp else 0)
+
+    def keep_outputs(self):
+        """make the last timed resident step receive every output of the call: the digest, and X_i / a1 / a2 on
+        one GPU (the library returns no rows through a communicator)"""
+        from mpvss_rs_b200.lib import buf
+        rows = self.box["n"] * self.box["eb"]
+        self.outputs = {k: (buf(size=rows) if self.world == 1 else None) for k in ("x", "a1", "a2")}
+        self.outputs["digest"] = buf(size=32)
+
+    def run_keep(self):
+        from mpvss_rs_b200.lib import ptr
+        o = self.outputs
+        r = self.run(ptr(o["x"]), ptr(o["digest"]), ptr(o["a1"]), ptr(o["a2"]))
+        o["verdict"] = r[0]
+        return r
 
     def full(self):
         b = self.box
@@ -400,13 +422,14 @@ class Runner:
         self.dist.all_reduce(tns, op=self.dist.ReduceOp.MAX)
         return float(tns.item())
 
-    def timed(self, fn, steps, warmup):
+    def timed(self, fn, steps, warmup, last=None):
+        """warmup + steps calls of fn (the final one `last` when given); returns the timed steps"""
         out = []
         for i in range(warmup + steps):
             self.flush.zero_()
             self.barrier()
             t0 = time.perf_counter()
-            r = fn()
+            r = last() if last is not None and i == warmup + steps - 1 else fn()
             self.barrier()
             dt = self.maxr(time.perf_counter() - t0)
             if i >= warmup:
@@ -416,7 +439,7 @@ class Runner:
     def measure(self, steps, warmup):
         """resident steps, then full calls; returns a dict of means (max over ranks per step)"""
         self.stage()
-        res = self.timed(self.run, steps, warmup)
+        res = self.timed(self.run, steps, warmup, self.run_keep if self.outputs is not None else None)
         assert not self.check or all(r[1][0] == 1 for r in res), "synthetic box did not verify"
         launches = self.g.ctx.last_kernel_launches * steps * self.world
         sq, ml = self.g.ctx.last_horner_products()
@@ -426,6 +449,28 @@ class Runner:
                 "kernel_ms": statistics.mean(self.maxr(r[1][1]) for r in res),
                 "horner_ms": statistics.mean(self.maxr(r[1][2]) for r in res),
                 "e2e_ms": statistics.mean(r[0] for r in e2e) * 1e3, "launches": launches, "sqr": sq, "mul": ml}
+
+
+def dump_outputs(path, runner, seed):
+    """--dump-outputs: what the last timed resident step returned, one .npy per output.  verdict.npy (float64,
+    1 = the box verifies); digest.npy (float32, the 32 bytes of the transcript's SHA-256); on one GPU x.npy,
+    a1.npy and a2.npy (float32, [rows, element bytes], each row a participant's element in the ABI's boundary
+    encoding, one byte per entry) and participant_index.npy (float64, the 0-based participant of each row).  When
+    all rows would exceed DUMP_BYTES, the rows are a sample of participants drawn with the box's seed."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    o, eb = runner.outputs, runner.box["eb"]
+    save = lambda name, a: np.save(os.path.join(path, name + ".npy"), a)
+    save("verdict", np.array([o["verdict"]], dtype=np.float64))
+    save("digest", np.frombuffer(bytes(o["digest"]), dtype=np.uint8).astype(np.float32))
+    if o["x"] is None:
+        return
+    n = len(o["x"]) // eb
+    fit = (DUMP_BYTES - (1 << 20)) // (3 * 4 * eb + 8)
+    idx = np.arange(n) if n <= fit else np.sort(np.random.default_rng(seed).choice(n, fit, replace=False))
+    save("participant_index", idx.astype(np.float64))
+    for k in ("x", "a1", "a2"):
+        save(k, np.frombuffer(bytes(o[k]), dtype=np.uint8).reshape(n, eb)[idx].astype(np.float32))
 
 
 # dram__bytes_read.sum + dram__bytes_write.sum of the dominant launch at n = 4096, t = 2731 on one GPU, from the
@@ -493,7 +538,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--c5", action="store_true", help="also time BASELINE config 5 (n=65536 t=43691) [default at 8 GPUs]")
     ap.add_argument("--no-c5", action="store_true", help="skip config 5 at 8 GPUs (short re-runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     n = args.n
     t = args.t or -(-2 * n // 3)
@@ -508,6 +557,8 @@ def main():
                           "the framed transcript rows per step, every rank hashes"}
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs dumps the GPU path (--impl ours)")
         if rank == 0:
             print(json.dumps(reference_arm(args, n_total, t, config, cores)))
         return 0
@@ -549,7 +600,11 @@ def main():
         box = dict(box, n=args.subset)
         runner = Runner(group, box, torch, dist, rank, world)
         runner.check = False
+        if args.dump_outputs:
+            runner.keep_outputs()
         m_ = runner.measure(args.steps, args.warmup)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, runner, args.seed)
         if rank == 0:
             print(json.dumps({"experiment": f"first {args.subset} participants of a box of {n_total}, t={t}", "ms": m_["ms"],
                               "kernel_ms": m_["kernel_ms"], "horner_ms": m_["horner_ms"], "chunks": args.chunks}))
@@ -587,8 +642,12 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
+    if args.dump_outputs:
+        runner.keep_outputs()
     meas = runner.measure(args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, runner, args.seed)
 
     also = {}
     if world > 1 and not args.no_also:

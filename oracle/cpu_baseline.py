@@ -3,21 +3,35 @@ TEST + BENCH INFRASTRUCTURE ONLY."""
 import ctypes
 import os
 import subprocess
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "cpu_baseline.c")
 SO = os.path.join(HERE, "_build", "libcpu_baseline.so")
 
 
-def build(force=False):
-    os.makedirs(os.path.dirname(SO), exist_ok=True)
-    if force or not os.path.exists(SO) or os.path.getmtime(SRC) > os.path.getmtime(SO):
-        subprocess.check_call(["gcc", "-O2", "-Wno-deprecated-declarations", "-shared", "-fPIC", "-pthread", "-o", SO, SRC, "-lcrypto"])
-    return SO
+def _stale(so):
+    return not os.path.exists(so) or os.path.getmtime(SRC) > os.path.getmtime(so)
+
+
+def build(force=False, so=SO):
+    os.makedirs(os.path.dirname(so), exist_ok=True)
+    if force or _stale(so):
+        subprocess.check_call(["gcc", "-O2", "-Wno-deprecated-declarations", "-shared", "-fPIC", "-pthread", "-o", so, SRC, "-lcrypto"])
+    return so
+
+
+def _runtime_so():
+    """The library built into the tree; when it is missing or stale and the tree cannot be written (a read-only
+    checkout), a private copy in the temporary directory instead."""
+    out_dir = os.path.dirname(SO)
+    if not _stale(SO) or os.access(out_dir if os.path.isdir(out_dir) else HERE, os.W_OK):
+        return build()
+    return build(so=os.path.join(tempfile.gettempdir(), f"mpvss_cpu_baseline_{os.getuid()}", "libcpu_baseline.so"))
 
 
 def load():
-    lib = ctypes.CDLL(build())
+    lib = ctypes.CDLL(_runtime_so())
     p, sz = ctypes.c_char_p, ctypes.c_size_t
     lib.cpu_modp_verify.argtypes = [p, p, sz, ctypes.POINTER(ctypes.c_int64), p, p, p, p, sz, ctypes.c_int,
                                     ctypes.c_int, p, p, p]
