@@ -71,8 +71,8 @@ void mpvss_ctx_destroy(mpvss_ctx* ctx);
 const char* mpvss_last_error(const mpvss_ctx* ctx);
 /* tunables: "modp_tpi" (lanes per 2048-bit value: 4, 8, 16); "modp_comb" (0/1: fixed-base tables for
  * the two generators); "modp_overlap" (where the X-independent a2 = y^r Y^c runs during
- * verify_distribution: 0 before the X_i launch, 2 beside it on a side stream, 3 (default) beside it as
- * one persistent one-warp CTA per SM, which takes the warp slot the X_i launch leaves idle; the default falls
+ * verify_distribution and verify_distributions: 0 before the X_i launch, 2 beside it on a side stream,
+ * 3 (default) beside it as one persistent one-warp CTA per SM, which takes the warp slot the X_i launch leaves idle; the default falls
  * back to 0 when that slot does not exist, or to 2 for small boxes whose two launches fit the chip together);
  * "modp_chunks" (contiguous chunks per position of the X_i launch, 0 = automatic: more than one only when the
  * launch would leave most of the chip idle); "modp_wpc" (warps per CTA of that launch); "modp_msm" /
@@ -147,6 +147,21 @@ int mpvss_verify_distribution_stage(mpvss_ctx* ctx, size_t n, size_t t, const ui
                                     const uint8_t* responses, const uint8_t* challenge);
 int mpvss_verify_distribution_run(mpvss_ctx* ctx, int* ok, uint8_t* x_out, uint8_t* a1_out, uint8_t* a2_out,
                                   uint8_t* digest_out);
+/* n_boxes independent Participant::verify_distribution_shares calls in one (e.g. the n boxes of one PVSS
+ * round).  Box b has n[b] participants and t[b] commitments.  Every array is the concatenation, in box order,
+ * of what mpvss_verify_distribution takes for one box: commitments (sum t[b] elements), positions (sum n[b];
+ * NULL = 1..n[b] in every box), publickeys and shares (sum n[b] elements), responses (sum n[b] scalars),
+ * challenges (n_boxes scalars).  ok_out[b] = 1 iff box b verifies.  digests_out (optional, 32 bytes per box)
+ * receives the transcript digest that mpvss_verify_distribution returns for that box alone.  Box contents that
+ * do not decode, fail the "validate" check, or carry a position outside [1, 2^31) make that box verify as
+ * false (its digest is then zero) and leave the other boxes alone; the call still returns MPVSS_OK.  The
+ * boxes' transcripts are always hashed on the host ("device_hash" does not apply).  The staged state of
+ * mpvss_verify_distribution_stage is left untouched.  Not collective: on a context with a communicator it
+ * returns MPVSS_ERR_UNSUPPORTED. */
+int mpvss_verify_distributions(mpvss_ctx* ctx, size_t n_boxes, const size_t* n, const size_t* t,
+                               const uint8_t* commitments, const int64_t* positions, const uint8_t* publickeys,
+                               const uint8_t* shares, const uint8_t* responses, const uint8_t* challenges,
+                               int* ok_out, uint8_t* digests_out);
 
 /* Participant::distribute_secret (participant.rs:160-286 / 1094-1274 / 1573-1717) with the
  * randomness injected: `coeffs` (t scalars) replaces Polynomial::init (polynomial.rs:34-47),

@@ -252,6 +252,28 @@ int mpvss_verify_distribution(mpvss_ctx* ctx, size_t n, size_t t, const uint8_t*
   if (s != MPVSS_OK) return box_verdict(s, ok);
   return box_verdict(mpvss_verify_distribution_run(ctx, ok, x_out, a1_out, a2_out, digest_out), ok);
 }
+int mpvss_verify_distributions(mpvss_ctx* ctx, size_t n_boxes, const size_t* n, const size_t* t,
+                               const uint8_t* commitments, const int64_t* positions, const uint8_t* publickeys,
+                               const uint8_t* shares, const uint8_t* responses, const uint8_t* challenges,
+                               int* ok_out, uint8_t* digests_out) {
+  if (!ctx) return MPVSS_ERR_ARG;
+  Guard hold(ctx);
+  if (n_boxes == 0 || !n || !t || !commitments || !publickeys || !shares || !responses || !challenges || !ok_out)
+    return mpvss_fail(ctx, MPVSS_ERR_ARG, "verify_distributions: bad arguments");
+  // the kernels count positions and commitments in 32 bits
+  const size_t limit = 0x7fffffff;
+  size_t sum_n = 0, sum_t = 0;
+  for (size_t b = 0; b < n_boxes; ++b) {
+    if (n[b] == 0 || t[b] == 0 || n[b] > limit - sum_n || t[b] > limit - sum_t)
+      return mpvss_fail(ctx, MPVSS_ERR_ARG, "verify_distributions: box " + std::to_string(b) +
+                                                " has no participants or commitments, or the boxes are too many");
+    sum_n += n[b];
+    sum_t += t[b];
+  }
+  if (ctx->nranks > 1) return mpvss_fail(ctx, MPVSS_ERR_UNSUPPORTED, "verify_distributions: not collective");
+  DISPATCH(ctx, verify_batch, n_boxes, n, t, commitments, positions, publickeys, shares, responses, challenges, ok_out,
+           digests_out);
+}
 int mpvss_scalar_poly_eval(mpvss_ctx* ctx, const uint8_t* coeffs, size_t t, const int64_t* positions, size_t n,
                            uint8_t* out) {
   DISPATCH(ctx, scalar_poly_eval, coeffs, t, positions, n, out);

@@ -163,6 +163,8 @@ int multi_exp(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
 int verify_stage(mpvss_ctx*, size_t, size_t, const uint8_t*, const int64_t*, const uint8_t*, const uint8_t*,
                  const uint8_t*, const uint8_t*);
 int verify_run(mpvss_ctx*, int*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
+int verify_batch(mpvss_ctx*, size_t, const size_t*, const size_t*, const uint8_t*, const int64_t*, const uint8_t*,
+                 const uint8_t*, const uint8_t*, const uint8_t*, int*, uint8_t*);
 int scalar_poly_eval(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
 int distribute(mpvss_ctx*, size_t, size_t, const uint8_t*, size_t, const uint8_t*, const uint8_t*, const uint8_t*,
                uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
@@ -185,6 +187,8 @@ int multi_exp(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
 int verify_stage(mpvss_ctx*, size_t, size_t, const uint8_t*, const int64_t*, const uint8_t*, const uint8_t*,
                  const uint8_t*, const uint8_t*);
 int verify_run(mpvss_ctx*, int*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
+int verify_batch(mpvss_ctx*, size_t, const size_t*, const size_t*, const uint8_t*, const int64_t*, const uint8_t*,
+                 const uint8_t*, const uint8_t*, const uint8_t*, int*, uint8_t*);
 int scalar_poly_eval(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
 int distribute(mpvss_ctx*, size_t, size_t, const uint8_t*, size_t, const uint8_t*, const uint8_t*, const uint8_t*,
                uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
@@ -207,6 +211,8 @@ int multi_exp(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
 int verify_stage(mpvss_ctx*, size_t, size_t, const uint8_t*, const int64_t*, const uint8_t*, const uint8_t*,
                  const uint8_t*, const uint8_t*);
 int verify_run(mpvss_ctx*, int*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
+int verify_batch(mpvss_ctx*, size_t, const size_t*, const size_t*, const uint8_t*, const int64_t*, const uint8_t*,
+                 const uint8_t*, const uint8_t*, const uint8_t*, int*, uint8_t*);
 int scalar_poly_eval(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
 int distribute(mpvss_ctx*, size_t, size_t, const uint8_t*, size_t, const uint8_t*, const uint8_t*, const uint8_t*,
                uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);

@@ -29,6 +29,9 @@ template <class Cv> __global__ void __launch_bounds__(TPB) fixed_kernel(FixedArg
 template <class Cv> __global__ void __launch_bounds__(TPB) comb_build_kernel(CombArgs<Cv> A) { comb_build_body<Cv>(A, TID); }
 template <class Cv> __global__ void __launch_bounds__(TPB) decode_kernel(DecodeArgs<Cv> A) { decode_body<Cv>(A, TID); }
 template <class Cv> __global__ void __launch_bounds__(TPB, EC_HORNER_MIN_BLOCKS) horner_kernel(HornerArgs<Cv> A) { horner_body<Cv>(A, TID); }
+template <class Cv> __global__ void __launch_bounds__(TPB, EC_HORNER_MIN_BLOCKS) horner_boxes_kernel(HornerBoxesArgs<Cv> A) {
+  horner_boxes_body<Cv>(A, TID);
+}
 template <class Cv> __global__ void __launch_bounds__(TPB) sum_kernel(SumArgs<Cv> A) { sum_body<Cv>(A, TID); }
 template <class Cv> __global__ void __launch_bounds__(TPB) add_kernel(AddArgs<Cv> A) { add_body<Cv>(A, TID); }
 __global__ void __launch_bounds__(TPB) frame_kernel(FrameArgs A) { frame_body(A, TID); }
@@ -67,6 +70,11 @@ template <class Cv> cudaError_t launch_decode(const DecodeArgs<Cv>& A, cudaStrea
 template <class Cv> cudaError_t launch_horner(const HornerArgs<Cv>& A, cudaStream_t s) {
   if (A.n == 0 || A.K == 0 || A.t == 0) return cudaErrorInvalidValue;
   horner_kernel<Cv><<<blocks(A.n * A.K), TPB, 0, s>>>(A);
+  return cudaGetLastError();
+}
+template <class Cv> cudaError_t launch_horner_boxes(const HornerBoxesArgs<Cv>& A, cudaStream_t s) {
+  if (A.n == 0 || A.K == 0) return cudaErrorInvalidValue;
+  horner_boxes_kernel<Cv><<<blocks(A.n * A.K), TPB, 0, s>>>(A);
   return cudaGetLastError();
 }
 template <class Cv> cudaError_t launch_sum(const SumArgs<Cv>& A, cudaStream_t s) {
@@ -112,6 +120,7 @@ cudaError_t launch_proof(const ProofArgs& A, cudaStream_t s) {
   template cudaError_t launch_comb_build<Cv>(const CombArgs<Cv>&, cudaStream_t);         \
   template cudaError_t launch_decode<Cv>(const DecodeArgs<Cv>&, cudaStream_t);           \
   template cudaError_t launch_horner<Cv>(const HornerArgs<Cv>&, cudaStream_t);           \
+  template cudaError_t launch_horner_boxes<Cv>(const HornerBoxesArgs<Cv>&, cudaStream_t); \
   template cudaError_t launch_sum<Cv>(const SumArgs<Cv>&, cudaStream_t);                 \
   template cudaError_t launch_add<Cv>(const AddArgs<Cv>&, cudaStream_t);
 INSTANTIATE(secp::SecpCurve)

@@ -156,8 +156,9 @@ struct Ec {
     return reinterpret_cast<const fp256::Modulus*>(ctx->ec_consts.as<char>() + sizeof(fp256::Modulus));
   }
 
-  // boundary scalars -> device limb layout (8 little-endian u32 per scalar)
-  static int scalars_in(mpvss_ctx* ctx, const uint8_t* s, size_t n, std::vector<uint32_t>& out) {
+  // boundary scalars -> device limb layout (8 little-endian u32 per scalar); report = false: a non-canonical
+  // scalar returns MPVSS_ERR_ENCODING without recording a context error (per-box checks of a batch)
+  static int scalars_in(mpvss_ctx* ctx, const uint8_t* s, size_t n, std::vector<uint32_t>& out, bool report = true) {
     out.resize(n * 8);
     uint32_t ord[8];
     put8(ord, ctx->ec_order);
@@ -178,8 +179,10 @@ struct Ec {
       if (below) continue;
       big::Int v = T::SCALAR_BE ? big::from_be(s + i * SB, SB) : big::from_le(s + i * SB, SB);
       if (big::cmp(v, ctx->ec_order) >= 0) {
-        if (T::SCALAR_BE)  // k256 Scalar::from_repr rejects non-canonical values
+        if (T::SCALAR_BE) {  // k256 Scalar::from_repr rejects non-canonical values
+          if (!report) return MPVSS_ERR_ENCODING;
           return mpvss_fail(ctx, MPVSS_ERR_ENCODING, "scalar " + std::to_string(i) + " is not below the group order");
+        }
         v = big::mod(v, ctx->ec_order);  // dalek Scalar::from_bytes_mod_order
       }
       put8(out.data() + i * 8, v);
@@ -286,28 +289,30 @@ struct Ec {
     return MPVSS_OK;
   }
   // field products of the Horner + chunk-scaling + chunk-sum launches for these positions (roofline accounting)
-  static void count_horner(mpvss_ctx* ctx, const std::vector<uint32_t>& pos, size_t t) {
-    const uint64_t Kc = ctx->ec_chunks ? ctx->ec_chunks : 1;
-    uint64_t M = 0, S = 0;
+  // one position p of a polynomial of t coefficients cut into Kc non-empty chunks
+  static void count_position(uint32_t p, uint64_t t, uint64_t Kc, uint64_t& M, uint64_t& S) {
     auto add = [&](OpCost c, uint64_t times) {
       M += c.m * times;
       S += c.s * times;
     };
-    for (uint32_t p : pos) {
-      uint32_t nd = 1, nz = 0;
-      while (nd < 16 && (p >> (2 * nd))) ++nd;
-      for (uint32_t d = 0; d + 1 < nd; ++d) nz += ((p >> (2 * d)) & 3u) != 0;
-      const uint64_t steps = t - Kc;                       // Horner steps of all chunks of this position
-      add(T::SMALL_FIXED, steps);
-      add(T::DBL_NOT, steps * (nd - 1));
-      add(T::DBL, steps * (nd - 1));
-      add(T::WIN_ADD, steps * (nz + (T::TOP_ADD_FREE ? 0 : 1)));
-      add(T::MADD, steps);
-      // chunks 1..K-1: acc <- pos^(kB) * acc, fixed 4-bit windows (7 dbl + 7 add table, 63 x 4 dbl, ~60 adds)
-      add(T::DBL, (Kc - 1) * (7 + 252));
-      add(T::ADD, (Kc - 1) * (7 + 60));
-      add(T::ADD, Kc - 1);                                  // chunk sum
-    }
+    uint32_t nd = 1, nz = 0;
+    while (nd < 16 && (p >> (2 * nd))) ++nd;
+    for (uint32_t d = 0; d + 1 < nd; ++d) nz += ((p >> (2 * d)) & 3u) != 0;
+    const uint64_t steps = t - Kc;                       // Horner steps of all chunks of this position
+    add(T::SMALL_FIXED, steps);
+    add(T::DBL_NOT, steps * (nd - 1));
+    add(T::DBL, steps * (nd - 1));
+    add(T::WIN_ADD, steps * (nz + (T::TOP_ADD_FREE ? 0 : 1)));
+    add(T::MADD, steps);
+    // chunks 1..K-1: acc <- pos^(kB) * acc, fixed 4-bit windows (7 dbl + 7 add table, 63 x 4 dbl, ~60 adds)
+    add(T::DBL, (Kc - 1) * (7 + 252));
+    add(T::ADD, (Kc - 1) * (7 + 60));
+    add(T::ADD, Kc - 1);                                  // chunk sum
+  }
+  static void count_horner(mpvss_ctx* ctx, const std::vector<uint32_t>& pos, size_t t) {
+    const uint64_t Kc = ctx->ec_chunks ? ctx->ec_chunks : 1;
+    uint64_t M = 0, S = 0;
+    for (uint32_t p : pos) count_position(p, t, Kc, M, S);
     ctx->horner_sqr = S;
     ctx->horner_mul = M;
   }
@@ -636,6 +641,120 @@ struct Ec {
     return sync(ctx);
   }
 
+  // ---- mpvss_verify_distributions: many boxes, one launch per kernel ---------------------------------
+  // Positions and scalars are checked per box on the host; a box that fails verifies as false with a zero
+  // digest and leaves the others alone.  All commitments are decoded in one launch, X_i of every box comes
+  // from one multi-box Horner launch and one chunk sum, a1 / a2 take one challenge per instance, and the
+  // frames of all boxes come to the host in one copy, where each box's row range is hashed on its own.
+  // Uses scratch buffers only: the staged single-box state (v_*) is left as it was.
+  static int verify_batch(mpvss_ctx* ctx, size_t nb, const size_t* nv, const size_t* tv, const uint8_t* commitments,
+                          const int64_t* positions, const uint8_t* publickeys, const uint8_t* shares,
+                          const uint8_t* responses, const uint8_t* challenges, int* ok_out, uint8_t* digests_out) {
+    std::vector<size_t> noff(nb + 1, 0), toff(nb + 1, 0);
+    size_t tmax = 1;
+    for (size_t b = 0; b < nb; ++b) {
+      noff[b + 1] = noff[b] + nv[b];
+      toff[b + 1] = toff[b] + tv[b];
+      tmax = std::max(tmax, tv[b]);
+    }
+    const size_t N = noff[nb], Tt = toff[nb];
+    std::vector<uint8_t> live(nb, 1);
+    // a rejected box is only false: these checks record no context error, the call succeeds
+    std::vector<uint32_t> pos(N, 1), coff(N), ct(N), rl(N * 8, 0), cl(N * 8, 0), br, bc;
+    for (size_t b = 0; b < nb; ++b) {
+      for (size_t i = noff[b]; positions && i < noff[b + 1] && live[b]; ++i)
+        live[b] = positions[i] >= 1 && positions[i] <= 0x7fffffff;
+      if (!live[b] || scalars_in(ctx, responses + noff[b] * SB, nv[b], br, false) != MPVSS_OK ||
+          scalars_in(ctx, challenges + b * SB, 1, bc, false) != MPVSS_OK)
+        live[b] = 0;
+      for (size_t j = 0, i = noff[b]; j < nv[b]; ++j, ++i) {
+        coff[i] = (uint32_t)toff[b];
+        ct[i] = (uint32_t)tv[b];
+        if (!live[b]) continue;
+        pos[i] = positions ? (uint32_t)positions[i] : (uint32_t)(j + 1);
+        memcpy(&rl[i * 8], &br[j * 8], 32);
+        memcpy(&cl[i * 8], bc.data(), 32);
+      }
+    }
+    DevBuf &dc = ctx->buf(0), &dxy = ctx->buf(1), &dcst = ctx->buf(2), &dpos = ctx->buf(3), &dcoff = ctx->buf(4),
+           &dct = ctx->buf(5), &dpk = ctx->buf(6), &dy = ctx->buf(7), &dr = ctx->buf(8), &dch = ctx->buf(9),
+           &dpart = ctx->buf(10), &dx = ctx->buf(11), &da1 = ctx->buf(12), &da2 = ctx->buf(13), &dst = ctx->buf(14),
+           &dfr = ctx->buf(15);
+    MPVSS_TRY(h2d(ctx, dc, commitments, Tt * EB));
+    MPVSS_TRY(h2d(ctx, dpos, pos.data(), N * 4));
+    MPVSS_TRY(h2d(ctx, dcoff, coff.data(), N * 4));
+    MPVSS_TRY(h2d(ctx, dct, ct.data(), N * 4));
+    MPVSS_TRY(h2d(ctx, dpk, publickeys, N * EB));
+    MPVSS_TRY(h2d(ctx, dy, shares, N * EB));
+    MPVSS_TRY(h2d(ctx, dr, rl.data(), N * 32));
+    MPVSS_TRY(h2d(ctx, dch, cl.data(), N * 32));
+    const transcript::Geom g = geom();
+    const size_t row = g.row();
+    for (DevBuf* b : {&dx, &da1, &da2}) MPVSS_CUDA(ctx, b->ensure(N * EB));
+    MPVSS_CUDA(ctx, dxy.ensure(Tt * 64));
+    MPVSS_CUDA(ctx, dcst.ensure(Tt * 4));
+    MPVSS_CUDA(ctx, dst.ensure(2 * N * 4));
+    MPVSS_CUDA(ctx, dfr.ensure(N * row));
+    // chunks per position: the one-wave rule of dev_horner on the total position count
+    const size_t target = ctx->ec_threads ? ctx->ec_threads : (size_t)ctx->sm_count * ec::HORNER_CTAS_PER_SM * 128;
+    const size_t Kc = std::max<size_t>(1, std::min<size_t>(target / N, std::max<size_t>(1, tmax / 16)));
+    MPVSS_CUDA(ctx, dpart.ensure(Kc * N * sizeof(Point)));
+    uint32_t* st = dst.as<uint32_t>();
+    timing_begin(ctx);
+    ec::DecodeArgs<Cv> D{K(ctx), dc.as<uint8_t>(), dxy.as<uint32_t>(), dcst.as<uint32_t>(), (uint32_t)Tt};
+    MPVSS_CUDA(ctx, ec::launch_decode<Cv>(D, ctx->stream));
+    timing_launch(ctx);
+    ec::HornerBoxesArgs<Cv> H{K(ctx), dxy.as<uint32_t>(), dcst.as<uint32_t>(), dpos.as<uint32_t>(), dcoff.as<uint32_t>(),
+                              dct.as<uint32_t>(), dpart.as<Point>(), (uint32_t)N, (uint32_t)Kc};
+    MPVSS_CUDA(ctx, ec::launch_horner_boxes<Cv>(H, ctx->stream));
+    timing_launch(ctx);
+    ec::SumArgs<Cv> S{K(ctx), dpart.as<Point>(), nullptr, dx.as<uint8_t>(), (uint32_t)N, (uint32_t)Kc, 1, (uint32_t)N,
+                      (uint32_t)(Kc * N)};
+    MPVSS_CUDA(ctx, ec::launch_sum<Cv>(S, ctx->stream));
+    timing_launch(ctx);
+    // a2 = r*y + c*Y, a1 = r*g + c*X  (dleq.rs:66-84), one challenge per instance
+    MPVSS_TRY(dev_exp2(ctx, dpk.as<uint8_t>(), EB, dr.as<uint32_t>(), dy.as<uint8_t>(), EB, dch.as<uint32_t>(), 8, N,
+                       da2.as<uint8_t>(), nullptr, st + N));
+    MPVSS_TRY(dev_exp2(ctx, ctx->gens.as<uint8_t>(), 0, dr.as<uint32_t>(), dx.as<uint8_t>(), EB, dch.as<uint32_t>(), 8, N,
+                       da1.as<uint8_t>(), nullptr, st, nullptr, true));
+    ec::FrameArgs FA{dx.as<uint8_t>(), dy.as<uint8_t>(), da1.as<uint8_t>(), da2.as<uint8_t>(), dfr.as<uint8_t>(),
+                     (uint32_t)N, (uint32_t)EB};
+    MPVSS_CUDA(ctx, ec::launch_frames(FA, ctx->stream));
+    timing_launch(ctx);
+    MPVSS_TRY(timing_end(ctx));
+    uint64_t M = 0, Sq = 0;
+    for (size_t b = 0; b < nb; ++b) {
+      const uint64_t B = (tv[b] + Kc - 1) / Kc, Kb = (tv[b] + B - 1) / B;
+      for (size_t i = noff[b]; i < noff[b + 1]; ++i) count_position(pos[i], tv[b], Kb, M, Sq);
+    }
+    ctx->horner_sqr = Sq;
+    ctx->horner_mul = M;
+    // rows, then the decode status of the commitments and of the two DLEQ launches, in one pinned buffer
+    PinBuf& host = ctx->pin(0);
+    MPVSS_CUDA(ctx, host.ensure(N * row + (Tt + 2 * N) * 4));
+    uint8_t* rows = host.as<uint8_t>();
+    uint32_t* hcst = reinterpret_cast<uint32_t*>(rows + N * row);
+    uint32_t* hst = hcst + Tt;
+    MPVSS_TRY(d2h(ctx, rows, dfr, N * row));
+    MPVSS_TRY(d2h(ctx, hcst, dcst, Tt * 4));
+    MPVSS_TRY(d2h(ctx, hst, dst, 2 * N * 4));
+    MPVSS_TRY(sync(ctx));
+    for (size_t b = 0; b < nb; ++b) {
+      for (size_t j = toff[b]; j < toff[b + 1] && live[b]; ++j) live[b] = hcst[j] != 1;
+      for (size_t i = noff[b]; i < noff[b + 1] && live[b]; ++i) live[b] = hst[i] != 1 && hst[N + i] != 1;
+      uint8_t digest[32] = {0};
+      ok_out[b] = 0;
+      if (live[b]) {
+        sha2::Sha256 h;
+        transcript::hash_ordered(h, rows, noff[b], noff[b + 1], g);
+        const big::Int c = challenge_of(ctx, h, digest);
+        ok_out[b] = big::cmp(c, scalar_big(challenges + b * SB)) == 0;
+      }
+      if (digests_out) memcpy(digests_out + 32 * b, digest, 32);
+    }
+    return MPVSS_OK;
+  }
+
   static int scalar_poly_eval(mpvss_ctx* ctx, const uint8_t* coeffs, size_t t, const int64_t* positions, size_t n,
                               uint8_t* out) {
     MPVSS_TRY(bad(ctx, coeffs && out && n > 0 && t > 0, "scalar_poly_eval: bad arguments"));
@@ -940,6 +1059,10 @@ struct Ec {
   }                                                                                                                  \
   int verify_run(mpvss_ctx* c, int* ok, uint8_t* x, uint8_t* a1, uint8_t* a2, uint8_t* d) {                          \
     return Ec<Traits>::verify_run(c, ok, x, a1, a2, d);                                                              \
+  }                                                                                                                  \
+  int verify_batch(mpvss_ctx* c, size_t nb, const size_t* n, const size_t* t, const uint8_t* cm, const int64_t* p,   \
+                   const uint8_t* pk, const uint8_t* y, const uint8_t* r, const uint8_t* ch, int* ok, uint8_t* d) {  \
+    return Ec<Traits>::verify_batch(c, nb, n, t, cm, p, pk, y, r, ch, ok, d);                                        \
   }                                                                                                                  \
   int scalar_poly_eval(mpvss_ctx* c, const uint8_t* co, size_t t, const int64_t* p, size_t n, uint8_t* o) {        \
     return Ec<Traits>::scalar_poly_eval(c, co, t, p, n, o);                                                          \

@@ -263,6 +263,66 @@ MP_DEV void horner_body(const HornerArgs<Cv>& A, uint32_t tid) {
   A.out[tid] = acc;
 }
 
+// Multi-box Horner (mpvss_verify_distributions): the positions of several boxes are concatenated, and
+// position i belongs to a box whose t_b commitments start at cxy row coff[i].  Instance (k, i) evaluates
+// chunk k = [k B_b, min((k+1) B_b, t_b)), B_b = ceil(t_b / K), of that box's polynomial; a chunk that lies
+// past t_b (boxes with fewer than K coefficients) contributes the identity.  The body repeats horner_body
+// instead of sharing a helper with it so that the single-box kernel's code stays exactly as it is.
+template <class Cv>
+struct HornerBoxesArgs {
+  const typename Cv::Consts* C;
+  const uint32_t* cxy;      // commitments of all boxes, concatenated (decode_body layout)
+  const uint32_t* cstatus;  // decode status per commitment (2 = identity)
+  const uint32_t* pos;      // n positions, concatenated over the boxes
+  const uint32_t* coff;     // per position: first commitment of its box
+  const uint32_t* ct;       // per position: commitments t_b of its box
+  typename Cv::Point* out;  // K * n partial results, index k * n + i
+  uint32_t n, K;
+};
+
+template <class Cv>
+MP_DEV void horner_boxes_body(const HornerBoxesArgs<Cv>& A, uint32_t tid) {
+  if (tid >= A.n * A.K) return;
+  using Point = typename Cv::Point;
+  const typename Cv::Consts& C = *A.C;
+  const uint32_t k = tid / A.n, i = tid % A.n;
+  const uint32_t t = A.ct[i], B = (t + A.K - 1) / A.K, lo = k * B;
+  if (lo >= t) {
+    A.out[tid] = Cv::infinity(C);
+    return;
+  }
+  const uint32_t hi = (lo + B < t) ? lo + B : t;
+  const uint32_t* cxy = A.cxy + (size_t)A.coff[i] * 16;
+  const uint32_t* cst = A.cstatus + A.coff[i];
+  const uint32_t pos = A.pos[i], nd = digits4(pos);
+  Point acc = Cv::from_aff(load_aff<Cv>(cxy + (size_t)(hi - 1) * 16, cst[hi - 1]), C);
+#pragma unroll 1
+  for (int j = (int)hi - 2; j >= (int)lo; --j) {
+    acc = Cv::small_mul(acc, pos, nd, C);
+    acc = Cv::madd(acc, load_aff<Cv>(cxy + (size_t)j * 16, cst[j]), C);
+  }
+  if (k > 0) {
+    // e = pos^(k*B) mod n in the scalar field, then acc <- e * acc
+    using namespace fp256;
+    Fe b = fe_zero();
+    b.v[0] = pos;
+    b = to_mont(b, C.N);
+    Fe e = mont_one(C.N);
+    bool started = false;
+#pragma unroll 1
+    for (int bit = 31; bit >= 0; --bit) {
+      if (started) e = sqr(e, C.N);
+      if ((lo >> bit) & 1u) {
+        e = started ? mul(e, b, C.N) : b;
+        started = true;
+      }
+    }
+    e = from_mont(e, C.N);
+    acc = Cv::scalar_mul_wide(acc, e.v, C);
+  }
+  A.out[tid] = acc;
+}
+
 // --------------------------------------------------------- sums / encoding ----
 template <class Cv>
 struct SumArgs {

@@ -17,6 +17,7 @@ template <class Cv> cudaError_t launch_fixed(const FixedArgs<Cv>& A, cudaStream_
 template <class Cv> cudaError_t launch_comb_build(const CombArgs<Cv>& A, cudaStream_t s);
 template <class Cv> cudaError_t launch_decode(const DecodeArgs<Cv>& A, cudaStream_t s);
 template <class Cv> cudaError_t launch_horner(const HornerArgs<Cv>& A, cudaStream_t s);
+template <class Cv> cudaError_t launch_horner_boxes(const HornerBoxesArgs<Cv>& A, cudaStream_t s);
 template <class Cv> cudaError_t launch_sum(const SumArgs<Cv>& A, cudaStream_t s);
 template <class Cv> cudaError_t launch_add(const AddArgs<Cv>& A, cudaStream_t s);
 cudaError_t launch_frames(const FrameArgs& A, cudaStream_t s);

@@ -287,61 +287,91 @@ struct PosPlan {
 static modp_chain::PowerTree g_tree;  // shared by all contexts; grown under g_tree_mu
 static std::mutex g_tree_mu;
 
+// One box of a plan: its positions (nullptr = 1..n), its t commitments at rows [cm_off, cm_off + t) of the
+// commitment array, and its results at rows row_off + k n + i.
+struct PlanBox {
+  const int64_t* positions;
+  size_t n, t;
+  uint32_t cm_off, row_off;
+};
+
 // Positions are sorted by the length of their op list (longest first) and every length class is padded to
 // a whole number of CTAs, so all lane groups of a CTA run the same number of products per step while
 // one launch covers every class; shorter lists inside a class do not occur, padding instances repeat
-// the last live one.
-static int prep_positions(mpvss_ctx* ctx, const int64_t* positions, size_t n, size_t t, PosPlan& plan) {
+// the last live one.  With several boxes the padding is per (box, length class), so that every CTA holds
+// instances of one box and reads that box's coefficients through its (first, steps) pair.  `chunked`: one
+// box, cut into K chunks by horner_chunks (the single-box plan).  A batch plan (chunked = false) is always
+// unchunked, K = 1, whatever its number of boxes: the batch fills the chip, and chunking inside a batch is
+// not implemented (its chunk exponents and combination would have to follow each box's rows).
+static int prep_boxes(mpvss_ctx* ctx, const PlanBox* boxes, size_t nb, bool chunked, PosPlan& plan) {
   static_assert(modp_chain::SLOTS == modp::HC_SLOTS && modp_chain::OPS_MAX == modp::HC_OPS, "kernel / host op format");
+  auto position = [&](const PlanBox& bx, size_t i) { return bx.positions ? bx.positions[i] : (int64_t)i + 1; };
   uint32_t maxp = 1;
-  for (size_t i = 0; i < n; ++i) {
-    int64_t p = positions ? positions[i] : (int64_t)i + 1;
-    if (p < 1 || p > 0x7fffffff) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
-    maxp = std::max<uint32_t>(maxp, (uint32_t)p);
+  size_t n_all = 0;
+  for (size_t b = 0; b < nb; ++b) {
+    for (size_t i = 0; i < boxes[b].n; ++i) {
+      int64_t p = position(boxes[b], i);
+      if (p < 1 || p > 0x7fffffff) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
+      maxp = std::max<uint32_t>(maxp, (uint32_t)p);
+    }
+    n_all += boxes[b].n;
   }
   std::lock_guard<std::mutex> lk(g_tree_mu);
   g_tree.build(std::min<uint32_t>(maxp, modp_chain::TREE_LIMIT));
-  std::vector<std::vector<uint16_t>> ops(n);
-  std::vector<std::vector<uint32_t>> by(modp_chain::OPS_MAX + 1);
-  std::vector<uint32_t> sq(n), ml(n);
-  for (size_t i = 0; i < n; ++i) {
-    if (!modp_chain::step_ops((uint32_t)(positions ? positions[i] : (int64_t)i + 1), g_tree, ops[i], &sq[i], &ml[i]))
-      return mpvss_fail(ctx, MPVSS_ERR_UNSUPPORTED, "no addition chain within the kernel's slot budget");
-    by[ops[i].size()].push_back((uint32_t)i);
-  }
-  plan.K = horner_chunks(ctx, n, t);
-  plan.B = (uint32_t)((t + plan.K - 1) / plan.K);
-  plan.K = (uint32_t)((t + plan.B - 1) / plan.B);
-  plan.tpi = plan.K > 1 ? ctx->modp_tpi : horner_tpi(ctx, n);
-  plan.wpc = horner_wpc(ctx, n, plan.tpi);
+  std::vector<std::vector<uint16_t>> ops(n_all);
+  std::vector<std::vector<std::vector<uint32_t>>> by(nb, std::vector<std::vector<uint32_t>>(modp_chain::OPS_MAX + 1));
+  std::vector<uint32_t> sq(n_all), ml(n_all);
+  for (size_t b = 0, g = 0; b < nb; ++b)
+    for (size_t i = 0; i < boxes[b].n; ++i, ++g) {  // g: instance index over all boxes
+      if (!modp_chain::step_ops((uint32_t)position(boxes[b], i), g_tree, ops[g], &sq[g], &ml[g]))
+        return mpvss_fail(ctx, MPVSS_ERR_UNSUPPORTED, "no addition chain within the kernel's slot budget");
+      by[b][ops[g].size()].push_back((uint32_t)g);
+    }
+  const size_t t0 = boxes[0].t;
+  if (chunked && nb != 1) return mpvss_fail(ctx, MPVSS_ERR_ARG, "a chunked plan covers one box");
+  plan.K = chunked ? horner_chunks(ctx, n_all, t0) : 1;
+  plan.B = (uint32_t)((t0 + plan.K - 1) / plan.K);
+  plan.K = (uint32_t)((t0 + plan.B - 1) / plan.B);
+  plan.tpi = plan.K > 1 ? ctx->modp_tpi : horner_tpi(ctx, n_all);
+  plan.wpc = horner_wpc(ctx, n_all, plan.tpi);
   const size_t per_cta = (size_t)plan.wpc * (32 / plan.tpi);
   plan.slot.clear(); plan.ops.clear(); plan.nops.clear(); plan.first.clear(); plan.steps.clear();
   plan.nops_max = 1;
   plan.sqr = plan.mul = 0;
+  std::vector<uint32_t> base(nb, 0);  // instance index of each box's first position
+  for (size_t b = 1; b < nb; ++b) base[b] = base[b - 1] + (uint32_t)boxes[b - 1].n;
   for (uint32_t k = 0; k < plan.K; ++k) {  // chunk k: coefficients [k B, min((k+1) B, t)), results in rows k n + i
-    const uint32_t lo = k * plan.B, hi = (uint32_t)std::min<size_t>(t, (size_t)lo + plan.B);
     for (uint32_t len = modp_chain::OPS_MAX; len >= 1; --len) {
-      if (by[len].empty()) continue;
-      plan.nops_max = std::max(plan.nops_max, len);
-      auto emit = [&](uint32_t i, uint32_t slot) {
-        plan.slot.push_back(slot);
-        size_t base = plan.ops.size();
-        plan.ops.resize(base + modp_chain::OPS_MAX, (uint16_t)modp_chain::B_ONE);
-        std::copy(ops[i].begin(), ops[i].end(), plan.ops.begin() + base);
-      };
-      for (uint32_t i : by[len]) {
-        emit(i, k * (uint32_t)n + i);
-        plan.sqr += (uint64_t)sq[i] * (hi - lo - 1);
-        plan.mul += (uint64_t)ml[i] * (hi - lo - 1);
+      for (size_t b = 0; b < nb; ++b) {
+        const std::vector<uint32_t>& cls = by[b][len];
+        if (cls.empty()) continue;
+        const PlanBox& bx = boxes[b];
+        const uint32_t lo = plan.K > 1 ? k * plan.B : 0, hi = (uint32_t)std::min<size_t>(bx.t, (size_t)lo + (plan.K > 1 ? plan.B : bx.t));
+        plan.nops_max = std::max(plan.nops_max, len);
+        auto emit = [&](uint32_t g, uint32_t slot) {
+          plan.slot.push_back(slot);
+          size_t at = plan.ops.size();
+          plan.ops.resize(at + modp_chain::OPS_MAX, (uint16_t)modp_chain::B_ONE);
+          std::copy(ops[g].begin(), ops[g].end(), plan.ops.begin() + at);
+        };
+        for (uint32_t g : cls) {
+          emit(g, bx.row_off + k * (uint32_t)bx.n + (g - base[b]));
+          plan.sqr += (uint64_t)sq[g] * (hi - lo - 1);
+          plan.mul += (uint64_t)ml[g] * (hi - lo - 1);
+        }
+        while (plan.slot.size() % per_cta) emit(cls.back(), 0xffffffffu);
+        const size_t ctas = plan.slot.size() / per_cta;
+        plan.nops.resize(ctas, len);
+        plan.first.resize(ctas, bx.cm_off + hi - 1);
+        plan.steps.resize(ctas, hi - lo - 1);
       }
-      while (plan.slot.size() % per_cta) emit(by[len].back(), 0xffffffffu);
-      const size_t ctas = plan.slot.size() / per_cta;
-      plan.nops.resize(ctas, len);
-      plan.first.resize(ctas, hi - 1);
-      plan.steps.resize(ctas, hi - lo - 1);
     }
   }
   return MPVSS_OK;
+}
+static int prep_positions(mpvss_ctx* ctx, const int64_t* positions, size_t n, size_t t, PosPlan& plan) {
+  const PlanBox box{positions, n, t, 0, 0};
+  return prep_boxes(ctx, &box, 1, true, plan);
 }
 
 // e_i = pos_i^E mod (q-1) for the chunk combination: q-1 = 2g, so by CRT e_i is the representative of
@@ -386,6 +416,7 @@ struct PlanDev {
   size_t n_padded;
   uint32_t K;
   int tpi, wpc;
+  bool boxes = false;  // a multi-box plan: only the per-CTA (first, steps) bounds describe it
 };
 // commitments (device, normal form) -> X (device): Montgomery conversion, Horner over every chunk, and for
 // K > 1 the combination X = H_0 * prod_{k >= 1} H_k^(pos^(k B)) (one exponentiation launch + K-1 products)
@@ -405,7 +436,7 @@ static int dev_horner(mpvss_ctx* ctx, const PlanDev& P, const uint32_t* comm, De
   // parameter bounds 220.2 ms (the code of round 2's first half), so the arrays are used always;
   // MPVSS_HORNER_UNIFORM=1 selects the other one for comparison runs.
   static const bool uniform = getenv("MPVSS_HORNER_UNIFORM") != nullptr;
-  const bool arrays = P.K > 1 || !uniform;
+  const bool arrays = P.K > 1 || P.boxes || !uniform;
   modp::HornerArgs A{Kq, cm.as<uint32_t>(), P.ops, P.slot, P.nops, h, (uint32_t)t, (uint32_t)P.n_padded, 0,
                      (uint32_t)P.wpc, arrays ? P.first : nullptr, arrays ? P.steps : nullptr};
   MPVSS_CUDA(ctx, cudaEventRecord(ctx->ev_h0, ctx->stream));
@@ -596,9 +627,9 @@ int scalar_poly_eval(mpvss_ctx* ctx, const uint8_t* coeffs, size_t t, const int6
 
 // Optional input validation ("validate" tunable; SURVEY 8f-3): the reference's bytes_to_element accepts any
 // integer (modp.rs:154-156).  Elements must satisfy 0 < x < q and lie in the subgroup of order g the
-// protocol works in: x^g = 1 (one exponentiation each, with the kernels of modulus q).  *valid = false
-// if any of the `count` device-resident elements fails.
-static int validate_elements(mpvss_ctx* ctx, const uint32_t* dev, size_t count, bool* valid) {
+// protocol works in: x^g = 1 (one exponentiation each, with the kernels of modulus q).  bad[i] = 1 for
+// each of the `count` device-resident elements that fails (the others are left as they are).
+static int validate_elements(mpvss_ctx* ctx, const uint32_t* dev, size_t count, uint8_t* bad) {
   std::vector<uint8_t> gexp(EB), res(count * EB), in(count * EB);
   big::to_le(ctx->g, gexp.data(), EB);
   DevBuf &de = ctx->buf(20), &dout = ctx->buf(21);
@@ -609,11 +640,11 @@ static int validate_elements(mpvss_ctx* ctx, const uint32_t* dev, size_t count, 
   MPVSS_TRY(d2h(ctx, res.data(), dout, count * EB));
   MPVSS_CUDA(ctx, cudaMemcpyAsync(in.data(), dev, count * EB, cudaMemcpyDeviceToHost, ctx->stream));
   MPVSS_TRY(sync(ctx));
-  for (size_t i = 0; i < count && *valid; ++i) {
+  for (size_t i = 0; i < count; ++i) {
     big::Int x = big::from_le(in.data() + i * EB, EB);
     bool one = res[i * EB] == 1;
     for (size_t k = 1; k < EB && one; ++k) one = res[i * EB + k] == 0;
-    if (big::is_zero(x) || big::cmp(x, ctx->q) >= 0 || !one) *valid = false;
+    if (big::is_zero(x) || big::cmp(x, ctx->q) >= 0 || !one) bad[i] = 1;
   }
   return MPVSS_OK;
 }
@@ -709,6 +740,36 @@ int verify_stage(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* commit
   return MPVSS_OK;
 }
 
+// Where a2 = y^r * Y^c (n instances, independent of X) runs beside an X_i launch of np padded instances at tpi
+// lanes per value whose longest chain takes `horner` products ("modp_overlap"; verify_kernels gives the
+// measurements): 0 before it on the main stream, 2 regular launch / 3 persistent one-warp CTAs on a side
+// stream after it.
+// Mode 3 only pays when the persistent CTAs finish inside the Horner launch: rounds of one
+// exponentiation per SM (about 5 products per 4-bit window) against the t-1 Horner steps of
+// nops products; measured break-even near 0.6 (tools/overlap_sweep.sh).  Otherwise a2 goes first.
+static int a2_placement(const mpvss_ctx* ctx, size_t n, double horner, size_t np, int tpi, uint32_t rwin, uint32_t cwin) {
+  int overlap = ctx->modp_overlap;
+  if (overlap == 3) {
+    const size_t groups_per_warp = 32 / (size_t)ctx->modp_tpi;
+    const size_t nwarps = (n + groups_per_warp - 1) / groups_per_warp;
+    const size_t rounds = (nwarps + (size_t)ctx->sm_count - 1) / (size_t)ctx->sm_count;
+    const double filler = (double)rounds * (5.0 * (rwin + cwin) + 30.0);
+    if (filler > 0.6 * horner) overlap = 0;
+    // ... and only when the Horner launch leaves a hole: W one-warp CTAs fill the 4 schedulers of every SM
+    // evenly when W is a multiple of 4 * SMs; the filler warp then becomes a third warp on one scheduler per SM
+    // and slows its two Horner warps for the whole launch (n = 4736 = 8 warps per SM: 308 instead of 261 ms)
+    const size_t slots = (size_t)4 * (size_t)ctx->sm_count;
+    const size_t hw = np / (32 / (size_t)tpi);
+    const size_t holes = (slots - hw % slots) % slots;
+    if (holes < (size_t)ctx->sm_count) overlap = 0;
+    // Small boxes: when both launches together stay below three warps per scheduler the chip has room for a2
+    // as a regular launch beside the X_i launch (measured, tools/small_box_overlap_sweep.sh: n = 1024, t = 683 36.5 -> 28.5 ms;
+    // n = 2048, t = 1366 72.9 -> 71.0 ms; at n = 4096 the same mode slows the X_i warps: 265.6 against 256.5 ms)
+    if (overlap == 0 && hw + nwarps <= (size_t)12 * (size_t)ctx->sm_count) overlap = 2;
+  }
+  return overlap;
+}
+
 // kernels of the staged verification: X (Horner), a1 = g^r * X^c, a2 = y^r * Y^c, then the framed rows
 static int verify_kernels(mpvss_ctx* ctx) {
   const size_t n = ctx->v_n, t = ctx->v_t;
@@ -733,29 +794,8 @@ static int verify_kernels(mpvss_ctx* ctx) {
                     ctx->v_y.as<uint32_t>(), EW, ctx->v_c.as<uint32_t>(), 0, ctx->v_cwin, n,
                     ctx->v_a2.as<uint32_t>(), s);
   };
-  // Mode 3 only pays when the persistent CTAs finish inside the Horner launch: rounds of one
-  // exponentiation per SM (about 5 products per 4-bit window) against the t-1 Horner steps of
-  // nops products; measured break-even near 0.6 (tools/overlap_sweep.sh).  Otherwise a2 goes first.
-  int overlap = ctx->modp_overlap;
-  if (overlap == 3) {
-    const size_t groups_per_warp = 32 / (size_t)ctx->modp_tpi;
-    const size_t nwarps = (n + groups_per_warp - 1) / groups_per_warp;
-    const size_t rounds = (nwarps + (size_t)ctx->sm_count - 1) / (size_t)ctx->sm_count;
-    const double filler = (double)rounds * (5.0 * (ctx->v_rwin + ctx->v_cwin) + 30.0);
-    const double horner = (double)(t > 1 ? t - 1 : 0) / (double)ctx->v_k * (double)ctx->v_nops_max;
-    if (filler > 0.6 * horner) overlap = 0;
-    // ... and only when the Horner launch leaves a hole: W one-warp CTAs fill the 4 schedulers of every SM
-    // evenly when W is a multiple of 4 * SMs; the filler warp then becomes a third warp on one scheduler per SM
-    // and slows its two Horner warps for the whole launch (n = 4736 = 8 warps per SM: 308 instead of 261 ms)
-    const size_t slots = (size_t)4 * (size_t)ctx->sm_count;
-    const size_t hw = ctx->v_np / (32 / (size_t)ctx->v_tpi);
-    const size_t holes = (slots - hw % slots) % slots;
-    if (holes < (size_t)ctx->sm_count) overlap = 0;
-    // Small boxes: when both launches together stay below three warps per scheduler the chip has room for a2
-    // as a regular launch beside the X_i launch (measured, tools/small_box_overlap_sweep.sh: n = 1024, t = 683 36.5 -> 28.5 ms;
-    // n = 2048, t = 1366 72.9 -> 71.0 ms; at n = 4096 the same mode slows the X_i warps: 265.6 against 256.5 ms)
-    if (overlap == 0 && hw + nwarps <= (size_t)12 * (size_t)ctx->sm_count) overlap = 2;
-  }
+  const int overlap = a2_placement(ctx, n, (double)(t > 1 ? t - 1 : 0) / (double)ctx->v_k * (double)ctx->v_nops_max,
+                                   ctx->v_np, ctx->v_tpi, ctx->v_rwin, ctx->v_cwin);
   const bool side = overlap == 2 || overlap == 3;
   if (!side) MPVSS_TRY(launch_a2(ctx->stream));
   // X_i from the commitments (participant.rs:423-434)
@@ -782,11 +822,12 @@ static int verify_kernels(mpvss_ctx* ctx) {
   MPVSS_CUDA(ctx, modp::launch_frames(FA, ctx->stream));
   timing_launch(ctx);
   if (ctx->validate) {
-    bool valid = true;
-    MPVSS_TRY(validate_elements(ctx, ctx->v_comm.as<uint32_t>(), t, &valid));
-    MPVSS_TRY(validate_elements(ctx, ctx->v_pk.as<uint32_t>(), n, &valid));
-    MPVSS_TRY(validate_elements(ctx, ctx->v_y.as<uint32_t>(), n, &valid));
-    if (!valid) {  // mark the rank's first row: 0xff is never part of a valid length (seen by all ranks)
+    std::vector<uint8_t> bad(t + 2 * n, 0);
+    MPVSS_TRY(validate_elements(ctx, ctx->v_comm.as<uint32_t>(), t, bad.data()));
+    MPVSS_TRY(validate_elements(ctx, ctx->v_pk.as<uint32_t>(), n, bad.data() + t));
+    MPVSS_TRY(validate_elements(ctx, ctx->v_y.as<uint32_t>(), n, bad.data() + t + n));
+    // mark the rank's first row: 0xff is never part of a valid length (seen by all ranks)
+    if (std::find(bad.begin(), bad.end(), 1) != bad.end()) {
       const uint8_t mark = 0xff;
       MPVSS_CUDA(ctx, cudaMemcpyAsync(ctx->v_frames.p, &mark, 1, cudaMemcpyHostToDevice, ctx->stream));
     }
@@ -830,6 +871,122 @@ int verify_run(mpvss_ctx* ctx, int* ok, uint8_t* x_out, uint8_t* a1_out, uint8_t
   if (a1_out) MPVSS_TRY(d2h(ctx, a1_out, ctx->v_a1, n * EB));
   if (a2_out) MPVSS_TRY(d2h(ctx, a2_out, ctx->v_a2, n * EB));
   return sync(ctx);
+}
+
+// ------------------------------------------------------ verify_distributions ----
+// Many boxes in one pass: one Horner launch evaluates X_i of every box (prep_boxes: each CTA reads its own
+// box's coefficients), a2 and a1 run once over all instances with one challenge per instance, the frames of
+// all boxes come to the host in one copy and each box's row range is hashed into its own digest.  a2 is
+// placed by the single-box rule (a2_placement) on the total instance count and the longest box's chain.
+// Only scratch buffers are used, so the staged single-box state and its cached plan stay valid.
+int verify_batch(mpvss_ctx* ctx, size_t nb, const size_t* nv, const size_t* tv, const uint8_t* commitments,
+                 const int64_t* positions, const uint8_t* publickeys, const uint8_t* shares, const uint8_t* responses,
+                 const uint8_t* challenges, int* ok_out, uint8_t* digests_out) {
+  std::vector<size_t> noff(nb + 1, 0), toff(nb + 1, 0);
+  for (size_t b = 0; b < nb; ++b) {
+    noff[b + 1] = noff[b] + nv[b];
+    toff[b + 1] = toff[b] + tv[b];
+  }
+  const size_t N = noff[nb], Tt = toff[nb];
+  // a position out of range makes its box false; the other boxes are planned
+  std::vector<uint8_t> live(nb, 1);
+  std::vector<PlanBox> boxes;
+  for (size_t b = 0; b < nb; ++b) {
+    const int64_t* p = positions ? positions + noff[b] : nullptr;
+    for (size_t i = 0; p && i < nv[b] && live[b]; ++i) live[b] = p[i] >= 1 && p[i] <= 0x7fffffff;
+    if (live[b]) boxes.push_back(PlanBox{p, nv[b], tv[b], (uint32_t)toff[b], (uint32_t)noff[b]});
+  }
+  std::vector<uint8_t> cexp(N * EB);  // the box's challenge for every instance
+  for (size_t b = 0; b < nb; ++b)
+    for (size_t i = noff[b]; i < noff[b + 1]; ++i) memcpy(cexp.data() + i * EB, challenges + b * EB, EB);
+  const uint32_t rwin = windows_for(responses, EB, N), cwin = windows_for(challenges, EB, nb);
+  DevBuf &dcomm = ctx->buf(0), &dcm = ctx->buf(1), &dpk = ctx->buf(2), &dy = ctx->buf(3), &dr = ctx->buf(4),
+         &dc = ctx->buf(5), &dx = ctx->buf(6), &da1 = ctx->buf(7), &da2 = ctx->buf(8), &dfr = ctx->buf(9),
+         &dops = ctx->buf(10), &dsl = ctx->buf(11), &dno = ctx->buf(12), &dfi = ctx->buf(13), &dstp = ctx->buf(14);
+  MPVSS_TRY(h2d(ctx, dcomm, commitments, Tt * EB));
+  MPVSS_TRY(h2d(ctx, dpk, publickeys, N * EB));
+  MPVSS_TRY(h2d(ctx, dy, shares, N * EB));
+  MPVSS_TRY(h2d(ctx, dr, responses, N * EB));
+  MPVSS_TRY(h2d(ctx, dc, cexp.data(), N * EB));
+  for (DevBuf* b : {&dx, &da1, &da2}) MPVSS_CUDA(ctx, b->ensure(N * EB));
+  MPVSS_CUDA(ctx, dfr.ensure(N * GEOM.row()));
+  if (boxes.size() < nb) MPVSS_CUDA(ctx, cudaMemsetAsync(dx.p, 0, N * EB, ctx->stream));  // rows no plan writes
+  PosPlan plan;
+  if (!boxes.empty()) {
+    MPVSS_TRY(prep_boxes(ctx, boxes.data(), boxes.size(), false, plan));
+    MPVSS_TRY(h2d(ctx, dops, plan.ops.data(), plan.ops.size() * 2));
+    MPVSS_TRY(h2d(ctx, dsl, plan.slot.data(), plan.slot.size() * 4));
+    MPVSS_TRY(h2d(ctx, dno, plan.nops.data(), plan.nops.size() * 4));
+    MPVSS_TRY(h2d(ctx, dfi, plan.first.data(), plan.first.size() * 4));
+    MPVSS_TRY(h2d(ctx, dstp, plan.steps.data(), plan.steps.size() * 4));
+  }
+  const uint32_t* comb;
+  MPVSS_TRY(comb_table(ctx, 1, &comb));
+  const uint32_t* K = ctx->consts_q.as<uint32_t>();
+  std::vector<uint8_t> bad(Tt + 2 * N, 0);  // validate: per commitment, public key and share
+  timing_begin(ctx);
+  if (!boxes.empty()) {
+    // a2 = y^r * Y^c (independent of X)
+    auto launch_a2 = [&](cudaStream_t s) {
+      return dev_exp2(ctx, K, dpk.as<uint32_t>(), EW, dr.as<uint32_t>(), EW, rwin, dy.as<uint32_t>(), EW,
+                      dc.as<uint32_t>(), EW, cwin, N, da2.as<uint32_t>(), s);
+    };
+    size_t tmax = 1;
+    for (const PlanBox& bx : boxes) tmax = std::max(tmax, bx.t);
+    const int overlap = a2_placement(ctx, N, (double)(tmax - 1) * (double)plan.nops_max, plan.slot.size(), plan.tpi,
+                                     rwin, cwin);
+    const bool side = overlap == 2 || overlap == 3;
+    MPVSS_CUDA(ctx, cudaEventRecord(ctx->ev_fork, ctx->stream));
+    if (!side) MPVSS_TRY(launch_a2(ctx->stream));
+    // X_i of every box (participant.rs:423-434); rows of boxes left out of the plan stay unwritten
+    PlanDev P{dops.as<uint16_t>(), dsl.as<uint32_t>(), dno.as<uint32_t>(), dfi.as<uint32_t>(), dstp.as<uint32_t>(),
+              nullptr, plan.slot.size(), plan.K, plan.tpi, plan.wpc, true};
+    MPVSS_TRY(dev_horner(ctx, P, dcomm.as<uint32_t>(), dcm, Tt, N, ctx->buf(15), ctx->buf(16), dx.as<uint32_t>()));
+    if (side) {
+      MPVSS_CUDA(ctx, cudaStreamWaitEvent(ctx->aux[0], ctx->ev_fork, 0));
+      if (overlap == 3) ctx->exp2_filler_ctas = (size_t)ctx->sm_count;
+      int rc = launch_a2(ctx->aux[0]);
+      ctx->exp2_filler_ctas = 0;
+      MPVSS_TRY(rc);
+      MPVSS_CUDA(ctx, cudaEventRecord(ctx->ev_join[0], ctx->aux[0]));
+    }
+    // a1 = g^r * X^c  (g^r from the fixed-base table)
+    MPVSS_TRY(dev_exp2(ctx, K, ctx->gens.as<uint32_t>() + 64, 0, dr.as<uint32_t>(), EW, rwin, dx.as<uint32_t>(), EW,
+                       dc.as<uint32_t>(), EW, cwin, N, da1.as<uint32_t>(), nullptr, comb));
+    if (side) MPVSS_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join[0], 0));
+    modp::FrameArgs FA{dx.as<uint32_t>(), dy.as<uint32_t>(), da1.as<uint32_t>(), da2.as<uint32_t>(), dfr.as<uint8_t>(),
+                       (uint32_t)N};
+    MPVSS_CUDA(ctx, modp::launch_frames(FA, ctx->stream));
+    timing_launch(ctx);
+    if (ctx->validate) {
+      MPVSS_TRY(validate_elements(ctx, dcomm.as<uint32_t>(), Tt, bad.data()));
+      MPVSS_TRY(validate_elements(ctx, dpk.as<uint32_t>(), N, bad.data() + Tt));
+      MPVSS_TRY(validate_elements(ctx, dy.as<uint32_t>(), N, bad.data() + Tt + N));
+    }
+  }
+  MPVSS_TRY(timing_end(ctx));
+  ctx->horner_sqr = plan.sqr;
+  ctx->horner_mul = plan.mul;
+  PinBuf& host = ctx->pin(0);
+  MPVSS_CUDA(ctx, host.ensure(N * GEOM.row()));
+  uint8_t* rows = host.as<uint8_t>();
+  MPVSS_TRY(d2h(ctx, rows, dfr, N * GEOM.row()));
+  MPVSS_TRY(sync(ctx));
+  for (size_t b = 0; b < nb; ++b) {
+    for (size_t j = toff[b]; j < toff[b + 1] && live[b]; ++j) live[b] = !bad[j];
+    for (size_t i = noff[b]; i < noff[b + 1] && live[b]; ++i) live[b] = !bad[Tt + i] && !bad[Tt + N + i];
+    uint8_t digest[32] = {0}, c[EB];
+    ok_out[b] = 0;
+    if (live[b]) {
+      sha2::Sha256 h;
+      transcript::hash_ordered(h, rows, noff[b], noff[b + 1], GEOM);
+      h.finalize(digest);
+      challenge_from_digest(ctx, digest, c);
+      ok_out[b] = memcmp(c, challenges + b * EB, EB) == 0;  // participant.rs:451-454
+    }
+    if (digests_out) memcpy(digests_out + 32 * b, digest, 32);
+  }
+  return MPVSS_OK;
 }
 
 // --------------------------------------------------------------- distribute ----

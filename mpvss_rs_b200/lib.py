@@ -47,6 +47,8 @@ SIGNATURES = {
                                                  _u8p, _u8p, _u8p, _u8p]),
     "mpvss_verify_distribution_stage": (ctypes.c_int, [_ctxp, _sz, _sz, _u8p, _i64p, _u8p, _u8p, _u8p, _u8p]),
     "mpvss_verify_distribution_run": (ctypes.c_int, [_ctxp, _intp, _u8p, _u8p, _u8p, _u8p]),
+    "mpvss_verify_distributions": (ctypes.c_int, [_ctxp, _sz, ctypes.POINTER(_sz), ctypes.POINTER(_sz), _u8p, _i64p,
+                                                  _u8p, _u8p, _u8p, _u8p, _intp, _u8p]),
     "mpvss_distribute": (ctypes.c_int, [_ctxp, _sz, _sz, _u8p, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p,
                                         _u8p, _u8p]),
     "mpvss_extract_shares": (ctypes.c_int, [_ctxp, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _intp]),

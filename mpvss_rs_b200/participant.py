@@ -6,7 +6,7 @@ tests read like the reference's own tests; every group operation goes through
 libmpvss_b200.so (CUDA).  The only additions are the randomness-injection
 arguments (`coeffs`, `witnesses`, `private_key`) -- the reference draws those from
 `thread_rng` internally (polynomial.rs:34-47, participant.rs:223, 139-146) -- and
-the batch forms `extract_secret_shares` / `verify_shares`.
+the batch forms `extract_secret_shares` / `verify_shares` / `verify_distributions`.
 
 Value representation at this level: MODP elements and all scalars are Python
 ints (the reference uses BigInt); secp256k1 / ristretto255 elements are their
@@ -283,6 +283,36 @@ class Participant:
         if trace is not None:
             trace["digest"] = bytes(dig)
         return bool(ok.value)
+
+    def verify_distributions(self, boxes, traces=None) -> list:
+        """Batch form of verify_distribution_shares: one verdict per box, all boxes in one library call
+        (mpvss_verify_distributions).  traces[b]["digest"] receives box b's transcript digest."""
+        g, c = self.group, self.group.codec
+        res = [False] * len(boxes)
+        live, flats = [], []
+        for b, box in enumerate(boxes):
+            flat = self._flatten(box)
+            if flat is not None:                                # participant.rs:415-420
+                live.append(b)
+                flats.append(flat)
+        if not live:
+            return res
+        m = len(live)
+        ns = [len(f[0]) for f in flats]
+        ts = [len(boxes[b].commitments) for b in live]
+        pos = [p for f in flats for p in f[0]]
+        ok, dig = (ctypes.c_int * m)(), buf(size=32 * m)
+        g.ctx.check(g.ctx.lib.mpvss_verify_distributions(
+            g.ctx.h, m, (ctypes.c_size_t * m)(*ns), (ctypes.c_size_t * m)(*ts),
+            ptr(buf(b"".join(c.enc_elems(boxes[b].commitments) for b in live))), (ctypes.c_int64 * len(pos))(*pos),
+            ptr(buf(b"".join(c.enc_elems(boxes[b].publickeys) for b in live))),
+            ptr(buf(b"".join(c.enc_elems(f[1]) for f in flats))), ptr(buf(b"".join(c.enc_scalars(f[2]) for f in flats))),
+            ptr(buf(b"".join(c.enc_scalar(boxes[b].challenge) for b in live))), ok, ptr(dig)))
+        for j, b in enumerate(live):
+            res[b] = bool(ok[j])
+            if traces is not None:
+                traces[b]["digest"] = bytes(dig)[32 * j:32 * j + 32]
+        return res
 
     # -- extract_secret_share: participant.rs:294-353 / 1282-1338 / 1725-1781 --
     def extract_secret_shares(self, box, private_keys, ws):
