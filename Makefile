@@ -20,7 +20,7 @@ $(CSRC)/sha256_ni.o: $(CSRC)/sha256_ni.cpp
 $(LIB): $(OBJ)
 	$(NVCC) -shared -o $@ $(OBJ) -Xcompiler -pthread -ldl
 
-emu: tests/emu/libemu_modp.so tests/emu/libemu_ec.so tests/emu/libemu_multibox.so
+emu: tests/emu/libemu_modp.so tests/emu/libemu_ec.so tests/emu/libemu_multibox.so tests/emu/libemu_reconstruct_batch.so
 tests/emu/libemu_%.so: tests/emu/emu_%.cpp $(HDR)
 	$(CXX) -std=c++20 -O2 -DMPVSS_SIMT_EMU -shared -fPIC -pthread -o $@ $<
 

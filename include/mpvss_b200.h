@@ -191,6 +191,20 @@ int mpvss_verify_shares(mpvss_ctx* ctx, size_t n, const uint8_t* publickeys, con
  * left-padded).  gs_out (optional) receives G^s. */
 int mpvss_reconstruct(mpvss_ctx* ctx, size_t k, const int64_t* positions, const uint8_t* shares, const uint8_t* u,
                       uint8_t* secret_out, uint8_t* gs_out);
+/* n_boxes independent Participant::reconstruct calls in one (e.g. every dealer's secret of one PVSS round).
+ * Box b has k[b] decrypted shares.  positions (sum k[b], 1-based) and shares (sum k[b] elements) are
+ * concatenated in box order, u holds n_boxes elements (element-size big-endian each, as mpvss_reconstruct takes
+ * U).  secrets_out[b] (element size) and gs_out[b] (optional) are what mpvss_reconstruct returns for box b
+ * alone, and status_out[b] is its status: MPVSS_ERR_ARG for a position outside [1, 2^31) or, in ModpGroup, a
+ * duplicate position; MPVSS_ERR_ENCODING for a share that does not decode or a mask the group rejects.  A box
+ * that fails has zero rows in secrets_out / gs_out and leaves the other boxes alone; the call still returns
+ * MPVSS_OK and records no error.  Caller errors return MPVSS_ERR_ARG: no boxes, a null pointer other than
+ * gs_out, an empty box, or more shares than 32-bit counts hold.  Staged mpvss_verify_distribution_stage state
+ * is left untouched.  Not collective: on a context with a communicator it runs on that context's device, as
+ * mpvss_reconstruct does. */
+int mpvss_reconstruct_secrets(mpvss_ctx* ctx, size_t n_boxes, const size_t* k, const int64_t* positions,
+                              const uint8_t* shares, const uint8_t* u, uint8_t* secrets_out, uint8_t* gs_out,
+                              int* status_out);
 
 /* ---- multi-GPU --------------------------------------------------------------------- */
 /* One context per GPU.  Rank 0 obtains an id (ncclGetUniqueId), the caller distributes its

@@ -309,5 +309,22 @@ int mpvss_reconstruct(mpvss_ctx* ctx, size_t k, const int64_t* positions, const 
                       uint8_t* secret_out, uint8_t* gs_out) {
   DISPATCH(ctx, reconstruct, k, positions, shares, u, secret_out, gs_out);
 }
+int mpvss_reconstruct_secrets(mpvss_ctx* ctx, size_t n_boxes, const size_t* k, const int64_t* positions,
+                              const uint8_t* shares, const uint8_t* u, uint8_t* secrets_out, uint8_t* gs_out,
+                              int* status_out) {
+  if (!ctx) return MPVSS_ERR_ARG;
+  Guard hold(ctx);
+  if (n_boxes == 0 || !k || !positions || !shares || !u || !secrets_out || !status_out)
+    return mpvss_fail(ctx, MPVSS_ERR_ARG, "reconstruct_secrets: bad arguments");
+  const size_t limit = 0x7fffffff;  // the kernels count shares in 32 bits
+  size_t sum_k = 0;
+  for (size_t b = 0; b < n_boxes; ++b) {
+    if (k[b] == 0 || k[b] > limit - sum_k)
+      return mpvss_fail(ctx, MPVSS_ERR_ARG, "reconstruct_secrets: box " + std::to_string(b) +
+                                                " has no shares, or the boxes are too many");
+    sum_k += k[b];
+  }
+  DISPATCH(ctx, reconstruct_batch, n_boxes, k, positions, shares, u, secrets_out, gs_out, status_out);
+}
 
 }  // extern "C"

@@ -90,6 +90,11 @@ struct mpvss_ctx {
   int modp_msm = 2;          // multi_exp / reconstruct by buckets: 0 never, 1 always, 2 from msm_threshold bases on
   int msm_threshold = 512;   // measured on B200: buckets 9.0 / 9.8 / 12.4 / 22.5 ms against 9.2 / 13.4 / 33.1 / 119.6 ms direct
                              // at k = 683 / 2731 / 10923 / 43691 (profiles/msm_r02.json)
+  // reconstruct_secrets with two or more live boxes (modp_msm = 2): a box takes the bucket method from this many
+  // shares on, otherwise its exponentiations join the batch's one direct launch, where it pays only its share of
+  // a launch that is already full.  Measured on B200 (profiles/reconstruct_batch_r03.json, whole batch direct vs
+  // every box by buckets): 4 x 2731 shares 41.0 vs 57.5 ms, 2 x 5462 43.8 vs 35.8 ms, 2 x 10923 98.5 vs 62.1 ms.
+  static constexpr size_t msm_batch_threshold = 4096;
   bool device_hash = false;  // whole-box transcript as one SHA-256 chain on one device thread (measured alternative)
   bool validate = false;     // range / subgroup check of ModpGroup elements entering the verify calls
   bool modp_np1 = false;     // -q^-1 = 1 mod 2^32: Horner kernels skip the Montgomery-digit multiply
@@ -173,6 +178,8 @@ int extract_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uin
 int verify_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
                   int*);
 int reconstruct(mpvss_ctx*, size_t, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*);
+int reconstruct_batch(mpvss_ctx*, size_t, const size_t*, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*,
+                      uint8_t*, int*);
 }  // namespace modp_api
 namespace secp_api {
 int init(mpvss_ctx* ctx);
@@ -197,6 +204,8 @@ int extract_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uin
 int verify_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
                   int*);
 int reconstruct(mpvss_ctx*, size_t, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*);
+int reconstruct_batch(mpvss_ctx*, size_t, const size_t*, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*,
+                      uint8_t*, int*);
 }  // namespace secp_api
 namespace rist_api {
 int init(mpvss_ctx* ctx);
@@ -221,4 +230,6 @@ int extract_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uin
 int verify_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
                   int*);
 int reconstruct(mpvss_ctx*, size_t, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*);
+int reconstruct_batch(mpvss_ctx*, size_t, const size_t*, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*,
+                      uint8_t*, int*);
 }  // namespace rist_api

@@ -33,10 +33,12 @@ template <class Cv> __global__ void __launch_bounds__(TPB, EC_HORNER_MIN_BLOCKS)
   horner_boxes_body<Cv>(A, TID);
 }
 template <class Cv> __global__ void __launch_bounds__(TPB) sum_kernel(SumArgs<Cv> A) { sum_body<Cv>(A, TID); }
+template <class Cv> __global__ void __launch_bounds__(TPB) sum_boxes_kernel(SumBoxesArgs<Cv> A) { sum_boxes_body<Cv>(A, TID); }
 template <class Cv> __global__ void __launch_bounds__(TPB) add_kernel(AddArgs<Cv> A) { add_body<Cv>(A, TID); }
 __global__ void __launch_bounds__(TPB) frame_kernel(FrameArgs A) { frame_body(A, TID); }
 __global__ void __launch_bounds__(TPB) poly_kernel(PolyArgs A) { poly_body(A, TID); }
 __global__ void __launch_bounds__(TPB) lagrange_kernel(LagrangeArgs A) { lagrange_body(A, TID); }
+__global__ void __launch_bounds__(TPB) lagrange_boxes_kernel(LagrangeBoxesArgs A) { lagrange_boxes_body(A, TID); }
 __global__ void __launch_bounds__(TPB) inv_kernel(InvArgs A) { inv_body(A, TID); }
 __global__ void __launch_bounds__(TPB) proof_kernel(ProofArgs A) { proof_body(A, TID); }
 
@@ -82,6 +84,11 @@ template <class Cv> cudaError_t launch_sum(const SumArgs<Cv>& A, cudaStream_t s)
   sum_kernel<Cv><<<blocks(A.groups), TPB, 0, s>>>(A);
   return cudaGetLastError();
 }
+template <class Cv> cudaError_t launch_sum_boxes(const SumBoxesArgs<Cv>& A, cudaStream_t s) {
+  if (A.groups == 0) return cudaErrorInvalidValue;
+  sum_boxes_kernel<Cv><<<blocks(A.groups), TPB, 0, s>>>(A);
+  return cudaGetLastError();
+}
 template <class Cv> cudaError_t launch_add(const AddArgs<Cv>& A, cudaStream_t s) {
   if (A.n == 0) return cudaErrorInvalidValue;
   add_kernel<Cv><<<blocks(A.n), TPB, 0, s>>>(A);
@@ -100,6 +107,11 @@ cudaError_t launch_poly(const PolyArgs& A, cudaStream_t s) {
 cudaError_t launch_lagrange(const LagrangeArgs& A, cudaStream_t s) {
   if (A.k == 0) return cudaErrorInvalidValue;
   lagrange_kernel<<<blocks(A.k), TPB, 0, s>>>(A);
+  return cudaGetLastError();
+}
+cudaError_t launch_lagrange_boxes(const LagrangeBoxesArgs& A, cudaStream_t s) {
+  if (A.n == 0) return cudaErrorInvalidValue;
+  lagrange_boxes_kernel<<<blocks(A.n), TPB, 0, s>>>(A);
   return cudaGetLastError();
 }
 cudaError_t launch_inv(const InvArgs& A, cudaStream_t s) {
@@ -122,6 +134,7 @@ cudaError_t launch_proof(const ProofArgs& A, cudaStream_t s) {
   template cudaError_t launch_horner<Cv>(const HornerArgs<Cv>&, cudaStream_t);           \
   template cudaError_t launch_horner_boxes<Cv>(const HornerBoxesArgs<Cv>&, cudaStream_t); \
   template cudaError_t launch_sum<Cv>(const SumArgs<Cv>&, cudaStream_t);                 \
+  template cudaError_t launch_sum_boxes<Cv>(const SumBoxesArgs<Cv>&, cudaStream_t);      \
   template cudaError_t launch_add<Cv>(const AddArgs<Cv>&, cudaStream_t);
 INSTANTIATE(secp::SecpCurve)
 INSTANTIATE(rist::RistCurve)

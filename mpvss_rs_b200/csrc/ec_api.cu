@@ -1023,6 +1023,109 @@ struct Ec {
     if (gs_out) memcpy(gs_out, gs, EB);
     return MPVSS_OK;
   }
+
+  // Many reconstruct calls in one (mpvss_reconstruct_secrets): the live boxes' positions and shares are
+  // concatenated; one box-aware Lagrange launch, one dev_exp2 launch over every share into projective points
+  // (its per-share status gives a box's ERR_ENCODING), then segmented 64-way sums that never cross a box
+  // boundary until each box has one point, which the last level encodes.
+  static int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t* positions,
+                               const uint8_t* shares, const uint8_t* u, uint8_t* secrets_out, uint8_t* gs_out,
+                               int* status_out) {
+    memset(secrets_out, 0, nb * EB);
+    if (gs_out) memset(gs_out, 0, nb * EB);
+    ctx->last_ms = 0.f;
+    ctx->last_launches = 0;
+    std::vector<size_t> live, first(nb);  // boxes whose positions are in range; each box's first share
+    for (size_t b = 0, off = 0; b < nb; off += kv[b], ++b) {
+      first[b] = off;
+      status_out[b] = MPVSS_OK;
+      for (size_t i = off; i < off + kv[b]; ++i)
+        if (positions[i] < 1 || positions[i] > 0x7fffffff) status_out[b] = MPVSS_ERR_ARG;
+      if (status_out[b] == MPVSS_OK) live.push_back(b);
+    }
+    if (live.empty()) return MPVSS_OK;
+    const size_t L = live.size();
+    size_t n = 0;
+    std::vector<uint32_t> start(L), cnt(L);
+    for (size_t j = 0; j < L; ++j) {
+      start[j] = (uint32_t)n;
+      cnt[j] = (uint32_t)kv[live[j]];
+      n += cnt[j];
+    }
+    std::vector<uint32_t> idx(3 * n);  // positions, then per position its box's first row, then its box's k
+    std::vector<uint8_t> host(n * EB);
+    for (size_t j = 0; j < L; ++j) {
+      for (uint32_t i = 0; i < cnt[j]; ++i) {
+        idx[start[j] + i] = (uint32_t)positions[first[live[j]] + i];
+        idx[n + start[j] + i] = start[j];
+        idx[2 * n + start[j] + i] = cnt[j];
+      }
+      memcpy(host.data() + (size_t)start[j] * EB, shares + first[live[j]] * EB, cnt[j] * EB);
+    }
+    // every level of the segmented sum, planned here and uploaded at once
+    std::vector<uint32_t> seg, level_end;
+    {
+      std::vector<uint32_t> s(start), c(cnt);
+      for (bool last = false; !last;) {
+        last = *std::max_element(c.begin(), c.end()) <= 64;
+        size_t groups = 0;
+        for (uint32_t x : c) groups += (x + 63) / 64;
+        const size_t lo = seg.size() / 2;
+        seg.resize(2 * (lo + groups));
+        ec::sum_boxes_level(s.data(), c.data(), (uint32_t)L, seg.data() + 2 * lo);
+        level_end.push_back((uint32_t)(lo + groups));
+      }
+    }
+    DevBuf &dsh = ctx->buf(0), &didx = ctx->buf(1), &dlam = ctx->buf(2), &dj = ctx->buf(3), &dst = ctx->buf(4),
+           &dseg = ctx->buf(5), &dtmp = ctx->buf(6), &dout = ctx->buf(7);
+    MPVSS_TRY(h2d(ctx, dsh, host.data(), n * EB));
+    MPVSS_TRY(h2d(ctx, didx, idx.data(), 3 * n * 4));
+    MPVSS_TRY(h2d(ctx, dseg, seg.data(), seg.size() * 4));
+    const size_t g1 = level_end[0];  // the first level has the most groups
+    MPVSS_CUDA(ctx, dlam.ensure(n * 32));
+    MPVSS_CUDA(ctx, dj.ensure(n * sizeof(Point)));
+    MPVSS_CUDA(ctx, dst.ensure(n * 4));
+    MPVSS_CUDA(ctx, dtmp.ensure(2 * g1 * sizeof(Point)));
+    MPVSS_CUDA(ctx, dout.ensure(L * EB));
+    const uint32_t* di = didx.as<uint32_t>();
+    ec::LagrangeBoxesArgs LA{KN(ctx), di, di + n, di + 2 * n, dlam.as<uint32_t>(), (uint32_t)n};
+    timing_begin(ctx);
+    MPVSS_CUDA(ctx, ec::launch_lagrange_boxes(LA, ctx->stream));
+    timing_launch(ctx);
+    MPVSS_TRY(dev_exp2(ctx, dsh.as<uint8_t>(), EB, dlam.as<uint32_t>(), nullptr, 0, nullptr, 0, n, nullptr,
+                       dj.as<Point>(), dst.as<uint32_t>()));
+    const Point* cur = dj.as<Point>();
+    Point* nxt = dtmp.as<Point>();
+    Point* alt = nxt + g1;
+    for (size_t l = 0; l < level_end.size(); ++l) {
+      const uint32_t lo = l ? level_end[l - 1] : 0;
+      const bool last = l + 1 == level_end.size();
+      ec::SumBoxesArgs<Cv> S{K(ctx), cur, dseg.as<uint32_t>() + 2 * lo, last ? nullptr : nxt,
+                             last ? dout.as<uint8_t>() : nullptr, level_end[l] - lo};
+      MPVSS_CUDA(ctx, ec::launch_sum_boxes<Cv>(S, ctx->stream));
+      timing_launch(ctx);
+      cur = nxt;
+      std::swap(nxt, alt);
+    }
+    MPVSS_TRY(timing_end(ctx));
+    std::vector<uint32_t> st(n);
+    std::vector<uint8_t> gs(L * EB);
+    MPVSS_TRY(d2h(ctx, st.data(), dst, n * 4));
+    MPVSS_TRY(d2h(ctx, gs.data(), dout, L * EB));
+    MPVSS_TRY(sync(ctx));
+    for (size_t j = 0; j < L; ++j) {
+      const size_t b = live[j];
+      big::Int mask;
+      if (std::find(st.begin() + start[j], st.begin() + start[j] + cnt[j], 1u) != st.begin() + start[j] + cnt[j] ||
+          !T::mask_of(gs.data() + j * EB, ctx->ec_order, &mask)) {
+        status_out[b] = MPVSS_ERR_ENCODING;
+        continue;
+      }
+      big::to_be(big::bxor(mask, big::from_be(u + b * EB, EB)), secrets_out + b * EB, EB);
+      if (gs_out) memcpy(gs_out + b * EB, gs.data() + j * EB, EB);
+    }
+    return MPVSS_OK;
+  }
 };
 
 }  // namespace
@@ -1082,6 +1185,10 @@ struct Ec {
   int reconstruct(mpvss_ctx* c, size_t k, const int64_t* p, const uint8_t* s, const uint8_t* u, uint8_t* o,          \
                   uint8_t* gs) {                                                                                     \
     return Ec<Traits>::reconstruct(c, k, p, s, u, o, gs);                                                            \
+  }                                                                                                                  \
+  int reconstruct_batch(mpvss_ctx* c, size_t nb, const size_t* k, const int64_t* p, const uint8_t* s,              \
+                        const uint8_t* u, uint8_t* o, uint8_t* gs, int* st) {                                        \
+    return Ec<Traits>::reconstruct_batch(c, nb, k, p, s, u, o, gs, st);                                              \
   }                                                                                                                  \
   }
 

@@ -347,6 +347,48 @@ MP_DEV void sum_body(const SumArgs<Cv>& A, uint32_t tid) {
   if (A.out) Cv::encode(A.out + (size_t)tid * Cv::EB, acc, C);
 }
 
+// Segmented sum (mpvss_reconstruct_secrets): group g adds the seg[2g + 1] >= 1 points from row seg[2g]; the host
+// plans the segments with sum_boxes_level so that none crosses a box boundary.
+template <class Cv>
+struct SumBoxesArgs {
+  const typename Cv::Consts* C;
+  const typename Cv::Point* in;
+  const uint32_t* seg;           // groups x (first row, count)
+  typename Cv::Point* out_jac;   // groups results (or nullptr)
+  uint8_t* out;                  // groups encoded results (or nullptr)
+  uint32_t groups;
+};
+template <class Cv>
+MP_DEV void sum_boxes_body(const SumBoxesArgs<Cv>& A, uint32_t tid) {
+  if (tid >= A.groups) return;
+  const typename Cv::Consts& C = *A.C;
+  const uint32_t first = A.seg[2 * tid], count = A.seg[2 * tid + 1];
+  typename Cv::Point acc = A.in[first];
+#pragma unroll 1
+  for (uint32_t j = 1; j < count; ++j) acc = Cv::add(acc, A.in[first + j], C);
+  if (A.out_jac) A.out_jac[tid] = acc;
+  if (A.out) Cv::encode(A.out + (size_t)tid * Cv::EB, acc, C);
+}
+
+// One level of the segmented sum (host planning, shared with the tests): box b holds cnt[b] points from row
+// start[b]; every 64 consecutive points of a box form one group, and the groups are numbered in box order.
+// Writes the groups' (first row, count) to `seg`, moves start / cnt to the box's group results and returns the
+// group count.  A level planned while every cnt is at most 64 has one group per box: group b is box b.
+inline uint32_t sum_boxes_level(uint32_t* start, uint32_t* cnt, uint32_t boxes, uint32_t* seg) {
+  uint32_t m = 0;
+  for (uint32_t b = 0; b < boxes; ++b) {
+    const uint32_t first = m;
+    for (uint32_t j = 0; j < cnt[b]; j += 64) {
+      seg[2 * m] = start[b] + j;
+      seg[2 * m + 1] = cnt[b] - j < 64 ? cnt[b] - j : 64;
+      ++m;
+    }
+    start[b] = first;
+    cnt[b] = m - first;
+  }
+  return m;
+}
+
 // out[i] = a[i] + b[i]   (Group::mul)
 template <class Cv>
 struct AddArgs {
@@ -467,6 +509,23 @@ MP_DEV void lagrange_body(const LagrangeArgs& A, uint32_t tid) {
   Fe lam = mul(num, inv(den, N), N);  // den = 0 (duplicate position) -> lambda = 0, as ristretto255.rs falls back
   if (negative) lam = neg(lam, N);
   store(A.out + (size_t)tid * 8, from_mont(lam, N));
+}
+
+// Several boxes at once (mpvss_reconstruct_secrets): the positions of the boxes are concatenated, position i
+// belongs to the box of bk[i] positions that starts at boff[i], and its coefficient is lagrange_body's over
+// that box alone.
+struct LagrangeBoxesArgs {
+  const Modulus* N;
+  const uint32_t* pos;   // n positions, concatenated over the boxes
+  const uint32_t* boff;  // per position: first position of its box
+  const uint32_t* bk;    // per position: positions k_b of its box
+  uint32_t* out;         // n x 8 limbs
+  uint32_t n;
+};
+MP_DEV void lagrange_boxes_body(const LagrangeBoxesArgs& A, uint32_t tid) {
+  if (tid >= A.n) return;
+  const uint32_t off = A.boff[tid];
+  lagrange_body(LagrangeArgs{A.N, A.pos + off, A.out + (size_t)off * 8, A.bk[tid]}, tid - off);
 }
 
 // out[i] = in[i]^-1 in the scalar field (0 -> 0, flagged in status)

@@ -19,10 +19,12 @@ template <class Cv> cudaError_t launch_decode(const DecodeArgs<Cv>& A, cudaStrea
 template <class Cv> cudaError_t launch_horner(const HornerArgs<Cv>& A, cudaStream_t s);
 template <class Cv> cudaError_t launch_horner_boxes(const HornerBoxesArgs<Cv>& A, cudaStream_t s);
 template <class Cv> cudaError_t launch_sum(const SumArgs<Cv>& A, cudaStream_t s);
+template <class Cv> cudaError_t launch_sum_boxes(const SumBoxesArgs<Cv>& A, cudaStream_t s);
 template <class Cv> cudaError_t launch_add(const AddArgs<Cv>& A, cudaStream_t s);
 cudaError_t launch_frames(const FrameArgs& A, cudaStream_t s);
 cudaError_t launch_poly(const PolyArgs& A, cudaStream_t s);
 cudaError_t launch_lagrange(const LagrangeArgs& A, cudaStream_t s);
+cudaError_t launch_lagrange_boxes(const LagrangeBoxesArgs& A, cudaStream_t s);
 cudaError_t launch_inv(const InvArgs& A, cudaStream_t s);
 cudaError_t launch_proof(const ProofArgs& A, cudaStream_t s);
 }  // namespace ec

@@ -55,6 +55,16 @@ __global__ void __launch_bounds__(128) frame_kernel(FrameArgs A) { frame_body(A,
 __global__ void __launch_bounds__(64) resp_kernel(RespArgs A) { resp_body(A, blockIdx.x * 64 + threadIdx.x); }
 __global__ void __launch_bounds__(64) poly_kernel(PolyArgs A) { poly_body(A, blockIdx.x * 64 + threadIdx.x); }
 __global__ void __launch_bounds__(64) lagrange_kernel(LagrangeArgs A) { lagrange_body(A, blockIdx.x * 64 + threadIdx.x); }
+__global__ void __launch_bounds__(64) lagrange_boxes_kernel(LagrangeBoxesArgs A) {
+  lagrange_boxes_body(A, blockIdx.x * 64 + threadIdx.x);
+}
+
+template <int TPI>
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32) mul_rows_kernel(MulRowsArgs A) {
+  extern __shared__ __align__(16) uint32_t smem[];
+  uint32_t w = threadIdx.x >> 5;
+  mul_rows_body<TPI>(A, blockIdx.x * WARPS_PER_CTA + w, smem + w * mul_smem_words<TPI>);
+}
 
 // Counting sort of the exponent bytes for the bucket method: CTA w orders the indices 0..k-1 by byte w of
 // their exponent (idx, window-major) and writes the 257 bucket boundaries (start).  The order inside a
@@ -191,6 +201,13 @@ cudaError_t launch_lagrange(const LagrangeArgs& A, cudaStream_t s) {
   return cudaGetLastError();
 }
 
+cudaError_t launch_lagrange_boxes(const LagrangeBoxesArgs& A, cudaStream_t s) {
+  if (A.n == 0) return cudaErrorInvalidValue;
+  const uint32_t threads = 2u * (A.parts ? A.parts : 1u) * A.n;
+  lagrange_boxes_kernel<<<(threads + 63) / 64, 64, 0, s>>>(A);
+  return cudaGetLastError();
+}
+
 cudaError_t launch_comb_build(int tpi, const CombArgs& A, cudaStream_t s) {
   MODP_DISPATCH(tpi, {
     size_t sm = comb_smem_words<T> * 4;
@@ -223,6 +240,17 @@ cudaError_t launch_mul(int tpi, const MulArgs& A, cudaStream_t s) {
     cudaError_t e = set_smem(mul_kernel<T>, sm);
     if (e != cudaSuccess) return e;
     mul_kernel<T><<<ctas_for<T>(A.n), WARPS_PER_CTA * 32, sm, s>>>(A);
+  });
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mul_rows(int tpi, const MulRowsArgs& A, cudaStream_t s) {
+  if (A.n == 0) return cudaErrorInvalidValue;
+  MODP_DISPATCH(tpi, {
+    size_t sm = WARPS_PER_CTA * mul_smem_words<T> * 4;
+    cudaError_t e = set_smem(mul_rows_kernel<T>, sm);
+    if (e != cudaSuccess) return e;
+    mul_rows_kernel<T><<<ctas_for<T>(A.n), WARPS_PER_CTA * 32, sm, s>>>(A);
   });
   return cudaGetLastError();
 }

@@ -1366,4 +1366,141 @@ int reconstruct(mpvss_ctx* ctx, size_t k, const int64_t* positions, const uint8_
   return MPVSS_OK;
 }
 
+// Many reconstruct calls in one (mpvss_reconstruct_secrets).  The live boxes' positions and shares are
+// concatenated, the boxes that take the direct method first.  One box-aware Lagrange launch, the part products,
+// ONE batch inversion mod g over every box's denominators, and the signs folded on the host as reconstruct
+// does; then one dev_exp2 launch over every direct box's shares, reduced by a segmented product tree (one
+// gather-multiply launch per level), and the bucket method box after box for the others.
+int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t* positions, const uint8_t* shares,
+                      const uint8_t* u, uint8_t* secrets_out, uint8_t* gs_out, int* status_out) {
+  memset(secrets_out, 0, nb * EB);
+  if (gs_out) memset(gs_out, 0, nb * EB);
+  ctx->last_ms = 0.f;
+  ctx->last_launches = 0;
+  std::vector<size_t> live, first(nb);  // boxes that pass reconstruct's checks; each box's first share
+  for (size_t b = 0, off = 0; b < nb; off += kv[b], ++b) {
+    first[b] = off;
+    status_out[b] = MPVSS_OK;
+    std::vector<int64_t> sorted(positions + off, positions + off + kv[b]);
+    std::sort(sorted.begin(), sorted.end());
+    if (sorted.front() < 1 || sorted.back() > 0x7fffffff || std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
+      status_out[b] = MPVSS_ERR_ARG;
+    else
+      live.push_back(b);
+  }
+  if (live.empty()) return MPVSS_OK;
+  // a lone box chooses as reconstruct does; in a batch a box joins the direct launch below msm_batch_threshold
+  const size_t threshold = live.size() == 1 ? (size_t)ctx->msm_threshold : mpvss_ctx::msm_batch_threshold;
+  auto buckets = [&](size_t b) { return ctx->modp_msm == 1 || (ctx->modp_msm == 2 && kv[b] >= threshold); };
+  std::stable_partition(live.begin(), live.end(), [&](size_t b) { return !buckets(b); });
+  const size_t L = live.size();
+  size_t n = 0, n_direct = 0, L_direct = 0, kmax = 0;  // rows / boxes of the direct launch
+  std::vector<uint32_t> start(L), cnt(L);
+  for (size_t j = 0; j < L; ++j) {
+    start[j] = (uint32_t)n;
+    cnt[j] = (uint32_t)kv[live[j]];
+    n += cnt[j];
+    kmax = std::max<size_t>(kmax, cnt[j]);
+    if (!buckets(live[j])) n_direct = n, L_direct = j + 1;
+  }
+  std::vector<uint32_t> idx(3 * n);  // positions, then per position its box's first row, then its box's k
+  std::vector<uint8_t> host(n * EB);
+  for (size_t j = 0; j < L; ++j) {
+    const size_t b = live[j];
+    for (uint32_t i = 0; i < cnt[j]; ++i) {
+      idx[start[j] + i] = (uint32_t)positions[first[b] + i];
+      idx[n + start[j] + i] = start[j];
+      idx[2 * n + start[j] + i] = cnt[j];
+    }
+    memcpy(host.data() + (size_t)start[j] * EB, shares + first[b] * EB, cnt[j] * EB);
+  }
+  // multi_exp_buckets holds buf(15..19) and dev_batch_inverse_g buf(21..23)
+  DevBuf &dshares = ctx->buf(0), &dexp = ctx->buf(1), &dpow = ctx->buf(2), &dplan = ctx->buf(4), &didx = ctx->buf(10),
+         &dord = ctx->buf(11), &dnum = ctx->buf(12), &dden = ctx->buf(13), &dneg = ctx->buf(14), &dinv = ctx->buf(20);
+  std::vector<uint32_t> order(EW, 0);
+  for (size_t i = 0; i < ctx->qm1.size(); ++i) order[i] = ctx->qm1[i];
+  MPVSS_TRY(h2d(ctx, didx, idx.data(), 3 * n * 4));
+  MPVSS_TRY(h2d(ctx, dord, order.data(), EB));
+  MPVSS_TRY(h2d(ctx, dshares, host.data(), n * EB));
+  const size_t parts = kmax >= 64 ? 8 : 1;  // as reconstruct cuts a box of kmax positions
+  for (DevBuf* b : {&dnum, &dden}) MPVSS_CUDA(ctx, b->ensure(parts * n * EB));
+  MPVSS_CUDA(ctx, dinv.ensure(n * EB));
+  MPVSS_CUDA(ctx, dneg.ensure(parts * n * 4));
+  MPVSS_CUDA(ctx, dpow.ensure(n * EB));
+  const uint32_t* K = ctx->consts_q.as<uint32_t>();
+  const uint32_t* Kg = ctx->consts_g.as<uint32_t>();
+  const uint32_t* di = didx.as<uint32_t>();
+  modp::LagrangeBoxesArgs LA{dord.as<uint32_t>(), di, di + n, di + 2 * n, dnum.as<uint32_t>(), dden.as<uint32_t>(),
+                             dneg.as<uint32_t>(), (uint32_t)n, (uint32_t)parts};
+  timing_begin(ctx);
+  MPVSS_CUDA(ctx, modp::launch_lagrange_boxes(LA, ctx->stream));
+  timing_launch(ctx);
+  for (size_t half = parts / 2; half >= 1; half /= 2)
+    for (DevBuf* b : {&dnum, &dden})
+      MPVSS_TRY(dev_mul(ctx, Kg, b->as<uint32_t>(), EW, b->as<uint32_t>() + half * n * EW, EW, 0, half * n,
+                        b->as<uint32_t>()));
+  MPVSS_TRY(dev_batch_inverse_g(ctx, dden.as<uint32_t>(), n, dinv.as<uint32_t>()));
+  MPVSS_TRY(dev_mul(ctx, Kg, dnum.as<uint32_t>(), EW, dinv.as<uint32_t>(), EW, 0, n, dnum.as<uint32_t>()));  // lambda
+  MPVSS_TRY(timing_end(ctx));
+  const float ms_lambda = ctx->last_ms;
+  const int launches_lambda = ctx->last_launches;
+  std::vector<uint8_t> lam(n * EB);
+  std::vector<uint32_t> negf(parts * n);
+  MPVSS_TRY(d2h(ctx, lam.data(), dnum, n * EB));
+  MPVSS_TRY(d2h(ctx, negf.data(), dneg, parts * n * 4));
+  MPVSS_TRY(sync(ctx));
+  for (size_t i = 0; i < n; ++i) {
+    for (size_t p = 1; p < parts; ++p) negf[i] ^= negf[p * n + i];
+    if (!negf[i]) continue;
+    big::Int l = big::from_le(lam.data() + i * EB, EB);
+    if (!big::is_zero(l)) big::to_le(big::sub(ctx->qm1, l), lam.data() + i * EB, EB);
+  }
+  MPVSS_TRY(h2d(ctx, dexp, lam.data(), n * EB));
+  // the direct boxes' product trees, every level planned here and uploaded at once
+  std::vector<uint32_t> rows(3 * n_direct), level_end;
+  {
+    std::vector<uint32_t> c(cnt.begin(), cnt.begin() + L_direct);
+    for (size_t m = 0, total = 0; (m = modp::product_tree_level(start.data(), c.data(), (uint32_t)L_direct,
+                                                                rows.data() + 3 * total)) > 0;) {
+      total += m;
+      level_end.push_back((uint32_t)total);
+    }
+  }
+  if (!level_end.empty()) MPVSS_TRY(h2d(ctx, dplan, rows.data(), (size_t)level_end.back() * 3 * 4));
+  timing_begin(ctx);
+  if (n_direct) {
+    MPVSS_TRY(dev_exp2(ctx, K, dshares.as<uint32_t>(), EW, dexp.as<uint32_t>(), EW, windows_for(lam.data(), EB, n_direct),
+                       nullptr, 0, nullptr, 0, 0, n_direct, dpow.as<uint32_t>()));
+    for (size_t l = 0; l < level_end.size(); ++l) {
+      const uint32_t lo = l ? level_end[l - 1] : 0;
+      modp::MulRowsArgs MA{K, dpow.as<uint32_t>(), dplan.as<uint32_t>() + 3 * lo, level_end[l] - lo};
+      MPVSS_CUDA(ctx, modp::launch_mul_rows(ctx->modp_tpi, MA, ctx->stream));
+      timing_launch(ctx);
+    }
+  }
+  for (size_t j = L_direct; j < L; ++j) {
+    DevBuf vb, ve, vo;  // views of box j's rows (not owned)
+    vb.p = dshares.as<uint32_t>() + (size_t)start[j] * EW;
+    ve.p = dexp.as<uint32_t>() + (size_t)start[j] * EW;
+    vo.p = dpow.as<uint32_t>() + (size_t)start[j] * EW;
+    const uint32_t windows = (windows_for(lam.data() + (size_t)start[j] * EB, EB, cnt[j]) + 1) / 2;
+    MPVSS_TRY(multi_exp_buckets(ctx, vb, ve, windows, cnt[j], vo));
+  }
+  MPVSS_TRY(timing_end(ctx));
+  ctx->last_ms += ms_lambda;
+  ctx->last_launches += launches_lambda;
+  MPVSS_TRY(d2h(ctx, host.data(), dpow, n * EB));
+  MPVSS_TRY(sync(ctx));
+  for (size_t j = 0; j < L; ++j) {
+    const size_t b = live[j];
+    const uint8_t* gs = host.data() + (size_t)start[j] * EB;
+    uint8_t tmp[EB], hs[32];
+    sha2::sha256(tmp, min_be(gs, tmp), hs);
+    big::Int mask = big::mod(big::from_be(hs, 32), ctx->q);  // participant.rs:512-518
+    big::to_be(big::bxor(mask, big::from_be(u + b * EB, EB)), secrets_out + b * EB, EB);
+    if (gs_out) memcpy(gs_out + b * EB, gs, EB);
+  }
+  return MPVSS_OK;
+}
+
 }  // namespace modp_api

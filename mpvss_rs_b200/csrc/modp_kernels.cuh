@@ -649,6 +649,32 @@ MP_DEV void lagrange_body(const LagrangeArgs& A, uint32_t tid) {
                    denominator ? A.negative + row : nullptr, j0 < A.k ? j0 : A.k, j1);
 }
 
+// Several boxes at once (mpvss_reconstruct_secrets): the positions of the boxes are concatenated, and position i
+// belongs to the box of k_b = bk[i] positions that starts at boff[i].  Each product runs over that box only, cut
+// into `parts` ranges of the box as lagrange_body cuts its k positions; part p of position i lands in row
+// p * n + i.
+struct LagrangeBoxesArgs {
+  const uint32_t* order;  // 64 limbs, all-ones top limb
+  const uint32_t* pos;    // n positions, concatenated over the boxes
+  const uint32_t* boff;   // per position: first position of its box
+  const uint32_t* bk;     // per position: positions k_b of its box
+  uint32_t* num;          // parts x n x 64 limbs
+  uint32_t* den;          // parts x n x 64 limbs
+  uint32_t* negative;     // parts x n flags (partial signs)
+  uint32_t n, parts;
+};
+MP_DEV void lagrange_boxes_body(const LagrangeBoxesArgs& A, uint32_t tid) {
+  const uint32_t P = A.parts ? A.parts : 1u;
+  if (tid >= 2u * P * A.n) return;
+  const bool denominator = tid >= P * A.n;
+  const uint32_t row = denominator ? tid - P * A.n : tid, part = row / A.n, i = row % A.n;
+  const uint32_t off = A.boff[i], k = A.bk[i];
+  const uint32_t per = (k + P - 1) / P, j0 = part * per, j1 = j0 + per < k ? j0 + per : k;
+  const LagrangeArgs box{A.order, A.pos + off, nullptr, nullptr, nullptr, k, P};
+  lagrange_product((denominator ? A.den : A.num) + (size_t)row * 64, box, i - off, denominator,
+                   denominator ? A.negative + row : nullptr, j0 < k ? j0 : k, j1);
+}
+
 // --------------------------------------------- bucket multi-exponentiation ----
 // prod_i S_i^(e_i) for k distinct bases and unstructured full-width exponents (the reconstruct fold,
 // participant.rs:490-509, and Group-level multi_exp): Pippenger's bucket method with 8-bit windows.
@@ -841,6 +867,63 @@ MP_DEV void mul_body(const MulArgs& A, uint32_t wg, uint32_t* wsm) {
   }
   canonical<TPI>(acc, M, ln);
   if (live) stage<TPI>(A.out + (size_t)inst * 64, acc, ln);
+}
+
+// ------------------------------------------------ gathered products (segmented tree) ----
+// v[rows[3i + 2]] = v[rows[3i]] * v[rows[3i + 1]] mod q (canonical) for n host-planned row triples.  A level of
+// product_tree_level writes each product over its first factor and no row is read by one triple and written by
+// another, so the level runs in place.
+struct MulRowsArgs {
+  const uint32_t* consts;
+  uint32_t* v;           // values, 64 limbs each
+  const uint32_t* rows;  // n x (a, b, out)
+  uint32_t n;
+};
+
+template <int TPI>
+MP_DEV void mul_rows_body(const MulRowsArgs& A, uint32_t wg, uint32_t* wsm) {
+  constexpr int L = Cfg<TPI>::L;
+  constexpr int GPW = 32 / TPI;
+  Lane ln = make_lane<TPI>();
+  const int gi = (int)simt::lane_id() / TPI;
+  uint32_t inst = wg * GPW + gi;
+  const bool live = inst < A.n;
+  if (!live) inst = A.n - 1;
+  const uint32_t* t = A.rows + (size_t)inst * 3;
+  Mod<L> M;
+  load_mod<TPI>(M, A.consts, ln);
+  uint32_t* r2 = wsm;
+  uint32_t* sq = wsm + 64 + gi * (64 + GPAD);
+  warp_copy64(r2, A.consts + C_R2);
+  simt::syncwarp();
+  uint32_t acc[L], y[L];
+  load_slice<TPI>(acc, A.v + (size_t)t[0] * 64, ln);
+  load_slice<TPI>(y, A.v + (size_t)t[1] * 64, ln);
+  mont_mul<TPI>(acc, acc, r2, M, ln);  // a*R
+  stage_shared<TPI>(sq, y, ln);
+  simt::syncwarp();
+  mont_mul<TPI>(acc, acc, sq, M, ln);  // a*R*b/R = a*b
+  canonical<TPI>(acc, M, ln);
+  if (live) stage<TPI>(A.v + (size_t)t[2] * 64, acc, ln);
+}
+
+// One level of the segmented product tree (host planning, shared with the tests): segment s holds cnt[s] values
+// from row start[s].  Its first cnt / 2 rows are multiplied by the rows h = ceil(cnt / 2) further on, in place,
+// and cnt becomes h; an odd middle row stays where it is.  Writes the level's (a, b, out) triples to `rows` and
+// returns their number (0 once every segment is down to its product, at row start[s]).
+inline uint32_t product_tree_level(const uint32_t* start, uint32_t* cnt, uint32_t segments, uint32_t* rows) {
+  uint32_t m = 0;
+  for (uint32_t s = 0; s < segments; ++s) {
+    const uint32_t c = cnt[s], h = (c + 1) / 2;
+    for (uint32_t i = 0; i < c / 2; ++i) {
+      rows[3 * m] = start[s] + i;
+      rows[3 * m + 1] = start[s] + i + h;
+      rows[3 * m + 2] = start[s] + i;
+      ++m;
+    }
+    cnt[s] = h;
+  }
+  return m;
 }
 
 // ---- split squaring, test entry (TPI = 8): out = a*a/R mod q, a taken as is ----

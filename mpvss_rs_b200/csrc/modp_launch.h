@@ -17,7 +17,9 @@ cudaError_t launch_resp(const RespArgs& A, cudaStream_t s);
 cudaError_t launch_comb_build(int tpi, const CombArgs& A, cudaStream_t s);
 cudaError_t launch_poly(const PolyArgs& A, cudaStream_t s);
 cudaError_t launch_lagrange(const LagrangeArgs& A, cudaStream_t s);
+cudaError_t launch_lagrange_boxes(const LagrangeBoxesArgs& A, cudaStream_t s);
 cudaError_t launch_mul(int tpi, const MulArgs& A, cudaStream_t s);
+cudaError_t launch_mul_rows(int tpi, const MulRowsArgs& A, cudaStream_t s);
 cudaError_t launch_msm(const MsmBucketArgs& B, const uint32_t* scalars, uint32_t* idx, uint32_t* start, uint32_t* wprod,
                        uint32_t* out, cudaStream_t s);
 }  // namespace modp

@@ -54,6 +54,8 @@ SIGNATURES = {
     "mpvss_extract_shares": (ctypes.c_int, [_ctxp, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _intp]),
     "mpvss_verify_shares": (ctypes.c_int, [_ctxp, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _intp]),
     "mpvss_reconstruct": (ctypes.c_int, [_ctxp, _sz, _i64p, _u8p, _u8p, _u8p, _u8p]),
+    "mpvss_reconstruct_secrets": (ctypes.c_int, [_ctxp, _sz, ctypes.POINTER(_sz), _i64p, _u8p, _u8p, _u8p, _u8p,
+                                                 _intp]),
     "mpvss_comm_unique_id": (ctypes.c_int, [_u8p, _sz]),
     "mpvss_comm_init": (ctypes.c_int, [_ctxp, _u8p, _sz, ctypes.c_int, ctypes.c_int]),
     "mpvss_comm_destroy": (ctypes.c_int, [_ctxp]),

@@ -6,7 +6,8 @@ tests read like the reference's own tests; every group operation goes through
 libmpvss_b200.so (CUDA).  The only additions are the randomness-injection
 arguments (`coeffs`, `witnesses`, `private_key`) -- the reference draws those from
 `thread_rng` internally (polynomial.rs:34-47, participant.rs:223, 139-146) -- and
-the batch forms `extract_secret_shares` / `verify_shares` / `verify_distributions`.
+the batch forms `extract_secret_shares` / `verify_shares` / `verify_distributions` /
+`reconstruct_secrets`.
 
 Value representation at this level: MODP elements and all scalars are Python
 ints (the reference uses BigInt); secp256k1 / ristretto255 elements are their
@@ -373,8 +374,9 @@ class Participant:
         return self.verify_shares([sharebox], box, [publickey])[0]
 
     # -- reconstruct: participant.rs:462-519 / 1452-1513 / 1895-1950 --
-    def reconstruct(self, share_boxes, box, trace=None):
-        g, c = self.group, self.group.codec
+    def _shares_by_position(self, share_boxes, box):
+        """(positions in ascending order, their shares), or None where reconstruct returns None"""
+        c = self.group.codec
         if len(share_boxes) < len(box.commitments):             # participant.rs:469
             return None
         shares = {}
@@ -384,14 +386,51 @@ class Participant:
                 return None
             shares[p] = sb.share
         pos = sorted(shares)
+        return pos, [shares[p] for p in pos]
+
+    def reconstruct(self, share_boxes, box, trace=None):
+        g, c = self.group, self.group.codec
+        flat = self._shares_by_position(share_boxes, box)
+        if flat is None:
+            return None
+        pos, ss = flat
         k = len(pos)
         sec, gs = buf(size=c.eb), buf(size=c.eb)
         g.ctx.check(g.ctx.lib.mpvss_reconstruct(
-            g.ctx.h, k, (ctypes.c_int64 * k)(*pos), ptr(buf(c.enc_elems([shares[p] for p in pos]))),
+            g.ctx.h, k, (ctypes.c_int64 * k)(*pos), ptr(buf(c.enc_elems(ss))),
             ptr(buf(box.U.to_bytes(c.eb, "big"))), ptr(sec), ptr(gs)))
         if trace is not None:
             trace["G_s"] = c.dec_elem(bytes(gs))
         return int.from_bytes(bytes(sec), "big")
+
+    def reconstruct_secrets(self, jobs, traces=None) -> list:
+        """Batch form of reconstruct: one secret (or None) per (share_boxes, box) job, all jobs in one library call
+        (mpvss_reconstruct_secrets).  A job for which reconstruct returns None, or whose box the library rejects
+        (where reconstruct would raise), is None without disturbing the others.  traces[j]["G_s"] receives G^s."""
+        g, c = self.group, self.group.codec
+        res = [None] * len(jobs)
+        live, flats = [], []
+        for j, (share_boxes, box) in enumerate(jobs):
+            flat = self._shares_by_position(share_boxes, box)
+            if flat is not None:
+                live.append(j)
+                flats.append(flat)
+        if not live:
+            return res
+        m = len(live)
+        pos = [p for f in flats for p in f[0]]
+        sec, gs, st = buf(size=m * c.eb), buf(size=m * c.eb), (ctypes.c_int * m)()
+        g.ctx.check(g.ctx.lib.mpvss_reconstruct_secrets(
+            g.ctx.h, m, (ctypes.c_size_t * m)(*[len(f[0]) for f in flats]), (ctypes.c_int64 * len(pos))(*pos),
+            ptr(buf(b"".join(c.enc_elems(f[1]) for f in flats))),
+            ptr(buf(b"".join(jobs[j][1].U.to_bytes(c.eb, "big") for j in live))), ptr(sec), ptr(gs), st))
+        for i, j in enumerate(live):
+            if st[i] != _lib.OK:
+                continue
+            res[j] = int.from_bytes(bytes(sec)[i * c.eb:(i + 1) * c.eb], "big")
+            if traces is not None:
+                traces[j]["G_s"] = c.dec_elem(bytes(gs)[i * c.eb:(i + 1) * c.eb])
+        return res
 
 
 def string_to_secret(message: str) -> int:
