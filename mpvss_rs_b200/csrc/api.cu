@@ -37,21 +37,13 @@ struct Guard {
   }
   ~Guard() { c->mu.unlock(); }
 };
-int unsupported(mpvss_ctx* ctx, const char* fn) {
-  return mpvss_fail(ctx, MPVSS_ERR_UNSUPPORTED, std::string(fn) + ": not available for this group in this build");
-}
 }  // namespace
 
-#define DISPATCH(ctx, fn, ...)                                             \
-  do {                                                                     \
-    if (!(ctx)) return MPVSS_ERR_ARG;                                      \
-    Guard _g(ctx);                                                         \
-    switch ((ctx)->group) {                                                \
-      case MPVSS_GROUP_MODP: return modp_api::fn(ctx, __VA_ARGS__);        \
-      case MPVSS_GROUP_SECP256K1: return secp_api::fn(ctx, __VA_ARGS__);   \
-      case MPVSS_GROUP_RISTRETTO255: return rist_api::fn(ctx, __VA_ARGS__); \
-      default: return unsupported(ctx, #fn);                               \
-    }                                                                      \
+#define DISPATCH(ctx, fn, ...)                 \
+  do {                                         \
+    if (!(ctx)) return MPVSS_ERR_ARG;          \
+    Guard _g(ctx);                             \
+    return (ctx)->ops->fn(ctx, __VA_ARGS__);   \
   } while (0)
 
 extern "C" {
@@ -66,7 +58,9 @@ int mpvss_ctx_create(int group, int device, mpvss_ctx** out) {
     return MPVSS_ERR_CUDA;  // no CPU fallback: the hot path exists only on the GPU
   }
   mpvss_ctx* ctx = new mpvss_ctx();
+  static const GroupOps* const ops[] = {&modp_ops, &secp_ops, &rist_ops};  // indexed by MPVSS_GROUP_*
   ctx->group = group;
+  ctx->ops = ops[group];
   ctx->device = device;
   auto bail = [&](int s) {
     mpvss_ctx_destroy(ctx);
@@ -87,10 +81,7 @@ int mpvss_ctx_create(int group, int device, mpvss_ctx** out) {
       return bail(MPVSS_ERR_CUDA);
   for (cudaEvent_t& e : ctx->ev_chunk)
     if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return bail(MPVSS_ERR_CUDA);
-  int s = MPVSS_OK;
-  if (group == MPVSS_GROUP_MODP) s = modp_api::init(ctx);
-  if (group == MPVSS_GROUP_SECP256K1) s = secp_api::init(ctx);
-  if (group == MPVSS_GROUP_RISTRETTO255) s = rist_api::init(ctx);
+  int s = ctx->ops->init(ctx);
   if (s != MPVSS_OK) return bail(s);
   *out = ctx;
   return MPVSS_OK;
@@ -106,7 +97,10 @@ void mpvss_ctx_destroy(mpvss_ctx* ctx) {
     if (b.p) cudaMemset(b.p, 0, b.cap);
   for (auto& b : ctx->pinned)
     if (b.p) memset(b.p, 0, b.cap);
-  modp_api::destroy(ctx);
+  for (DevBuf* b : {&ctx->consts_q, &ctx->consts_g, &ctx->gens, &ctx->comb[0], &ctx->comb[1], &ctx->v_comm, &ctx->v_cm, &ctx->v_pos, &ctx->v_pk,
+                    &ctx->v_y, &ctx->v_r, &ctx->v_c, &ctx->v_x, &ctx->v_a1, &ctx->v_a2, &ctx->v_slot, &ctx->v_nd, &ctx->v_ops, &ctx->v_frames, &ctx->v_gather, &ctx->v_ordered, &ctx->v_st, &ctx->v_cst, &ctx->v_first, &ctx->v_steps,
+                    &ctx->v_e, &ctx->v_h, &ctx->v_t2})
+    b->release();
   ctx->h_frames.release();
   for (cudaEvent_t e : ctx->ev_chunk)
     if (e) cudaEventDestroy(e);

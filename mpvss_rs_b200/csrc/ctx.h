@@ -52,8 +52,11 @@ struct PinBuf {
   T* as() const { return static_cast<T*>(p); }
 };
 
+struct GroupOps;
+
 struct mpvss_ctx {
   int group = 0;
+  const GroupOps* ops = nullptr;  // the group's entry points
   int device = 0;
   int sm_count = 148;  // multiprocessors of the device (read at context creation)
   cudaStream_t stream = nullptr;
@@ -153,83 +156,32 @@ void timing_begin(mpvss_ctx* ctx);
 void timing_launch(mpvss_ctx* ctx, int n = 1);
 int timing_end(mpvss_ctx* ctx);
 
-// ---- per-group implementations (modp_api.cu, secp_api.cu, rist_api.cu) ----
-namespace modp_api {
-int init(mpvss_ctx* ctx);
-void destroy(mpvss_ctx* ctx);
-int batch_exp(mpvss_ctx*, const uint8_t*, size_t, const uint8_t*, size_t, uint8_t*);
-int fixed_base_exp(mpvss_ctx*, int, const uint8_t*, size_t, uint8_t*);
-int batch_mul(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
-int poly_eval_exp(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
-int dleq_verify_commit(mpvss_ctx*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
-                       const uint8_t*, size_t, size_t, uint8_t*, uint8_t*);
-int dleq_prove_commit(mpvss_ctx*, const uint8_t*, const uint8_t*, const uint8_t*, size_t, uint8_t*, uint8_t*);
-int multi_exp(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
-int verify_stage(mpvss_ctx*, size_t, size_t, const uint8_t*, const int64_t*, const uint8_t*, const uint8_t*,
-                 const uint8_t*, const uint8_t*);
-int verify_run(mpvss_ctx*, int*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
-int verify_batch(mpvss_ctx*, size_t, const size_t*, const size_t*, const uint8_t*, const int64_t*, const uint8_t*,
-                 const uint8_t*, const uint8_t*, const uint8_t*, int*, uint8_t*);
-int scalar_poly_eval(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
-int distribute(mpvss_ctx*, size_t, size_t, const uint8_t*, size_t, const uint8_t*, const uint8_t*, const uint8_t*,
-               uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
-int extract_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*, uint8_t*,
-                   uint8_t*, int*);
-int verify_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
-                  int*);
-int reconstruct(mpvss_ctx*, size_t, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*);
-int reconstruct_batch(mpvss_ctx*, size_t, const size_t*, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*,
-                      uint8_t*, int*);
-}  // namespace modp_api
-namespace secp_api {
-int init(mpvss_ctx* ctx);
-int batch_exp(mpvss_ctx*, const uint8_t*, size_t, const uint8_t*, size_t, uint8_t*);
-int fixed_base_exp(mpvss_ctx*, int, const uint8_t*, size_t, uint8_t*);
-int batch_mul(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
-int poly_eval_exp(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
-int dleq_verify_commit(mpvss_ctx*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
-                       const uint8_t*, size_t, size_t, uint8_t*, uint8_t*);
-int dleq_prove_commit(mpvss_ctx*, const uint8_t*, const uint8_t*, const uint8_t*, size_t, uint8_t*, uint8_t*);
-int multi_exp(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
-int verify_stage(mpvss_ctx*, size_t, size_t, const uint8_t*, const int64_t*, const uint8_t*, const uint8_t*,
-                 const uint8_t*, const uint8_t*);
-int verify_run(mpvss_ctx*, int*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
-int verify_batch(mpvss_ctx*, size_t, const size_t*, const size_t*, const uint8_t*, const int64_t*, const uint8_t*,
-                 const uint8_t*, const uint8_t*, const uint8_t*, int*, uint8_t*);
-int scalar_poly_eval(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
-int distribute(mpvss_ctx*, size_t, size_t, const uint8_t*, size_t, const uint8_t*, const uint8_t*, const uint8_t*,
-               uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
-int extract_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*, uint8_t*,
-                   uint8_t*, int*);
-int verify_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
-                  int*);
-int reconstruct(mpvss_ctx*, size_t, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*);
-int reconstruct_batch(mpvss_ctx*, size_t, const size_t*, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*,
-                      uint8_t*, int*);
-}  // namespace secp_api
-namespace rist_api {
-int init(mpvss_ctx* ctx);
-int batch_exp(mpvss_ctx*, const uint8_t*, size_t, const uint8_t*, size_t, uint8_t*);
-int fixed_base_exp(mpvss_ctx*, int, const uint8_t*, size_t, uint8_t*);
-int batch_mul(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
-int poly_eval_exp(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
-int dleq_verify_commit(mpvss_ctx*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
-                       const uint8_t*, size_t, size_t, uint8_t*, uint8_t*);
-int dleq_prove_commit(mpvss_ctx*, const uint8_t*, const uint8_t*, const uint8_t*, size_t, uint8_t*, uint8_t*);
-int multi_exp(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
-int verify_stage(mpvss_ctx*, size_t, size_t, const uint8_t*, const int64_t*, const uint8_t*, const uint8_t*,
-                 const uint8_t*, const uint8_t*);
-int verify_run(mpvss_ctx*, int*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
-int verify_batch(mpvss_ctx*, size_t, const size_t*, const size_t*, const uint8_t*, const int64_t*, const uint8_t*,
-                 const uint8_t*, const uint8_t*, const uint8_t*, int*, uint8_t*);
-int scalar_poly_eval(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
-int distribute(mpvss_ctx*, size_t, size_t, const uint8_t*, size_t, const uint8_t*, const uint8_t*, const uint8_t*,
-               uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
-int extract_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*, uint8_t*,
-                   uint8_t*, int*);
-int verify_shares(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
-                  int*);
-int reconstruct(mpvss_ctx*, size_t, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*);
-int reconstruct_batch(mpvss_ctx*, size_t, const size_t*, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*,
-                      uint8_t*, int*);
-}  // namespace rist_api
+// ---- per-group implementations ----
+// One group's entry points behind the C ABI (modp_api.cu, ec_api.cu); the context holds its group's table.
+struct GroupOps {
+  int (*init)(mpvss_ctx*);
+  int (*batch_exp)(mpvss_ctx*, const uint8_t*, size_t, const uint8_t*, size_t, uint8_t*);
+  int (*fixed_base_exp)(mpvss_ctx*, int, const uint8_t*, size_t, uint8_t*);
+  int (*batch_mul)(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
+  int (*poly_eval_exp)(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
+  int (*dleq_verify_commit)(mpvss_ctx*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
+                            const uint8_t*, size_t, size_t, uint8_t*, uint8_t*);
+  int (*dleq_prove_commit)(mpvss_ctx*, const uint8_t*, const uint8_t*, const uint8_t*, size_t, uint8_t*, uint8_t*);
+  int (*multi_exp)(mpvss_ctx*, const uint8_t*, const uint8_t*, size_t, uint8_t*);
+  int (*verify_stage)(mpvss_ctx*, size_t, size_t, const uint8_t*, const int64_t*, const uint8_t*, const uint8_t*,
+                      const uint8_t*, const uint8_t*);
+  int (*verify_run)(mpvss_ctx*, int*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
+  int (*verify_batch)(mpvss_ctx*, size_t, const size_t*, const size_t*, const uint8_t*, const int64_t*, const uint8_t*,
+                      const uint8_t*, const uint8_t*, const uint8_t*, int*, uint8_t*);
+  int (*scalar_poly_eval)(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
+  int (*distribute)(mpvss_ctx*, size_t, size_t, const uint8_t*, size_t, const uint8_t*, const uint8_t*, const uint8_t*,
+                    uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
+  int (*extract_shares)(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*,
+                        uint8_t*, uint8_t*, int*);
+  int (*verify_shares)(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
+                       const uint8_t*, int*);
+  int (*reconstruct)(mpvss_ctx*, size_t, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*);
+  int (*reconstruct_batch)(mpvss_ctx*, size_t, const size_t*, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*,
+                           uint8_t*, int*);
+};
+extern const GroupOps modp_ops, secp_ops, rist_ops;

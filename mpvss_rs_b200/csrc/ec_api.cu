@@ -9,7 +9,7 @@
 //   responses r = w - alpha*c     participant.rs:1221-1231 / 1679-1688
 //   U mask                        participant.rs:1234-1260 / 1691-1703, unmask :1495-1512 / 1938-1949
 //   Lagrange sign handling        participant.rs:1518-1557 / 1955-2002
-#include "ctx.h"
+#include "host_common.h"
 #include "ec_launch.h"
 #include "hash_launch.h"
 #include "sha2.h"
@@ -19,16 +19,6 @@ namespace {
 
 constexpr size_t SB = 32;  // scalar bytes at the boundary
 
-big::Int hex_int(const char* s) {
-  size_t n = strlen(s);
-  std::vector<uint8_t> be((n + 1) / 2, 0);
-  for (size_t i = 0; i < n; ++i) {
-    char c = s[n - 1 - i];
-    uint8_t v = c <= '9' ? c - '0' : (c | 32) - 'a' + 10;
-    be[be.size() - 1 - i / 2] |= v << (4 * (i % 2));
-  }
-  return big::from_be(be.data(), be.size());
-}
 void put8(uint32_t* dst, const big::Int& v) {
   for (int i = 0; i < 8; ++i) dst[i] = i < (int)v.size() ? v[i] : 0;
 }
@@ -56,18 +46,18 @@ struct SecpTraits {
   static constexpr bool TOP_ADD_FREE = true;
   static constexpr size_t EB = 33;
   static constexpr bool SCALAR_BE = true;
-  static big::Int order() { return hex_int("fffffffffffffffffffffffffffffffebaaedce6af48a03bbfd25e8cd0364141"); }
+  static big::Int order() { return from_hex("fffffffffffffffffffffffffffffffebaaedce6af48a03bbfd25e8cd0364141"); }
   static void consts(secp::Consts& C) {
-    big::Int p = hex_int("fffffffffffffffffffffffffffffffffffffffffffffffffffffffefffffc2f");
+    big::Int p = from_hex("fffffffffffffffffffffffffffffffffffffffffffffffffffffffefffffc2f");
     fill_modulus(C.P, p);
     fill_modulus(C.N, order());
     put8(C.b7, big::from_u64(7));  // base-field constants in plain representation (fpspecial.cuh)
-    put8(C.gx, hex_int("79be667ef9dcbbac55a06295ce870b07029bfcdb2dce28d959f2815b16f81798"));
-    put8(C.gy, hex_int("483ada7726a3c4655da4fbfc0e1108a8fd17b448a68554199c47d08ffb10d4b8"));
+    put8(C.gx, from_hex("79be667ef9dcbbac55a06295ce870b07029bfcdb2dce28d959f2815b16f81798"));
+    put8(C.gy, from_hex("483ada7726a3c4655da4fbfc0e1108a8fd17b448a68554199c47d08ffb10d4b8"));
     put8(C.sqrt_e, big::shr1(big::shr1(big::add(p, big::from_u64(1)))));
   }
   static void generator(uint8_t* out) {  // secp256k1.rs:78-85 (both generators are G)
-    big::Int gx = hex_int("79be667ef9dcbbac55a06295ce870b07029bfcdb2dce28d959f2815b16f81798");
+    big::Int gx = from_hex("79be667ef9dcbbac55a06295ce870b07029bfcdb2dce28d959f2815b16f81798");
     out[0] = 2;
     big::to_be(gx, out + 1, 32);
   }
@@ -96,23 +86,23 @@ struct RistTraits {
   static constexpr bool TOP_ADD_FREE = false;
   static constexpr size_t EB = 32;
   static constexpr bool SCALAR_BE = false;
-  static big::Int order() { return hex_int("1000000000000000000000000000000014def9dea2f79cd65812631a5cf5d3ed"); }
+  static big::Int order() { return from_hex("1000000000000000000000000000000014def9dea2f79cd65812631a5cf5d3ed"); }
   static void consts(rist::Consts& C) {
-    big::Int p = hex_int("7fffffffffffffffffffffffffffffffffffffffffffffffffffffffffffffed");
+    big::Int p = from_hex("7fffffffffffffffffffffffffffffffffffffffffffffffffffffffffffffed");
     fill_modulus(C.P, p);
     fill_modulus(C.N, order());
-    put8(C.d, hex_int("52036cee2b6ffe738cc740797779e89800700a4d4141d8ab75eb4dca135978a3"));
-    put8(C.d2, hex_int("2406d9dc56dffce7198e80f2eef3d13000e0149a8283b156ebd69b9426b2f159"));
-    put8(C.sqrt_m1, hex_int("2b8324804fc1df0b2b4d00993dfbd7a72f431806ad2fe478c4ee1b274a0ea0b0"));
-    put8(C.invsqrt_a_minus_d, hex_int("786c8905cfaffca216c27b91fe01d8409d2f16175a4172be99c8fdaa805d40ea"));
-    put8(C.bx, hex_int("216936d3cd6e53fec0a4e231fdd6dc5c692cc7609525a7b2c9562d608f25d51a"));
-    put8(C.by, hex_int("6666666666666666666666666666666666666666666666666666666666666658"));
+    put8(C.d, from_hex("52036cee2b6ffe738cc740797779e89800700a4d4141d8ab75eb4dca135978a3"));
+    put8(C.d2, from_hex("2406d9dc56dffce7198e80f2eef3d13000e0149a8283b156ebd69b9426b2f159"));
+    put8(C.sqrt_m1, from_hex("2b8324804fc1df0b2b4d00993dfbd7a72f431806ad2fe478c4ee1b274a0ea0b0"));
+    put8(C.invsqrt_a_minus_d, from_hex("786c8905cfaffca216c27b91fe01d8409d2f16175a4172be99c8fdaa805d40ea"));
+    put8(C.bx, from_hex("216936d3cd6e53fec0a4e231fdd6dc5c692cc7609525a7b2c9562d608f25d51a"));
+    put8(C.by, from_hex("6666666666666666666666666666666666666666666666666666666666666658"));
     big::Int e;
     big::divmod(big::sub(p, big::from_u64(5)), big::from_u64(8), &e, nullptr);
     put8(C.pm5d8, e);
   }
   static void generator(uint8_t* out) {  // RISTRETTO_BASEPOINT_POINT, ristretto255.rs:148-155
-    big::Int g = hex_int("e2f2ae0a6abc4e71a884a961c500515f58e30b6aa582dd8db6a65945e08d2d76");  // encoding, read big-endian
+    big::Int g = from_hex("e2f2ae0a6abc4e71a884a961c500515f58e30b6aa582dd8db6a65945e08d2d76");  // encoding, read big-endian
     big::to_be(g, out, 32);
   }
   // ristretto255.rs:196-205: SHA-512, little-endian, from_bytes_mod_order_wide
@@ -129,21 +119,6 @@ struct RistTraits {
     return true;
   }
 };
-
-int h2d(mpvss_ctx* ctx, DevBuf& b, const void* src, size_t bytes) {
-  MPVSS_CUDA(ctx, b.ensure(bytes));
-  MPVSS_CUDA(ctx, cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
-  return MPVSS_OK;
-}
-int d2h(mpvss_ctx* ctx, void* dst, const DevBuf& b, size_t bytes) {
-  MPVSS_CUDA(ctx, cudaMemcpyAsync(dst, b.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  return MPVSS_OK;
-}
-int sync(mpvss_ctx* ctx) {
-  MPVSS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  return MPVSS_OK;
-}
-int bad(mpvss_ctx* ctx, bool ok, const char* what) { return ok ? MPVSS_OK : mpvss_fail(ctx, MPVSS_ERR_ARG, what); }
 
 template <class T>
 struct Ec {
@@ -317,21 +292,11 @@ struct Ec {
     ctx->horner_mul = M;
   }
 
-  static int positions_u32(mpvss_ctx* ctx, const int64_t* positions, size_t n, std::vector<uint32_t>& pos) {
-    pos.resize(n);
-    for (size_t i = 0; i < n; ++i) {
-      int64_t p = positions ? positions[i] : (int64_t)i + 1;
-      if (p < 1 || p > 0x7fffffff) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
-      pos[i] = (uint32_t)p;
-    }
-    return MPVSS_OK;
-  }
-
   // ---- batch forms of trait Group ------------------------------------------------------------
   static int batch_exp(mpvss_ctx* ctx, const uint8_t* bases, size_t base_stride, const uint8_t* scalars, size_t n,
                        uint8_t* out) {
-    MPVSS_TRY(bad(ctx, bases && scalars && out && n > 0 && (base_stride == 0 || base_stride == EB),
-                  "batch_exp: bad arguments"));
+    MPVSS_TRY(check_args(ctx, bases && scalars && out && n > 0 && (base_stride == 0 || base_stride == EB),
+                         "batch_exp: bad arguments"));
     std::vector<uint32_t> e;
     MPVSS_TRY(scalars_in(ctx, scalars, n, e));
     DevBuf &db = ctx->buf(0), &de = ctx->buf(1), &dout = ctx->buf(2), &dst = ctx->buf(3);
@@ -348,8 +313,8 @@ struct Ec {
     return sync(ctx);
   }
   static int fixed_base_exp(mpvss_ctx* ctx, int generator, const uint8_t* scalars, size_t n, uint8_t* out) {
-    MPVSS_TRY(bad(ctx, (generator == MPVSS_GEN_MAIN || generator == MPVSS_GEN_SUBGROUP) && scalars && out && n > 0,
-                  "fixed_base_exp: bad arguments"));
+    MPVSS_TRY(check_args(ctx, (generator == MPVSS_GEN_MAIN || generator == MPVSS_GEN_SUBGROUP) && scalars && out && n > 0,
+                         "fixed_base_exp: bad arguments"));
     std::vector<uint32_t> e;
     MPVSS_TRY(scalars_in(ctx, scalars, n, e));
     DevBuf &de = ctx->buf(1), &dout = ctx->buf(2);
@@ -363,7 +328,7 @@ struct Ec {
     return sync(ctx);
   }
   static int batch_mul(mpvss_ctx* ctx, const uint8_t* a, const uint8_t* b, size_t n, uint8_t* out) {
-    MPVSS_TRY(bad(ctx, a && b && out && n > 0, "batch_mul: bad arguments"));
+    MPVSS_TRY(check_args(ctx, a && b && out && n > 0, "batch_mul: bad arguments"));
     DevBuf &da = ctx->buf(0), &db = ctx->buf(1), &dout = ctx->buf(2), &dst = ctx->buf(3);
     MPVSS_TRY(h2d(ctx, da, a, n * EB));
     MPVSS_TRY(h2d(ctx, db, b, n * EB));
@@ -380,9 +345,9 @@ struct Ec {
   }
   static int poly_eval_exp(mpvss_ctx* ctx, const uint8_t* commitments, size_t t, const int64_t* positions, size_t n,
                            uint8_t* out) {
-    MPVSS_TRY(bad(ctx, commitments && out && n > 0 && t > 0, "poly_eval_exp: bad arguments"));
+    MPVSS_TRY(check_args(ctx, commitments && out && n > 0 && t > 0, "poly_eval_exp: bad arguments"));
     std::vector<uint32_t> pos;
-    MPVSS_TRY(positions_u32(ctx, positions, n, pos));
+    if (positions_u32(positions, n, pos) != n) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
     DevBuf &dc = ctx->buf(0), &dp = ctx->buf(1), &dout = ctx->buf(2);
     MPVSS_TRY(h2d(ctx, dc, commitments, t * EB));
     MPVSS_TRY(h2d(ctx, dp, pos.data(), n * 4));
@@ -401,9 +366,9 @@ struct Ec {
   static int dleq_verify_commit(mpvss_ctx* ctx, const uint8_t* g1, const uint8_t* h1, const uint8_t* g2,
                                 const uint8_t* h2, const uint8_t* r, const uint8_t* c, size_t c_stride, size_t n,
                                 uint8_t* a1, uint8_t* a2, std::vector<uint8_t>* undecodable = nullptr) {
-    MPVSS_TRY(bad(ctx, g1 && h1 && g2 && h2 && r && c && ((a1 && a2) || undecodable) && n > 0 &&
-                           (c_stride == 0 || c_stride == SB),
-                  "dleq_verify_commit: bad arguments"));
+    MPVSS_TRY(check_args(ctx, g1 && h1 && g2 && h2 && r && c && ((a1 && a2) || undecodable) && n > 0 &&
+                                  (c_stride == 0 || c_stride == SB),
+                         "dleq_verify_commit: bad arguments"));
     std::vector<uint32_t> rl, cl;
     if (undecodable) {
       undecodable->assign(n, 0);
@@ -457,7 +422,7 @@ struct Ec {
   }
   static int dleq_prove_commit(mpvss_ctx* ctx, const uint8_t* g1, const uint8_t* g2, const uint8_t* w, size_t n,
                                uint8_t* a1, uint8_t* a2) {
-    MPVSS_TRY(bad(ctx, g1 && g2 && w && a1 && a2 && n > 0, "dleq_prove_commit: bad arguments"));
+    MPVSS_TRY(check_args(ctx, g1 && g2 && w && a1 && a2 && n > 0, "dleq_prove_commit: bad arguments"));
     MPVSS_TRY(batch_exp(ctx, g1, 0, w, n, a1));
     float ms = ctx->last_ms;
     int l = ctx->last_launches;
@@ -486,7 +451,7 @@ struct Ec {
     return sync(ctx);
   }
   static int multi_exp(mpvss_ctx* ctx, const uint8_t* bases, const uint8_t* scalars, size_t n, uint8_t* out) {
-    MPVSS_TRY(bad(ctx, bases && scalars && out && n > 0, "multi_exp: bad arguments"));
+    MPVSS_TRY(check_args(ctx, bases && scalars && out && n > 0, "multi_exp: bad arguments"));
     std::vector<uint32_t> e;
     MPVSS_TRY(scalars_in(ctx, scalars, n, e));
     return multi_exp_limbs(ctx, bases, nullptr, e.data(), n, out);
@@ -494,23 +459,15 @@ struct Ec {
 
   // ---- verify_distribution_shares --------------------------------------------------------------
   static transcript::Geom geom() { return transcript::Geom{EB, false}; }
-  static const uint8_t* slice_rows(const mpvss_ctx* ctx, const uint8_t* all, size_t n_total, size_t width,
-                                   std::vector<uint8_t>& tmp) {
-    if (ctx->nranks <= 1) return all;
-    tmp.clear();
-    for (size_t i = (size_t)ctx->rank; i < n_total; i += (size_t)ctx->nranks)
-      tmp.insert(tmp.end(), all + i * width, all + (i + 1) * width);
-    return tmp.data();
-  }
   static int verify_stage(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* commitments,
                           const int64_t* positions, const uint8_t* publickeys, const uint8_t* shares,
                           const uint8_t* responses, const uint8_t* challenge) {
     ctx->v_n_total = 0;
-    MPVSS_TRY(bad(ctx, n_total > 0 && t > 0 && commitments && publickeys && shares && responses && challenge,
-                  "verify_distribution: bad arguments"));
+    MPVSS_TRY(check_args(ctx, n_total > 0 && t > 0 && commitments && publickeys && shares && responses && challenge,
+                         "verify_distribution: bad arguments"));
     // every rank checks ALL positions and scalars, so that a malformed box is rejected by all ranks alike
     std::vector<uint32_t> pos_all, rl_all, cl;
-    if (positions_u32(ctx, positions, n_total, pos_all) != MPVSS_OK)   // box content: verifies as false
+    if (positions_u32(positions, n_total, pos_all) != n_total)   // box content: verifies as false
       return mpvss_fail(ctx, MPVSS_ERR_ENCODING, "verify_distribution: position out of range [1, 2^31)");
     MPVSS_TRY(scalars_in(ctx, responses, n_total, rl_all));
     MPVSS_TRY(scalars_in(ctx, challenge, 1, cl));
@@ -605,9 +562,9 @@ struct Ec {
   }
   static int verify_run(mpvss_ctx* ctx, int* ok, uint8_t* x_out, uint8_t* a1_out, uint8_t* a2_out,
                         uint8_t* digest_out) {
-    MPVSS_TRY(bad(ctx, ok && ctx->v_n_total > 0, "verify_distribution_run: nothing staged"));
-    MPVSS_TRY(bad(ctx, ctx->nranks <= 1 || (!x_out && !a1_out && !a2_out),
-                  "verify_distribution: x/a1/a2 outputs are not available with a communicator"));
+    MPVSS_TRY(check_args(ctx, ok && ctx->v_n_total > 0, "verify_distribution_run: nothing staged"));
+    MPVSS_TRY(check_args(ctx, ctx->nranks <= 1 || (!x_out && !a1_out && !a2_out),
+                         "verify_distribution: x/a1/a2 outputs are not available with a communicator"));
     const size_t n = ctx->v_n, n_total = ctx->v_n_total;
     bool decoded = true;
     MPVSS_TRY(verify_kernels(ctx, &decoded));
@@ -660,18 +617,17 @@ struct Ec {
     const size_t N = noff[nb], Tt = toff[nb];
     std::vector<uint8_t> live(nb, 1);
     // a rejected box is only false: these checks record no context error, the call succeeds
-    std::vector<uint32_t> pos(N, 1), coff(N), ct(N), rl(N * 8, 0), cl(N * 8, 0), br, bc;
+    std::vector<uint32_t> pos(N, 1), coff(N), ct(N), rl(N * 8, 0), cl(N * 8, 0), bp, br, bc;
     for (size_t b = 0; b < nb; ++b) {
-      for (size_t i = noff[b]; positions && i < noff[b + 1] && live[b]; ++i)
-        live[b] = positions[i] >= 1 && positions[i] <= 0x7fffffff;
-      if (!live[b] || scalars_in(ctx, responses + noff[b] * SB, nv[b], br, false) != MPVSS_OK ||
+      if (positions_u32(positions ? positions + noff[b] : nullptr, nv[b], bp) != nv[b] ||
+          scalars_in(ctx, responses + noff[b] * SB, nv[b], br, false) != MPVSS_OK ||
           scalars_in(ctx, challenges + b * SB, 1, bc, false) != MPVSS_OK)
         live[b] = 0;
       for (size_t j = 0, i = noff[b]; j < nv[b]; ++j, ++i) {
         coff[i] = (uint32_t)toff[b];
         ct[i] = (uint32_t)tv[b];
         if (!live[b]) continue;
-        pos[i] = positions ? (uint32_t)positions[i] : (uint32_t)(j + 1);
+        pos[i] = bp[j];
         memcpy(&rl[i * 8], &br[j * 8], 32);
         memcpy(&cl[i * 8], bc.data(), 32);
       }
@@ -757,10 +713,10 @@ struct Ec {
 
   static int scalar_poly_eval(mpvss_ctx* ctx, const uint8_t* coeffs, size_t t, const int64_t* positions, size_t n,
                               uint8_t* out) {
-    MPVSS_TRY(bad(ctx, coeffs && out && n > 0 && t > 0, "scalar_poly_eval: bad arguments"));
+    MPVSS_TRY(check_args(ctx, coeffs && out && n > 0 && t > 0, "scalar_poly_eval: bad arguments"));
     std::vector<uint32_t> co, pos, p(n * 8);
     MPVSS_TRY(scalars_in(ctx, coeffs, t, co));
-    MPVSS_TRY(positions_u32(ctx, positions, n, pos));
+    if (positions_u32(positions, n, pos) != n) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
     DevBuf &dco = ctx->buf(0), &dp = ctx->buf(1), &dpos = ctx->buf(9);
     MPVSS_TRY(h2d(ctx, dco, co.data(), t * 32));
     MPVSS_TRY(h2d(ctx, dpos, pos.data(), n * 4));
@@ -789,9 +745,9 @@ struct Ec {
                         const uint8_t* coeffs, const uint8_t* witnesses, const uint8_t* publickeys,
                         uint8_t* commitments_out, uint8_t* shares_out, uint8_t* challenge_out, uint8_t* responses_out,
                         uint8_t* u_out, uint8_t* x_out) {
-    MPVSS_TRY(bad(ctx, n_total > 0 && t > 0 && t <= n_total && secret && coeffs && witnesses && publickeys &&
-                           commitments_out && shares_out && challenge_out && responses_out && u_out && secret_len <= EB,
-                  "distribute: bad arguments (threshold <= n, participant.rs:1100; secret at most one element long)"));
+    MPVSS_TRY(check_args(ctx, n_total > 0 && t > 0 && t <= n_total && secret && coeffs && witnesses && publickeys &&
+                                  commitments_out && shares_out && challenge_out && responses_out && u_out && secret_len <= EB,
+                         "distribute: bad arguments (threshold <= n, participant.rs:1100; secret at most one element long)"));
     std::vector<uint32_t> co, wl_all;
     MPVSS_TRY(scalars_in(ctx, coeffs, t, co));
     MPVSS_TRY(scalars_in(ctx, witnesses, n_total, wl_all));   // every rank checks all of them alike
@@ -925,9 +881,9 @@ struct Ec {
   static int extract_shares(mpvss_ctx* ctx, size_t n, const uint8_t* private_keys, const uint8_t* witnesses,
                             const uint8_t* enc_shares, uint8_t* publickeys_out, uint8_t* shares_out,
                             uint8_t* challenges_out, uint8_t* responses_out, int* status_out) {
-    MPVSS_TRY(bad(ctx, n > 0 && private_keys && witnesses && enc_shares && publickeys_out && shares_out &&
-                           challenges_out && responses_out,
-                  "extract_shares: bad arguments"));
+    MPVSS_TRY(check_args(ctx, n > 0 && private_keys && witnesses && enc_shares && publickeys_out && shares_out &&
+                                  challenges_out && responses_out,
+                         "extract_shares: bad arguments"));
     std::vector<uint32_t> sk, wl;
     MPVSS_TRY(scalars_in(ctx, private_keys, n, sk));
     MPVSS_TRY(scalars_in(ctx, witnesses, n, wl));
@@ -978,8 +934,8 @@ struct Ec {
   static int verify_shares(mpvss_ctx* ctx, size_t n, const uint8_t* publickeys, const uint8_t* shares,
                            const uint8_t* enc_shares, const uint8_t* challenges, const uint8_t* responses,
                            int* ok_out) {
-    MPVSS_TRY(bad(ctx, n > 0 && publickeys && shares && enc_shares && challenges && responses && ok_out,
-                  "verify_shares: bad arguments"));
+    MPVSS_TRY(check_args(ctx, n > 0 && publickeys && shares && enc_shares && challenges && responses && ok_out,
+                         "verify_shares: bad arguments"));
     std::vector<uint8_t> undecodable;
     // a1 = G^r pk^c, a2 = S^r Y^c stay on the device (a1 / a2 == nullptr): buf(1) = pk, buf(3) = Y, buf(6) = a1,
     // buf(7) = a2 afterwards; the per-share transcript is hashed and compared there (SURVEY 8 f1)
@@ -1001,9 +957,9 @@ struct Ec {
 
   static int reconstruct(mpvss_ctx* ctx, size_t k, const int64_t* positions, const uint8_t* shares, const uint8_t* u,
                          uint8_t* secret_out, uint8_t* gs_out) {
-    MPVSS_TRY(bad(ctx, k > 0 && positions && shares && u && secret_out, "reconstruct: bad arguments"));
+    MPVSS_TRY(check_args(ctx, k > 0 && positions && shares && u && secret_out, "reconstruct: bad arguments"));
     std::vector<uint32_t> pos;
-    MPVSS_TRY(positions_u32(ctx, positions, k, pos));
+    if (positions_u32(positions, k, pos) != k) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
     DevBuf &dpos = ctx->buf(10), &dlam = ctx->buf(11);
     MPVSS_TRY(h2d(ctx, dpos, pos.data(), k * 4));
     MPVSS_CUDA(ctx, dlam.ensure(k * 32));
@@ -1035,33 +991,16 @@ struct Ec {
     if (gs_out) memset(gs_out, 0, nb * EB);
     ctx->last_ms = 0.f;
     ctx->last_launches = 0;
-    std::vector<size_t> live, first(nb);  // boxes whose positions are in range; each box's first share
+    std::vector<size_t> live;  // boxes whose positions are in range
+    std::vector<uint32_t> pos;
     for (size_t b = 0, off = 0; b < nb; off += kv[b], ++b) {
-      first[b] = off;
-      status_out[b] = MPVSS_OK;
-      for (size_t i = off; i < off + kv[b]; ++i)
-        if (positions[i] < 1 || positions[i] > 0x7fffffff) status_out[b] = MPVSS_ERR_ARG;
+      status_out[b] = positions_u32(positions + off, kv[b], pos) == kv[b] ? MPVSS_OK : MPVSS_ERR_ARG;
       if (status_out[b] == MPVSS_OK) live.push_back(b);
     }
     if (live.empty()) return MPVSS_OK;
-    const size_t L = live.size();
-    size_t n = 0;
-    std::vector<uint32_t> start(L), cnt(L);
-    for (size_t j = 0; j < L; ++j) {
-      start[j] = (uint32_t)n;
-      cnt[j] = (uint32_t)kv[live[j]];
-      n += cnt[j];
-    }
-    std::vector<uint32_t> idx(3 * n);  // positions, then per position its box's first row, then its box's k
-    std::vector<uint8_t> host(n * EB);
-    for (size_t j = 0; j < L; ++j) {
-      for (uint32_t i = 0; i < cnt[j]; ++i) {
-        idx[start[j] + i] = (uint32_t)positions[first[live[j]] + i];
-        idx[n + start[j] + i] = start[j];
-        idx[2 * n + start[j] + i] = cnt[j];
-      }
-      memcpy(host.data() + (size_t)start[j] * EB, shares + first[live[j]] * EB, cnt[j] * EB);
-    }
+    const LiveBoxes B = pack_live_boxes(nb, kv, positions, shares, EB, live);
+    const size_t L = live.size(), n = B.n;
+    const std::vector<uint32_t> &start = B.start, &cnt = B.cnt;
     // every level of the segmented sum, planned here and uploaded at once
     std::vector<uint32_t> seg, level_end;
     {
@@ -1078,8 +1017,8 @@ struct Ec {
     }
     DevBuf &dsh = ctx->buf(0), &didx = ctx->buf(1), &dlam = ctx->buf(2), &dj = ctx->buf(3), &dst = ctx->buf(4),
            &dseg = ctx->buf(5), &dtmp = ctx->buf(6), &dout = ctx->buf(7);
-    MPVSS_TRY(h2d(ctx, dsh, host.data(), n * EB));
-    MPVSS_TRY(h2d(ctx, didx, idx.data(), 3 * n * 4));
+    MPVSS_TRY(h2d(ctx, dsh, B.shares.data(), n * EB));
+    MPVSS_TRY(h2d(ctx, didx, B.idx.data(), 3 * n * 4));
     MPVSS_TRY(h2d(ctx, dseg, seg.data(), seg.size() * 4));
     const size_t g1 = level_end[0];  // the first level has the most groups
     MPVSS_CUDA(ctx, dlam.ensure(n * 32));
@@ -1128,69 +1067,34 @@ struct Ec {
   }
 };
 
+template <class T>
+GroupOps ec_ops() {
+  using E = Ec<T>;
+  GroupOps o{};
+  o.init = E::init;
+  o.batch_exp = E::batch_exp;
+  o.fixed_base_exp = E::fixed_base_exp;
+  o.batch_mul = E::batch_mul;
+  o.poly_eval_exp = E::poly_eval_exp;
+  o.dleq_verify_commit = [](mpvss_ctx* c, const uint8_t* g1, const uint8_t* h1, const uint8_t* g2, const uint8_t* h2,
+                            const uint8_t* r, const uint8_t* ch, size_t cs, size_t n, uint8_t* a1, uint8_t* a2) {
+    return E::dleq_verify_commit(c, g1, h1, g2, h2, r, ch, cs, n, a1, a2);  // the ABI form: no undecodable flags
+  };
+  o.dleq_prove_commit = E::dleq_prove_commit;
+  o.multi_exp = E::multi_exp;
+  o.verify_stage = E::verify_stage;
+  o.verify_run = E::verify_run;
+  o.verify_batch = E::verify_batch;
+  o.scalar_poly_eval = E::scalar_poly_eval;
+  o.distribute = E::distribute;
+  o.extract_shares = E::extract_shares;
+  o.verify_shares = E::verify_shares;
+  o.reconstruct = E::reconstruct;
+  o.reconstruct_batch = E::reconstruct_batch;
+  return o;
+}
+
 }  // namespace
 
-#define EC_API_NAMESPACE(ns, Traits)                                                                                 \
-  namespace ns {                                                                                                     \
-  int init(mpvss_ctx* c) { return Ec<Traits>::init(c); }                                                             \
-  int batch_exp(mpvss_ctx* c, const uint8_t* b, size_t bs, const uint8_t* s, size_t n, uint8_t* o) {                 \
-    return Ec<Traits>::batch_exp(c, b, bs, s, n, o);                                                                 \
-  }                                                                                                                  \
-  int fixed_base_exp(mpvss_ctx* c, int g, const uint8_t* s, size_t n, uint8_t* o) {                                  \
-    return Ec<Traits>::fixed_base_exp(c, g, s, n, o);                                                                \
-  }                                                                                                                  \
-  int batch_mul(mpvss_ctx* c, const uint8_t* a, const uint8_t* b, size_t n, uint8_t* o) {                            \
-    return Ec<Traits>::batch_mul(c, a, b, n, o);                                                                     \
-  }                                                                                                                  \
-  int poly_eval_exp(mpvss_ctx* c, const uint8_t* cm, size_t t, const int64_t* p, size_t n, uint8_t* o) {             \
-    return Ec<Traits>::poly_eval_exp(c, cm, t, p, n, o);                                                             \
-  }                                                                                                                  \
-  int dleq_verify_commit(mpvss_ctx* c, const uint8_t* g1, const uint8_t* h1, const uint8_t* g2, const uint8_t* h2,   \
-                         const uint8_t* r, const uint8_t* ch, size_t cs, size_t n, uint8_t* a1, uint8_t* a2) {       \
-    return Ec<Traits>::dleq_verify_commit(c, g1, h1, g2, h2, r, ch, cs, n, a1, a2);                                  \
-  }                                                                                                                  \
-  int dleq_prove_commit(mpvss_ctx* c, const uint8_t* g1, const uint8_t* g2, const uint8_t* w, size_t n, uint8_t* a1, \
-                        uint8_t* a2) {                                                                               \
-    return Ec<Traits>::dleq_prove_commit(c, g1, g2, w, n, a1, a2);                                                   \
-  }                                                                                                                  \
-  int multi_exp(mpvss_ctx* c, const uint8_t* b, const uint8_t* s, size_t n, uint8_t* o) {                            \
-    return Ec<Traits>::multi_exp(c, b, s, n, o);                                                                     \
-  }                                                                                                                  \
-  int verify_stage(mpvss_ctx* c, size_t n, size_t t, const uint8_t* cm, const int64_t* p, const uint8_t* pk,         \
-                   const uint8_t* y, const uint8_t* r, const uint8_t* ch) {                                          \
-    return Ec<Traits>::verify_stage(c, n, t, cm, p, pk, y, r, ch);                                                   \
-  }                                                                                                                  \
-  int verify_run(mpvss_ctx* c, int* ok, uint8_t* x, uint8_t* a1, uint8_t* a2, uint8_t* d) {                          \
-    return Ec<Traits>::verify_run(c, ok, x, a1, a2, d);                                                              \
-  }                                                                                                                  \
-  int verify_batch(mpvss_ctx* c, size_t nb, const size_t* n, const size_t* t, const uint8_t* cm, const int64_t* p,   \
-                   const uint8_t* pk, const uint8_t* y, const uint8_t* r, const uint8_t* ch, int* ok, uint8_t* d) {  \
-    return Ec<Traits>::verify_batch(c, nb, n, t, cm, p, pk, y, r, ch, ok, d);                                        \
-  }                                                                                                                  \
-  int scalar_poly_eval(mpvss_ctx* c, const uint8_t* co, size_t t, const int64_t* p, size_t n, uint8_t* o) {        \
-    return Ec<Traits>::scalar_poly_eval(c, co, t, p, n, o);                                                          \
-  }                                                                                                                  \
-  int distribute(mpvss_ctx* c, size_t n, size_t t, const uint8_t* s, size_t sl, const uint8_t* co, const uint8_t* w, \
-                 const uint8_t* pk, uint8_t* cm, uint8_t* sh, uint8_t* ch, uint8_t* r, uint8_t* u, uint8_t* x) {     \
-    return Ec<Traits>::distribute(c, n, t, s, sl, co, w, pk, cm, sh, ch, r, u, x);                                   \
-  }                                                                                                                  \
-  int extract_shares(mpvss_ctx* c, size_t n, const uint8_t* sk, const uint8_t* w, const uint8_t* y, uint8_t* pk,     \
-                     uint8_t* s, uint8_t* ch, uint8_t* r, int* st) {                                                 \
-    return Ec<Traits>::extract_shares(c, n, sk, w, y, pk, s, ch, r, st);                                             \
-  }                                                                                                                  \
-  int verify_shares(mpvss_ctx* c, size_t n, const uint8_t* pk, const uint8_t* s, const uint8_t* y,                   \
-                    const uint8_t* ch, const uint8_t* r, int* ok) {                                                  \
-    return Ec<Traits>::verify_shares(c, n, pk, s, y, ch, r, ok);                                                     \
-  }                                                                                                                  \
-  int reconstruct(mpvss_ctx* c, size_t k, const int64_t* p, const uint8_t* s, const uint8_t* u, uint8_t* o,          \
-                  uint8_t* gs) {                                                                                     \
-    return Ec<Traits>::reconstruct(c, k, p, s, u, o, gs);                                                            \
-  }                                                                                                                  \
-  int reconstruct_batch(mpvss_ctx* c, size_t nb, const size_t* k, const int64_t* p, const uint8_t* s,              \
-                        const uint8_t* u, uint8_t* o, uint8_t* gs, int* st) {                                        \
-    return Ec<Traits>::reconstruct_batch(c, nb, k, p, s, u, o, gs, st);                                              \
-  }                                                                                                                  \
-  }
-
-EC_API_NAMESPACE(secp_api, SecpTraits)
-EC_API_NAMESPACE(rist_api, RistTraits)
+const GroupOps secp_ops = ec_ops<SecpTraits>();
+const GroupOps rist_ops = ec_ops<RistTraits>();

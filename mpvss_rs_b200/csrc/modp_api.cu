@@ -11,7 +11,7 @@
 //   Lagrange exponents            participant.rs:526-561, util.rs:47-64
 #include <algorithm>
 #include <cstdlib>
-#include "ctx.h"
+#include "host_common.h"
 #include "modp_chain.h"
 #include "modp_launch.h"
 #include "sha2.h"
@@ -32,17 +32,6 @@ const char* RFC3526_2048 =
     "9ed529077096966d670c354e4abc9804f1746c08ca18217c32905e462e36ce3b"
     "e39e772c180e86039b2783a2ec07a28fb5c55df06f4c52c9de2bcbf695581718"
     "3995497cea956ae515d2261898fa051015728e5a8aacaa68ffffffffffffffff";
-
-big::Int from_hex(const char* s) {
-  size_t n = strlen(s);
-  std::vector<uint8_t> be((n + 1) / 2, 0);
-  for (size_t i = 0; i < n; ++i) {
-    char c = s[n - 1 - i];
-    uint8_t v = c <= '9' ? c - '0' : (c | 32) - 'a' + 10;
-    be[be.size() - 1 - i / 2] |= v << (4 * (i % 2));
-  }
-  return big::from_be(be.data(), be.size());
-}
 
 void fill_consts(const big::Int& m, uint32_t* blk) {
   memset(blk, 0, modp::C_WORDS * 4);
@@ -70,6 +59,18 @@ size_t min_be(const uint8_t* le, uint8_t* out) {
   for (size_t i = 0; i < len; ++i) out[i] = le[len - 1 - i];
   return len;
 }
+// U mask of G^s (256-byte LE): int_be(SHA-256(minimal BE bytes)) mod q  (participant.rs:269-272, 512-518)
+big::Int u_mask(const mpvss_ctx* ctx, const uint8_t* gs) {
+  uint8_t tmp[EB], hs[32];
+  sha2::sha256(tmp, min_be(gs, tmp), hs);
+  return big::mod(big::from_be(hs, 32), ctx->q);
+}
+// the order q-1 as EW little-endian limbs (the scalar kernels' modulus)
+std::vector<uint32_t> order_limbs(const mpvss_ctx* ctx) {
+  std::vector<uint32_t> order(EW, 0);
+  for (size_t i = 0; i < ctx->qm1.size(); ++i) order[i] = ctx->qm1[i];
+  return order;
+}
 void framed_update(sha2::Sha256& h, const uint8_t* le) {  // dleq.rs:58-61
   uint8_t tmp[EB], len8[8] = {0};
   size_t len = min_be(le, tmp);
@@ -96,20 +97,6 @@ uint32_t windows_for(const uint8_t* scalars, size_t stride, size_t n) {
   }
   uint32_t w = (uint32_t)(top * 2);
   return w ? w : 1;
-}
-
-int h2d(mpvss_ctx* ctx, DevBuf& b, const void* src, size_t bytes) {
-  MPVSS_CUDA(ctx, b.ensure(bytes));
-  MPVSS_CUDA(ctx, cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
-  return MPVSS_OK;
-}
-int d2h(mpvss_ctx* ctx, void* dst, const DevBuf& b, size_t bytes) {
-  MPVSS_CUDA(ctx, cudaMemcpyAsync(dst, b.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  return MPVSS_OK;
-}
-int sync(mpvss_ctx* ctx) {
-  MPVSS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  return MPVSS_OK;
 }
 
 // device-pointer exponentiation:  out = b1^e1 [* b2^e2]
@@ -147,11 +134,6 @@ int comb_table(mpvss_ctx* ctx, int which, const uint32_t** out) {
   return MPVSS_OK;
 }
 
-int check_args(mpvss_ctx* ctx, bool ok, const char* what) {
-  if (!ok) return mpvss_fail(ctx, MPVSS_ERR_ARG, what);
-  return MPVSS_OK;
-}
-
 }  // namespace
 
 namespace modp_api {
@@ -172,13 +154,6 @@ int init(mpvss_ctx* ctx) {
   gens[128] = 1;  // the scalar / element 1
   MPVSS_TRY(h2d(ctx, ctx->gens, gens.data(), gens.size() * 4));
   return sync(ctx);
-}
-
-void destroy(mpvss_ctx* ctx) {
-  for (DevBuf* b : {&ctx->consts_q, &ctx->consts_g, &ctx->gens, &ctx->comb[0], &ctx->comb[1], &ctx->v_comm, &ctx->v_cm, &ctx->v_pos, &ctx->v_pk,
-                    &ctx->v_y, &ctx->v_r, &ctx->v_c, &ctx->v_x, &ctx->v_a1, &ctx->v_a2, &ctx->v_slot, &ctx->v_nd, &ctx->v_ops, &ctx->v_frames, &ctx->v_gather, &ctx->v_ordered, &ctx->v_st, &ctx->v_cst, &ctx->v_first, &ctx->v_steps,
-                    &ctx->v_e, &ctx->v_h, &ctx->v_t2})
-    b->release();
 }
 
 int batch_exp(mpvss_ctx* ctx, const uint8_t* bases, size_t base_stride, const uint8_t* scalars, size_t n,
@@ -305,15 +280,13 @@ struct PlanBox {
 // not implemented (its chunk exponents and combination would have to follow each box's rows).
 static int prep_boxes(mpvss_ctx* ctx, const PlanBox* boxes, size_t nb, bool chunked, PosPlan& plan) {
   static_assert(modp_chain::SLOTS == modp::HC_SLOTS && modp_chain::OPS_MAX == modp::HC_OPS, "kernel / host op format");
-  auto position = [&](const PlanBox& bx, size_t i) { return bx.positions ? bx.positions[i] : (int64_t)i + 1; };
+  std::vector<std::vector<uint32_t>> pos(nb);
   uint32_t maxp = 1;
   size_t n_all = 0;
   for (size_t b = 0; b < nb; ++b) {
-    for (size_t i = 0; i < boxes[b].n; ++i) {
-      int64_t p = position(boxes[b], i);
-      if (p < 1 || p > 0x7fffffff) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
-      maxp = std::max<uint32_t>(maxp, (uint32_t)p);
-    }
+    if (positions_u32(boxes[b].positions, boxes[b].n, pos[b]) != boxes[b].n)
+      return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
+    for (uint32_t p : pos[b]) maxp = std::max(maxp, p);
     n_all += boxes[b].n;
   }
   std::lock_guard<std::mutex> lk(g_tree_mu);
@@ -323,7 +296,7 @@ static int prep_boxes(mpvss_ctx* ctx, const PlanBox* boxes, size_t nb, bool chun
   std::vector<uint32_t> sq(n_all), ml(n_all);
   for (size_t b = 0, g = 0; b < nb; ++b)
     for (size_t i = 0; i < boxes[b].n; ++i, ++g) {  // g: instance index over all boxes
-      if (!modp_chain::step_ops((uint32_t)position(boxes[b], i), g_tree, ops[g], &sq[g], &ml[g]))
+      if (!modp_chain::step_ops(pos[b][i], g_tree, ops[g], &sq[g], &ml[g]))
         return mpvss_fail(ctx, MPVSS_ERR_UNSUPPORTED, "no addition chain within the kernel's slot budget");
       by[b][ops[g].size()].push_back((uint32_t)g);
     }
@@ -599,13 +572,9 @@ int multi_exp(mpvss_ctx* ctx, const uint8_t* bases, const uint8_t* scalars, size
 // P(i) mod (q-1) for the given positions (polynomial.rs:50-58 reduced as participant.rs:202 does)
 int scalar_poly_eval(mpvss_ctx* ctx, const uint8_t* coeffs, size_t t, const int64_t* positions, size_t n, uint8_t* out) {
   MPVSS_TRY(check_args(ctx, coeffs && out && n > 0 && t > 0, "scalar_poly_eval: bad arguments"));
-  std::vector<uint32_t> order(EW, 0), pos(n);
-  for (size_t i = 0; i < ctx->qm1.size(); ++i) order[i] = ctx->qm1[i];
-  for (size_t i = 0; i < n; ++i) {
-    int64_t p = positions ? positions[i] : (int64_t)i + 1;
-    if (p < 1 || p > 0x7fffffff) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
-    pos[i] = (uint32_t)p;
-  }
+  const std::vector<uint32_t> order = order_limbs(ctx);
+  std::vector<uint32_t> pos;
+  if (positions_u32(positions, n, pos) != n) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
   // the kernel wants coefficients below 2^2048 and reduces lazily; bring them below the order first
   std::vector<uint8_t> co(t * EB);
   for (size_t j = 0; j < t; ++j) big::to_le(big::mod(big::from_le(coeffs + j * EB, EB), ctx->qm1), co.data() + j * EB, EB);
@@ -652,31 +621,18 @@ static int validate_elements(mpvss_ctx* ctx, const uint32_t* dev, size_t count, 
 // ------------------------------------------------------------------- verify ----
 static const transcript::Geom GEOM{EB, true};
 
-// rows `rank, rank + nranks, ...` of a host array of n_total rows (the whole array without a communicator)
-static const uint8_t* slice_rows(const mpvss_ctx* ctx, const uint8_t* all, size_t n_total, size_t width,
-                                 std::vector<uint8_t>& tmp) {
-  if (ctx->nranks <= 1) return all;
-  tmp.clear();
-  for (size_t i = (size_t)ctx->rank; i < n_total; i += (size_t)ctx->nranks)
-    tmp.insert(tmp.end(), all + i * width, all + (i + 1) * width);
-  return tmp.data();
-}
-
 int verify_stage(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* commitments, const int64_t* positions,
                  const uint8_t* publickeys, const uint8_t* shares, const uint8_t* responses, const uint8_t* challenge) {
   ctx->v_n_total = 0;
   MPVSS_TRY(check_args(ctx, n_total > 0 && t > 0 && commitments && publickeys && shares && responses && challenge,
                        "verify_distribution: bad arguments"));
+  std::vector<uint32_t> pos_all;
+  if (positions_u32(positions, n_total, pos_all) != n_total)  // box content, checked alike by every rank: verifies as false
+    return mpvss_fail(ctx, MPVSS_ERR_ENCODING, "verify_distribution: position out of range [1, 2^31)");
   // this rank's participants: rank, rank + N, ... (every rank gets the same mix of short and long chains)
   const size_t n = transcript::local_count(n_total, ctx->nranks, ctx->rank);
   std::vector<int64_t> pos(n);
-  for (size_t j = 0; j < n; ++j) {
-    const size_t i = (size_t)ctx->rank + j * (size_t)ctx->nranks;
-    pos[j] = positions ? positions[i] : (int64_t)i + 1;
-  }
-  for (size_t i = 0; i < n_total; ++i)   // box content, checked alike by every rank: verifies as false
-    if (positions && (positions[i] < 1 || positions[i] > 0x7fffffff))
-      return mpvss_fail(ctx, MPVSS_ERR_ENCODING, "verify_distribution: position out of range [1, 2^31)");
+  for (size_t j = 0; j < n; ++j) pos[j] = pos_all[(size_t)ctx->rank + j * (size_t)ctx->nranks];
   // The plan depends on the positions and t only: a context that verifies boxes of the same shape again (the
   // usual case: positions 1..n) keeps the plan and its device copy from the previous call.
   PosPlan plan;
@@ -770,17 +726,21 @@ static int a2_placement(const mpvss_ctx* ctx, size_t n, double horner, size_t np
   return overlap;
 }
 
-// kernels of the staged verification: X (Horner), a1 = g^r * X^c, a2 = y^r * Y^c, then the framed rows
-static int verify_kernels(mpvss_ctx* ctx) {
-  const size_t n = ctx->v_n, t = ctx->v_t;
+// Device buffers of one verification pass over t commitments and n instances.
+struct VerifyBufs {
+  DevBuf &comm, &pk, &y, &r, &c;  // inputs: commitments, public keys, shares, responses, challenge(s)
+  DevBuf &cm, &h, &t2;            // dev_horner's working buffers
+  DevBuf &x, &a1, &a2, &frames;   // outputs: X, a1, a2, framed rows
+};
+
+// One DLEQ pass of the verify calls: X (Horner), a1 = g^r * X^c, a2 = y^r * Y^c, then the framed rows.  `cs` is the
+// challenge stride in limbs (0: one challenge for all instances), `horner` the products of the longest Horner chain
+// (a2_placement).  ev_mid marks the end of the X phase.  bad gets t + 2 n flags, set by validate_elements for the
+// commitments, public keys and shares when the "validate" tunable is on.
+static int verify_pass(mpvss_ctx* ctx, const PlanDev& P, const VerifyBufs& B, size_t t, size_t n, uint32_t cs,
+                       uint32_t rwin, uint32_t cwin, double horner, const uint32_t* comb, std::vector<uint8_t>& bad) {
   const uint32_t* K = ctx->consts_q.as<uint32_t>();
-  uint32_t* X = ctx->v_x.as<uint32_t>();
-  timing_begin(ctx);
-  if (n == 0) {  // more ranks than participants: this rank only takes part in the all-gather
-    MPVSS_TRY(timing_end(ctx));
-    ctx->phase_ms[0] = ctx->phase_ms[1] = ctx->phase_ms[2] = 0.f;
-    return MPVSS_OK;
-  }
+  uint32_t* X = B.x.as<uint32_t>();
   // a2 = y^r * Y^c does not depend on X.  The Horner launch puts 7 one-warp CTAs on the 4 schedulers
   // of an SM, i.e. one warp slot per SM stays empty for the whole launch.  modp_overlap = 3 (default)
   // issues a2 on a side stream right AFTER the Horner launch as persistent one-warp CTAs, one per SM:
@@ -790,18 +750,14 @@ static int verify_kernels(mpvss_ctx* ctx) {
   // claim SMs and unbalances the placement of the long-running Horner CTAs (40 % slower): no mode 1.
   MPVSS_CUDA(ctx, cudaEventRecord(ctx->ev_fork, ctx->stream));
   auto launch_a2 = [&](cudaStream_t s) {
-    return dev_exp2(ctx, K, ctx->v_pk.as<uint32_t>(), EW, ctx->v_r.as<uint32_t>(), EW, ctx->v_rwin,
-                    ctx->v_y.as<uint32_t>(), EW, ctx->v_c.as<uint32_t>(), 0, ctx->v_cwin, n,
-                    ctx->v_a2.as<uint32_t>(), s);
+    return dev_exp2(ctx, K, B.pk.as<uint32_t>(), EW, B.r.as<uint32_t>(), EW, rwin, B.y.as<uint32_t>(), EW,
+                    B.c.as<uint32_t>(), cs, cwin, n, B.a2.as<uint32_t>(), s);
   };
-  const int overlap = a2_placement(ctx, n, (double)(t > 1 ? t - 1 : 0) / (double)ctx->v_k * (double)ctx->v_nops_max,
-                                   ctx->v_np, ctx->v_tpi, ctx->v_rwin, ctx->v_cwin);
+  const int overlap = a2_placement(ctx, n, horner, P.n_padded, P.tpi, rwin, cwin);
   const bool side = overlap == 2 || overlap == 3;
   if (!side) MPVSS_TRY(launch_a2(ctx->stream));
   // X_i from the commitments (participant.rs:423-434)
-  PlanDev P{ctx->v_ops.as<uint16_t>(), ctx->v_slot.as<uint32_t>(), ctx->v_nd.as<uint32_t>(), ctx->v_first.as<uint32_t>(),
-            ctx->v_steps.as<uint32_t>(), ctx->v_e.as<uint32_t>(), ctx->v_np, ctx->v_k, ctx->v_tpi, ctx->v_wpc};
-  MPVSS_TRY(dev_horner(ctx, P, ctx->v_comm.as<uint32_t>(), ctx->v_cm, t, n, ctx->v_h, ctx->v_t2, X));
+  MPVSS_TRY(dev_horner(ctx, P, B.comm.as<uint32_t>(), B.cm, t, n, B.h, B.t2, X));
   if (side) {
     MPVSS_CUDA(ctx, cudaStreamWaitEvent(ctx->aux[0], ctx->ev_fork, 0));
     // 3: persistent one-warp CTAs, one per SM, into the warp slot the Horner CTAs leave empty
@@ -813,24 +769,43 @@ static int verify_kernels(mpvss_ctx* ctx) {
   }
   MPVSS_CUDA(ctx, cudaEventRecord(ctx->ev_mid, ctx->stream));
   // a1 = g^r * X^c  (g^r from the fixed-base table)
-  MPVSS_TRY(dev_exp2(ctx, K, ctx->gens.as<uint32_t>() + 64, 0, ctx->v_r.as<uint32_t>(), EW, ctx->v_rwin, X, EW,
-                     ctx->v_c.as<uint32_t>(), 0, ctx->v_cwin, n, ctx->v_a1.as<uint32_t>(), nullptr, ctx->v_comb));
+  MPVSS_TRY(dev_exp2(ctx, K, ctx->gens.as<uint32_t>() + 64, 0, B.r.as<uint32_t>(), EW, rwin, X, EW,
+                     B.c.as<uint32_t>(), cs, cwin, n, B.a1.as<uint32_t>(), nullptr, comb));
   if (side) MPVSS_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join[0], 0));
   // transcript rows F(X) F(Y) F(a1) F(a2) in local order (dleq.rs:87-99)
-  modp::FrameArgs FA{X, ctx->v_y.as<uint32_t>(), ctx->v_a1.as<uint32_t>(), ctx->v_a2.as<uint32_t>(),
-                     ctx->v_frames.as<uint8_t>(), (uint32_t)n};
+  modp::FrameArgs FA{X, B.y.as<uint32_t>(), B.a1.as<uint32_t>(), B.a2.as<uint32_t>(), B.frames.as<uint8_t>(),
+                     (uint32_t)n};
   MPVSS_CUDA(ctx, modp::launch_frames(FA, ctx->stream));
   timing_launch(ctx);
+  bad.assign(t + 2 * n, 0);
   if (ctx->validate) {
-    std::vector<uint8_t> bad(t + 2 * n, 0);
-    MPVSS_TRY(validate_elements(ctx, ctx->v_comm.as<uint32_t>(), t, bad.data()));
-    MPVSS_TRY(validate_elements(ctx, ctx->v_pk.as<uint32_t>(), n, bad.data() + t));
-    MPVSS_TRY(validate_elements(ctx, ctx->v_y.as<uint32_t>(), n, bad.data() + t + n));
-    // mark the rank's first row: 0xff is never part of a valid length (seen by all ranks)
-    if (std::find(bad.begin(), bad.end(), 1) != bad.end()) {
-      const uint8_t mark = 0xff;
-      MPVSS_CUDA(ctx, cudaMemcpyAsync(ctx->v_frames.p, &mark, 1, cudaMemcpyHostToDevice, ctx->stream));
-    }
+    MPVSS_TRY(validate_elements(ctx, B.comm.as<uint32_t>(), t, bad.data()));
+    MPVSS_TRY(validate_elements(ctx, B.pk.as<uint32_t>(), n, bad.data() + t));
+    MPVSS_TRY(validate_elements(ctx, B.y.as<uint32_t>(), n, bad.data() + t + n));
+  }
+  return MPVSS_OK;
+}
+
+// kernels of the staged verification
+static int verify_kernels(mpvss_ctx* ctx) {
+  const size_t n = ctx->v_n, t = ctx->v_t;
+  timing_begin(ctx);
+  if (n == 0) {  // more ranks than participants: this rank only takes part in the all-gather
+    MPVSS_TRY(timing_end(ctx));
+    ctx->phase_ms[0] = ctx->phase_ms[1] = ctx->phase_ms[2] = 0.f;
+    return MPVSS_OK;
+  }
+  PlanDev P{ctx->v_ops.as<uint16_t>(), ctx->v_slot.as<uint32_t>(), ctx->v_nd.as<uint32_t>(), ctx->v_first.as<uint32_t>(),
+            ctx->v_steps.as<uint32_t>(), ctx->v_e.as<uint32_t>(), ctx->v_np, ctx->v_k, ctx->v_tpi, ctx->v_wpc};
+  const VerifyBufs B{ctx->v_comm, ctx->v_pk, ctx->v_y, ctx->v_r, ctx->v_c, ctx->v_cm, ctx->v_h, ctx->v_t2,
+                     ctx->v_x, ctx->v_a1, ctx->v_a2, ctx->v_frames};
+  std::vector<uint8_t> bad;
+  MPVSS_TRY(verify_pass(ctx, P, B, t, n, 0, ctx->v_rwin, ctx->v_cwin,
+                        (double)(t > 1 ? t - 1 : 0) / (double)ctx->v_k * (double)ctx->v_nops_max, ctx->v_comb, bad));
+  // mark the rank's first row: 0xff is never part of a valid length (seen by all ranks)
+  if (std::find(bad.begin(), bad.end(), 1) != bad.end()) {
+    const uint8_t mark = 0xff;
+    MPVSS_CUDA(ctx, cudaMemcpyAsync(ctx->v_frames.p, &mark, 1, cudaMemcpyHostToDevice, ctx->stream));
   }
   MPVSS_TRY(timing_end(ctx));
   MPVSS_CUDA(ctx, cudaEventElapsedTime(&ctx->phase_ms[0], ctx->ev0, ctx->ev_mid));  // X_i (with a2 underneath)
@@ -891,9 +866,10 @@ int verify_batch(mpvss_ctx* ctx, size_t nb, const size_t* nv, const size_t* tv, 
   // a position out of range makes its box false; the other boxes are planned
   std::vector<uint8_t> live(nb, 1);
   std::vector<PlanBox> boxes;
+  std::vector<uint32_t> pos;
   for (size_t b = 0; b < nb; ++b) {
     const int64_t* p = positions ? positions + noff[b] : nullptr;
-    for (size_t i = 0; p && i < nv[b] && live[b]; ++i) live[b] = p[i] >= 1 && p[i] <= 0x7fffffff;
+    live[b] = positions_u32(p, nv[b], pos) == nv[b];
     if (live[b]) boxes.push_back(PlanBox{p, nv[b], tv[b], (uint32_t)toff[b], (uint32_t)noff[b]});
   }
   std::vector<uint8_t> cexp(N * EB);  // the box's challenge for every instance
@@ -922,47 +898,16 @@ int verify_batch(mpvss_ctx* ctx, size_t nb, const size_t* nv, const size_t* tv, 
   }
   const uint32_t* comb;
   MPVSS_TRY(comb_table(ctx, 1, &comb));
-  const uint32_t* K = ctx->consts_q.as<uint32_t>();
   std::vector<uint8_t> bad(Tt + 2 * N, 0);  // validate: per commitment, public key and share
   timing_begin(ctx);
   if (!boxes.empty()) {
-    // a2 = y^r * Y^c (independent of X)
-    auto launch_a2 = [&](cudaStream_t s) {
-      return dev_exp2(ctx, K, dpk.as<uint32_t>(), EW, dr.as<uint32_t>(), EW, rwin, dy.as<uint32_t>(), EW,
-                      dc.as<uint32_t>(), EW, cwin, N, da2.as<uint32_t>(), s);
-    };
     size_t tmax = 1;
     for (const PlanBox& bx : boxes) tmax = std::max(tmax, bx.t);
-    const int overlap = a2_placement(ctx, N, (double)(tmax - 1) * (double)plan.nops_max, plan.slot.size(), plan.tpi,
-                                     rwin, cwin);
-    const bool side = overlap == 2 || overlap == 3;
-    MPVSS_CUDA(ctx, cudaEventRecord(ctx->ev_fork, ctx->stream));
-    if (!side) MPVSS_TRY(launch_a2(ctx->stream));
-    // X_i of every box (participant.rs:423-434); rows of boxes left out of the plan stay unwritten
+    // rows of boxes left out of the plan stay unwritten
     PlanDev P{dops.as<uint16_t>(), dsl.as<uint32_t>(), dno.as<uint32_t>(), dfi.as<uint32_t>(), dstp.as<uint32_t>(),
               nullptr, plan.slot.size(), plan.K, plan.tpi, plan.wpc, true};
-    MPVSS_TRY(dev_horner(ctx, P, dcomm.as<uint32_t>(), dcm, Tt, N, ctx->buf(15), ctx->buf(16), dx.as<uint32_t>()));
-    if (side) {
-      MPVSS_CUDA(ctx, cudaStreamWaitEvent(ctx->aux[0], ctx->ev_fork, 0));
-      if (overlap == 3) ctx->exp2_filler_ctas = (size_t)ctx->sm_count;
-      int rc = launch_a2(ctx->aux[0]);
-      ctx->exp2_filler_ctas = 0;
-      MPVSS_TRY(rc);
-      MPVSS_CUDA(ctx, cudaEventRecord(ctx->ev_join[0], ctx->aux[0]));
-    }
-    // a1 = g^r * X^c  (g^r from the fixed-base table)
-    MPVSS_TRY(dev_exp2(ctx, K, ctx->gens.as<uint32_t>() + 64, 0, dr.as<uint32_t>(), EW, rwin, dx.as<uint32_t>(), EW,
-                       dc.as<uint32_t>(), EW, cwin, N, da1.as<uint32_t>(), nullptr, comb));
-    if (side) MPVSS_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join[0], 0));
-    modp::FrameArgs FA{dx.as<uint32_t>(), dy.as<uint32_t>(), da1.as<uint32_t>(), da2.as<uint32_t>(), dfr.as<uint8_t>(),
-                       (uint32_t)N};
-    MPVSS_CUDA(ctx, modp::launch_frames(FA, ctx->stream));
-    timing_launch(ctx);
-    if (ctx->validate) {
-      MPVSS_TRY(validate_elements(ctx, dcomm.as<uint32_t>(), Tt, bad.data()));
-      MPVSS_TRY(validate_elements(ctx, dpk.as<uint32_t>(), N, bad.data() + Tt));
-      MPVSS_TRY(validate_elements(ctx, dy.as<uint32_t>(), N, bad.data() + Tt + N));
-    }
+    const VerifyBufs B{dcomm, dpk, dy, dr, dc, dcm, ctx->buf(15), ctx->buf(16), dx, da1, da2, dfr};
+    MPVSS_TRY(verify_pass(ctx, P, B, Tt, N, EW, rwin, cwin, (double)(tmax - 1) * (double)plan.nops_max, comb, bad));
   }
   MPVSS_TRY(timing_end(ctx));
   ctx->horner_sqr = plan.sqr;
@@ -997,8 +942,7 @@ int distribute(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* secret, 
                                 commitments_out && shares_out && challenge_out && responses_out && u_out &&
                                 secret_len <= EB,
                        "distribute: bad arguments (threshold <= n, participant.rs:166; secret at most 256 bytes)"));
-  std::vector<uint32_t> order(EW, 0);
-  for (size_t i = 0; i < ctx->qm1.size(); ++i) order[i] = ctx->qm1[i];
+  const std::vector<uint32_t> order = order_limbs(ctx);
   if (order[EW - 1] != 0xffffffffu || order[EW - 2] != 0xffffffffu)
     return mpvss_fail(ctx, MPVSS_ERR_UNSUPPORTED, "distribute: scalar kernels need an order with all-ones top limbs");
   // this rank's participants: rank, rank + N, ... (all of them without a communicator)
@@ -1099,12 +1043,8 @@ int distribute(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* secret, 
   MPVSS_TRY(d2h(ctx, commitments_out, dC, t * EB));
   MPVSS_TRY(d2h(ctx, gs, dGs, EB));
   MPVSS_TRY(sync(ctx));
-  // U = secret XOR (int(SHA-256(bytes(G^s))) mod q)  (participant.rs:269-272)
-  uint8_t tmp[EB], hs[32];
-  size_t len = min_be(gs, tmp);
-  sha2::sha256(tmp, len, hs);
-  big::Int mask = big::mod(big::from_be(hs, 32), ctx->q);
-  big::Int u = big::bxor(big::from_be(secret, secret_len), mask);
+  // U = secret XOR (int(SHA-256(bytes(G^s))) mod q)
+  big::Int u = big::bxor(big::from_be(secret, secret_len), u_mask(ctx, gs));
   big::to_be(u, u_out, EB);
   // the scratch buffers held secrets (coefficients, P(i), witnesses)
   for (DevBuf* b : {&dco, &dp, &dw, &ds}) MPVSS_CUDA(ctx, cudaMemsetAsync(b->p, 0, b->cap, ctx->stream));
@@ -1246,8 +1186,7 @@ int extract_shares(mpvss_ctx* ctx, size_t n, const uint8_t* private_keys, const 
   {
     // challenge per share from the transcript (pk, Y, a1, a2) (participant.rs:330-340) and the response
     // r = w - sk*c mod (q-1) (dleq.rs:42-50 with modp.rs:180-192), both on the device: a1 / a2 stay there
-    std::vector<uint32_t> order(EW, 0);
-    for (size_t i = 0; i < ctx->qm1.size(); ++i) order[i] = ctx->qm1[i];
+    const std::vector<uint32_t> order = order_limbs(ctx);
     DevBuf &dord = ctx->buf(11), &dch = ctx->buf(12), &dR = ctx->buf(13);
     MPVSS_TRY(h2d(ctx, dord, order.data(), EB));
     MPVSS_CUDA(ctx, dch.ensure(n * EB));
@@ -1299,69 +1238,74 @@ int verify_shares(mpvss_ctx* ctx, size_t n, const uint8_t* publickeys, const uin
 }
 
 // -------------------------------------------------------------- reconstruct ----
+// The steps after a Lagrange launch that left `parts` partial products of n numerators / denominators mod g and
+// their sign flags in dnum / dden / dneg: the part products, den^-1 by one batch inversion, lambda = num * den^-1
+// into dlam (which may be dnum), the end of the timing bracket the Lagrange launch opened, then lam on the host
+// with the sign folded into the exponent: S^(-lambda) = S^((q-1) - lambda).
+static int lagrange_lambdas(mpvss_ctx* ctx, DevBuf& dnum, DevBuf& dden, DevBuf& dneg, DevBuf& dinv, DevBuf& dlam,
+                            size_t n, size_t parts, std::vector<uint8_t>& lam) {
+  const uint32_t* Kg = ctx->consts_g.as<uint32_t>();
+  for (size_t half = parts / 2; half >= 1; half /= 2)  // rows [0, half n) *= rows [half n, 2 half n), mod g
+    for (DevBuf* b : {&dnum, &dden})
+      MPVSS_TRY(dev_mul(ctx, Kg, b->as<uint32_t>(), EW, b->as<uint32_t>() + half * n * EW, EW, 0, half * n,
+                        b->as<uint32_t>()));
+  // den^-1 mod g: the denominators are products of non-zero integers below 2^31 < g, so none is 0 mod g
+  MPVSS_TRY(dev_batch_inverse_g(ctx, dden.as<uint32_t>(), n, dinv.as<uint32_t>()));
+  MPVSS_TRY(dev_mul(ctx, Kg, dnum.as<uint32_t>(), EW, dinv.as<uint32_t>(), EW, 0, n, dlam.as<uint32_t>()));
+  MPVSS_TRY(timing_end(ctx));
+  lam.resize(n * EB);
+  std::vector<uint32_t> negf(parts * n);
+  MPVSS_TRY(d2h(ctx, lam.data(), dlam, n * EB));
+  MPVSS_TRY(d2h(ctx, negf.data(), dneg, parts * n * 4));
+  MPVSS_TRY(sync(ctx));
+  for (size_t i = 0; i < n; ++i) {
+    for (size_t p = 1; p < parts; ++p) negf[i] ^= negf[p * n + i];
+    if (!negf[i]) continue;
+    big::Int l = big::from_le(lam.data() + i * EB, EB);
+    if (!big::is_zero(l)) big::to_le(big::sub(ctx->qm1, l), lam.data() + i * EB, EB);
+  }
+  return MPVSS_OK;
+}
+
 int reconstruct(mpvss_ctx* ctx, size_t k, const int64_t* positions, const uint8_t* shares, const uint8_t* u,
                 uint8_t* secret_out, uint8_t* gs_out) {
   MPVSS_TRY(check_args(ctx, k > 0 && positions && shares && u && secret_out, "reconstruct: bad arguments"));
-  for (size_t i = 0; i < k; ++i)
-    if (positions[i] < 1 || positions[i] > 0x7fffffff) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range");
+  std::vector<uint32_t> pos;
+  if (positions_u32(positions, k, pos) != k) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range");
   // lambda_i = prod_{j != i} j / (j - i) mod g with the sign folded into the exponent:
   // S^(-lambda) = S^((q-1) - lambda)  (participant.rs:535-558, element_inverse modp.rs:138-140).
   // Numerators / denominators mod q-1 on the device (one position per thread), then
-  // den^-1 = den^(g-2) mod g and lambda = num * den^-1 mod g with the kernels of modulus g.
-  std::vector<uint32_t> pos(k), order(EW, 0);
-  for (size_t i = 0; i < k; ++i) pos[i] = (uint32_t)positions[i];
+  // den^-1 mod g and lambda = num * den^-1 mod g with the kernels of modulus g (lagrange_lambdas).
   {
     std::vector<uint32_t> sorted(pos);
     std::sort(sorted.begin(), sorted.end());
     if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
       return mpvss_fail(ctx, MPVSS_ERR_ARG, "duplicate position");
   }
-  for (size_t i = 0; i < ctx->qm1.size(); ++i) order[i] = ctx->qm1[i];
-  std::vector<uint8_t> lam(k * EB);
+  const std::vector<uint32_t> order = order_limbs(ctx);
+  std::vector<uint8_t> lam;
   DevBuf &dpos = ctx->buf(12), &dord = ctx->buf(13), &dnum = ctx->buf(14), &dden = ctx->buf(15), &dneg = ctx->buf(16),
          &dinv = ctx->buf(18), &dlam = ctx->buf(19);
   MPVSS_TRY(h2d(ctx, dpos, pos.data(), k * 4));
   MPVSS_TRY(h2d(ctx, dord, order.data(), EB));
-  // the k-term products are cut into `parts` ranges (more, shorter threads), multiplied together mod g below
+  // the k-term products are cut into `parts` ranges (more, shorter threads), multiplied together mod g afterwards
   const size_t parts = k >= 64 ? 8 : 1;
   for (DevBuf* b : {&dnum, &dden}) MPVSS_CUDA(ctx, b->ensure(parts * k * EB));
   for (DevBuf* b : {&dinv, &dlam}) MPVSS_CUDA(ctx, b->ensure(k * EB));
   MPVSS_CUDA(ctx, dneg.ensure(parts * k * 4));
-  const uint32_t* Kg = ctx->consts_g.as<uint32_t>();
   modp::LagrangeArgs LA{dord.as<uint32_t>(), dpos.as<uint32_t>(), dnum.as<uint32_t>(), dden.as<uint32_t>(),
                         dneg.as<uint32_t>(), (uint32_t)k, (uint32_t)parts};
   timing_begin(ctx);  // the Lagrange part counts towards the kernel time of the call
   MPVSS_CUDA(ctx, modp::launch_lagrange(LA, ctx->stream));
   timing_launch(ctx);
-  for (size_t half = parts / 2; half >= 1; half /= 2)  // rows [0, half k) *= rows [half k, 2 half k), mod g
-    for (DevBuf* b : {&dnum, &dden})
-      MPVSS_TRY(dev_mul(ctx, Kg, b->as<uint32_t>(), EW, b->as<uint32_t>() + half * k * EW, EW, 0, half * k,
-                        b->as<uint32_t>()));
-  // den^-1 mod g: the denominators are products of non-zero integers below 2^31 < g, so none is 0 mod g
-  MPVSS_TRY(dev_batch_inverse_g(ctx, dden.as<uint32_t>(), k, dinv.as<uint32_t>()));
-  MPVSS_TRY(dev_mul(ctx, Kg, dnum.as<uint32_t>(), EW, dinv.as<uint32_t>(), EW, 0, k, dlam.as<uint32_t>()));
-  MPVSS_TRY(timing_end(ctx));
+  MPVSS_TRY(lagrange_lambdas(ctx, dnum, dden, dneg, dinv, dlam, k, parts, lam));
   const float ms_lambda = ctx->last_ms;
   const int launches_lambda = ctx->last_launches;
-  std::vector<uint32_t> negf(parts * k);
-  MPVSS_TRY(d2h(ctx, lam.data(), dlam, k * EB));
-  MPVSS_TRY(d2h(ctx, negf.data(), dneg, parts * k * 4));
-  MPVSS_TRY(sync(ctx));
-  for (size_t i = 0; i < k; ++i) {
-    for (size_t p = 1; p < parts; ++p) negf[i] ^= negf[p * k + i];
-    if (!negf[i]) continue;
-    big::Int l = big::from_le(lam.data() + i * EB, EB);
-    if (!big::is_zero(l)) big::to_le(big::sub(ctx->qm1, l), lam.data() + i * EB, EB);
-  }
   uint8_t gs[EB];
   MPVSS_TRY(multi_exp(ctx, shares, lam.data(), k, gs));
   ctx->last_ms += ms_lambda;
   ctx->last_launches += launches_lambda;
-  uint8_t tmp[EB], hs[32];
-  size_t len = min_be(gs, tmp);
-  sha2::sha256(tmp, len, hs);
-  big::Int mask = big::mod(big::from_be(hs, 32), ctx->q);  // participant.rs:512-518
-  big::to_be(big::bxor(mask, big::from_be(u, EB)), secret_out, EB);
+  big::to_be(big::bxor(u_mask(ctx, gs), big::from_be(u, EB)), secret_out, EB);
   if (gs_out) memcpy(gs_out, gs, EB);
   return MPVSS_OK;
 }
@@ -1377,84 +1321,53 @@ int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t
   if (gs_out) memset(gs_out, 0, nb * EB);
   ctx->last_ms = 0.f;
   ctx->last_launches = 0;
-  std::vector<size_t> live, first(nb);  // boxes that pass reconstruct's checks; each box's first share
+  std::vector<size_t> live;  // boxes that pass reconstruct's checks
+  std::vector<uint32_t> sorted;
   for (size_t b = 0, off = 0; b < nb; off += kv[b], ++b) {
-    first[b] = off;
-    status_out[b] = MPVSS_OK;
-    std::vector<int64_t> sorted(positions + off, positions + off + kv[b]);
-    std::sort(sorted.begin(), sorted.end());
-    if (sorted.front() < 1 || sorted.back() > 0x7fffffff || std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
-      status_out[b] = MPVSS_ERR_ARG;
-    else
-      live.push_back(b);
+    bool ok = positions_u32(positions + off, kv[b], sorted) == kv[b];
+    if (ok) {
+      std::sort(sorted.begin(), sorted.end());
+      ok = std::adjacent_find(sorted.begin(), sorted.end()) == sorted.end();
+    }
+    status_out[b] = ok ? MPVSS_OK : MPVSS_ERR_ARG;
+    if (ok) live.push_back(b);
   }
   if (live.empty()) return MPVSS_OK;
   // a lone box chooses as reconstruct does; in a batch a box joins the direct launch below msm_batch_threshold
   const size_t threshold = live.size() == 1 ? (size_t)ctx->msm_threshold : mpvss_ctx::msm_batch_threshold;
   auto buckets = [&](size_t b) { return ctx->modp_msm == 1 || (ctx->modp_msm == 2 && kv[b] >= threshold); };
   std::stable_partition(live.begin(), live.end(), [&](size_t b) { return !buckets(b); });
-  const size_t L = live.size();
-  size_t n = 0, n_direct = 0, L_direct = 0, kmax = 0;  // rows / boxes of the direct launch
-  std::vector<uint32_t> start(L), cnt(L);
+  LiveBoxes B = pack_live_boxes(nb, kv, positions, shares, EB, live);
+  const size_t L = live.size(), n = B.n;
+  const std::vector<uint32_t> &start = B.start, &cnt = B.cnt;
+  size_t n_direct = 0, L_direct = 0, kmax = 0;  // rows / boxes of the direct launch
   for (size_t j = 0; j < L; ++j) {
-    start[j] = (uint32_t)n;
-    cnt[j] = (uint32_t)kv[live[j]];
-    n += cnt[j];
     kmax = std::max<size_t>(kmax, cnt[j]);
-    if (!buckets(live[j])) n_direct = n, L_direct = j + 1;
-  }
-  std::vector<uint32_t> idx(3 * n);  // positions, then per position its box's first row, then its box's k
-  std::vector<uint8_t> host(n * EB);
-  for (size_t j = 0; j < L; ++j) {
-    const size_t b = live[j];
-    for (uint32_t i = 0; i < cnt[j]; ++i) {
-      idx[start[j] + i] = (uint32_t)positions[first[b] + i];
-      idx[n + start[j] + i] = start[j];
-      idx[2 * n + start[j] + i] = cnt[j];
-    }
-    memcpy(host.data() + (size_t)start[j] * EB, shares + first[b] * EB, cnt[j] * EB);
+    if (!buckets(live[j])) n_direct = start[j] + cnt[j], L_direct = j + 1;
   }
   // multi_exp_buckets holds buf(15..19) and dev_batch_inverse_g buf(21..23)
   DevBuf &dshares = ctx->buf(0), &dexp = ctx->buf(1), &dpow = ctx->buf(2), &dplan = ctx->buf(4), &didx = ctx->buf(10),
          &dord = ctx->buf(11), &dnum = ctx->buf(12), &dden = ctx->buf(13), &dneg = ctx->buf(14), &dinv = ctx->buf(20);
-  std::vector<uint32_t> order(EW, 0);
-  for (size_t i = 0; i < ctx->qm1.size(); ++i) order[i] = ctx->qm1[i];
-  MPVSS_TRY(h2d(ctx, didx, idx.data(), 3 * n * 4));
+  const std::vector<uint32_t> order = order_limbs(ctx);
+  MPVSS_TRY(h2d(ctx, didx, B.idx.data(), 3 * n * 4));
   MPVSS_TRY(h2d(ctx, dord, order.data(), EB));
-  MPVSS_TRY(h2d(ctx, dshares, host.data(), n * EB));
+  MPVSS_TRY(h2d(ctx, dshares, B.shares.data(), n * EB));
   const size_t parts = kmax >= 64 ? 8 : 1;  // as reconstruct cuts a box of kmax positions
   for (DevBuf* b : {&dnum, &dden}) MPVSS_CUDA(ctx, b->ensure(parts * n * EB));
   MPVSS_CUDA(ctx, dinv.ensure(n * EB));
   MPVSS_CUDA(ctx, dneg.ensure(parts * n * 4));
   MPVSS_CUDA(ctx, dpow.ensure(n * EB));
   const uint32_t* K = ctx->consts_q.as<uint32_t>();
-  const uint32_t* Kg = ctx->consts_g.as<uint32_t>();
   const uint32_t* di = didx.as<uint32_t>();
   modp::LagrangeBoxesArgs LA{dord.as<uint32_t>(), di, di + n, di + 2 * n, dnum.as<uint32_t>(), dden.as<uint32_t>(),
                              dneg.as<uint32_t>(), (uint32_t)n, (uint32_t)parts};
   timing_begin(ctx);
   MPVSS_CUDA(ctx, modp::launch_lagrange_boxes(LA, ctx->stream));
   timing_launch(ctx);
-  for (size_t half = parts / 2; half >= 1; half /= 2)
-    for (DevBuf* b : {&dnum, &dden})
-      MPVSS_TRY(dev_mul(ctx, Kg, b->as<uint32_t>(), EW, b->as<uint32_t>() + half * n * EW, EW, 0, half * n,
-                        b->as<uint32_t>()));
-  MPVSS_TRY(dev_batch_inverse_g(ctx, dden.as<uint32_t>(), n, dinv.as<uint32_t>()));
-  MPVSS_TRY(dev_mul(ctx, Kg, dnum.as<uint32_t>(), EW, dinv.as<uint32_t>(), EW, 0, n, dnum.as<uint32_t>()));  // lambda
-  MPVSS_TRY(timing_end(ctx));
+  std::vector<uint8_t> lam;
+  MPVSS_TRY(lagrange_lambdas(ctx, dnum, dden, dneg, dinv, dnum, n, parts, lam));  // lambda in place of num
   const float ms_lambda = ctx->last_ms;
   const int launches_lambda = ctx->last_launches;
-  std::vector<uint8_t> lam(n * EB);
-  std::vector<uint32_t> negf(parts * n);
-  MPVSS_TRY(d2h(ctx, lam.data(), dnum, n * EB));
-  MPVSS_TRY(d2h(ctx, negf.data(), dneg, parts * n * 4));
-  MPVSS_TRY(sync(ctx));
-  for (size_t i = 0; i < n; ++i) {
-    for (size_t p = 1; p < parts; ++p) negf[i] ^= negf[p * n + i];
-    if (!negf[i]) continue;
-    big::Int l = big::from_le(lam.data() + i * EB, EB);
-    if (!big::is_zero(l)) big::to_le(big::sub(ctx->qm1, l), lam.data() + i * EB, EB);
-  }
   MPVSS_TRY(h2d(ctx, dexp, lam.data(), n * EB));
   // the direct boxes' product trees, every level planned here and uploaded at once
   std::vector<uint32_t> rows(3 * n_direct), level_end;
@@ -1489,18 +1402,38 @@ int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t
   MPVSS_TRY(timing_end(ctx));
   ctx->last_ms += ms_lambda;
   ctx->last_launches += launches_lambda;
+  std::vector<uint8_t>& host = B.shares;  // uploaded already: takes the results
   MPVSS_TRY(d2h(ctx, host.data(), dpow, n * EB));
   MPVSS_TRY(sync(ctx));
   for (size_t j = 0; j < L; ++j) {
     const size_t b = live[j];
     const uint8_t* gs = host.data() + (size_t)start[j] * EB;
-    uint8_t tmp[EB], hs[32];
-    sha2::sha256(tmp, min_be(gs, tmp), hs);
-    big::Int mask = big::mod(big::from_be(hs, 32), ctx->q);  // participant.rs:512-518
-    big::to_be(big::bxor(mask, big::from_be(u + b * EB, EB)), secrets_out + b * EB, EB);
+    big::to_be(big::bxor(u_mask(ctx, gs), big::from_be(u + b * EB, EB)), secrets_out + b * EB, EB);
     if (gs_out) memcpy(gs_out + b * EB, gs, EB);
   }
   return MPVSS_OK;
 }
 
 }  // namespace modp_api
+
+const GroupOps modp_ops = [] {
+  GroupOps o{};
+  o.init = modp_api::init;
+  o.batch_exp = modp_api::batch_exp;
+  o.fixed_base_exp = modp_api::fixed_base_exp;
+  o.batch_mul = modp_api::batch_mul;
+  o.poly_eval_exp = modp_api::poly_eval_exp;
+  o.dleq_verify_commit = modp_api::dleq_verify_commit;
+  o.dleq_prove_commit = modp_api::dleq_prove_commit;
+  o.multi_exp = modp_api::multi_exp;
+  o.verify_stage = modp_api::verify_stage;
+  o.verify_run = modp_api::verify_run;
+  o.verify_batch = modp_api::verify_batch;
+  o.scalar_poly_eval = modp_api::scalar_poly_eval;
+  o.distribute = modp_api::distribute;
+  o.extract_shares = modp_api::extract_shares;
+  o.verify_shares = modp_api::verify_shares;
+  o.reconstruct = modp_api::reconstruct;
+  o.reconstruct_batch = modp_api::reconstruct_batch;
+  return o;
+}();
