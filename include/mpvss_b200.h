@@ -173,6 +173,26 @@ int mpvss_distribute(mpvss_ctx* ctx, size_t n, size_t t, const uint8_t* secret, 
                      const uint8_t* coeffs, const uint8_t* witnesses, const uint8_t* publickeys,
                      uint8_t* commitments_out, uint8_t* shares_out, uint8_t* challenge_out, uint8_t* responses_out,
                      uint8_t* u_out, uint8_t* x_out);
+/* n_boxes independent Participant::distribute_secret calls in one (e.g. the boxes of many future beacon epochs,
+ * or every dealer of a round played by one harness).  Box b has n[b] participants at positions 1..n[b] and t[b]
+ * coefficients.  Every array is the concatenation, in box order, of what mpvss_distribute takes or returns for
+ * one box: coeffs (sum t[b] scalars), witnesses (sum n[b] scalars), publickeys (sum n[b] elements),
+ * commitments_out (sum t[b] elements), shares_out (sum n[b] elements), responses_out (sum n[b] scalars), x_out
+ * (optional, sum n[b] elements), challenges_out (n_boxes scalars).  secrets and u_out hold n_boxes rows of
+ * element size, big-endian and left-padded (the width mpvss_reconstruct takes U and returns secrets in).  Every
+ * row of box b is byte-identical to what mpvss_distribute returns for box b alone.  status_out[b] is that box's
+ * status: in secp256k1 and ristretto255 MPVSS_ERR_ENCODING for an undecodable public key, and in secp256k1 also
+ * for a coefficient or witness not below the group order or a SHA-256(G^s) that is not a canonical scalar;
+ * ModpGroup rejects no box.  A rejected box has zero rows in every output and leaves the other boxes alone; the
+ * call still returns MPVSS_OK and records no error.  Caller errors return MPVSS_ERR_ARG: no boxes, a null
+ * pointer other than x_out, n[b] == 0, t[b] == 0, t[b] > n[b], or more participants or coefficients than 32-bit
+ * counts hold.  Staged mpvss_verify_distribution_stage state is left untouched.  Not collective: on a context
+ * with a communicator it returns MPVSS_ERR_UNSUPPORTED. */
+int mpvss_distribute_secrets(mpvss_ctx* ctx, size_t n_boxes, const size_t* n, const size_t* t,
+                             const uint8_t* secrets, const uint8_t* coeffs, const uint8_t* witnesses,
+                             const uint8_t* publickeys, uint8_t* commitments_out, uint8_t* shares_out,
+                             uint8_t* challenges_out, uint8_t* responses_out, uint8_t* u_out, uint8_t* x_out,
+                             int* status_out);
 
 /* n independent Participant::extract_secret_share calls (participant.rs:294-353 / 1282-1338 /
  * 1725-1781): private key, witness and encrypted share per participant ->

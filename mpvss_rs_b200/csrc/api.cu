@@ -289,6 +289,31 @@ int mpvss_distribute(mpvss_ctx* ctx, size_t n, size_t t, const uint8_t* secret, 
   DISPATCH(ctx, distribute, n, t, secret, secret_len, coeffs, witnesses, publickeys, commitments_out, shares_out,
            challenge_out, responses_out, u_out, x_out);
 }
+int mpvss_distribute_secrets(mpvss_ctx* ctx, size_t n_boxes, const size_t* n, const size_t* t,
+                             const uint8_t* secrets, const uint8_t* coeffs, const uint8_t* witnesses,
+                             const uint8_t* publickeys, uint8_t* commitments_out, uint8_t* shares_out,
+                             uint8_t* challenges_out, uint8_t* responses_out, uint8_t* u_out, uint8_t* x_out,
+                             int* status_out) {
+  if (!ctx) return MPVSS_ERR_ARG;
+  Guard hold(ctx);
+  if (n_boxes == 0 || !n || !t || !secrets || !coeffs || !witnesses || !publickeys || !commitments_out || !shares_out ||
+      !challenges_out || !responses_out || !u_out || !status_out)
+    return mpvss_fail(ctx, MPVSS_ERR_ARG, "distribute_secrets: bad arguments");
+  // the kernels count participants and coefficients in 32 bits
+  const size_t limit = 0x7fffffff;
+  size_t sum_n = 0, sum_t = 0;
+  for (size_t b = 0; b < n_boxes; ++b) {
+    if (n[b] == 0 || t[b] == 0 || t[b] > n[b] || n[b] > limit - sum_n || t[b] > limit - sum_t)
+      return mpvss_fail(ctx, MPVSS_ERR_ARG, "distribute_secrets: box " + std::to_string(b) +
+                                                " has no participants, no coefficients or more coefficients than "
+                                                "participants (participant.rs:166), or the boxes are too many");
+    sum_n += n[b];
+    sum_t += t[b];
+  }
+  if (ctx->nranks > 1) return mpvss_fail(ctx, MPVSS_ERR_UNSUPPORTED, "distribute_secrets: not collective");
+  DISPATCH(ctx, distribute_batch, n_boxes, n, t, secrets, coeffs, witnesses, publickeys, commitments_out, shares_out,
+           challenges_out, responses_out, u_out, x_out, status_out);
+}
 int mpvss_extract_shares(mpvss_ctx* ctx, size_t n, const uint8_t* private_keys, const uint8_t* witnesses,
                          const uint8_t* enc_shares, uint8_t* publickeys_out, uint8_t* shares_out,
                          uint8_t* challenges_out, uint8_t* responses_out, int* status_out) {

@@ -176,6 +176,8 @@ struct GroupOps {
   int (*scalar_poly_eval)(mpvss_ctx*, const uint8_t*, size_t, const int64_t*, size_t, uint8_t*);
   int (*distribute)(mpvss_ctx*, size_t, size_t, const uint8_t*, size_t, const uint8_t*, const uint8_t*, const uint8_t*,
                     uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*);
+  int (*distribute_batch)(mpvss_ctx*, size_t, const size_t*, const size_t*, const uint8_t*, const uint8_t*,
+                          const uint8_t*, const uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, uint8_t*, int*);
   int (*extract_shares)(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*,
                         uint8_t*, uint8_t*, int*);
   int (*verify_shares)(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,

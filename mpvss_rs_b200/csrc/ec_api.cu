@@ -738,6 +738,56 @@ struct Ec {
   }
 
   // ---- distribute_secret -------------------------------------------------------------------------
+  // Device buffers of one dealing launch sequence: coefficient and witness limbs, public keys and positions in;
+  // P(i) limbs, C, X, Y, a1, a2, the decode status of Y / a2 (2 x n) and the framed transcript rows out.
+  struct DealBufs {
+    const uint32_t *co, *w;
+    const uint8_t* pk;
+    uint32_t* p;
+    uint8_t *C, *X, *Y, *A1, *A2;
+    uint32_t* st;
+    uint8_t* frames;
+  };
+  // The dealer's launches: C over t coefficients, then, for n instances, P(i) mod order (`poly` enqueues that one
+  // launch), X, Y, a1, a2 and the frames.  An undecodable public key sets its instance's status.
+  template <class Poly>
+  static int deal_kernels(mpvss_ctx* ctx, const DealBufs& B, size_t t, size_t n, Poly poly) {
+    // C_j = a_j * g (participant.rs:1130-1146 / 1603-1610), fixed-base table; every rank computes all of them
+    MPVSS_TRY(dev_fixed(ctx, B.co, t, B.C));
+    if (!n) return MPVSS_OK;
+    // p_i = P(i) mod order (participant.rs:1155-1157 / 1619-1621)
+    MPVSS_CUDA(ctx, poly());
+    timing_launch(ctx);
+    // X_i = p_i * g (dealer shortcut: same element as sum_j i^j C_j) ; Y_i = p_i * y_i ; a1 = w * g ; a2 = w * y_i
+    MPVSS_TRY(dev_fixed(ctx, B.p, n, B.X));
+    MPVSS_TRY(dev_exp2(ctx, B.pk, EB, B.p, nullptr, 0, nullptr, 0, n, B.Y, nullptr, B.st));
+    MPVSS_TRY(dev_fixed(ctx, B.w, n, B.A1));
+    MPVSS_TRY(dev_exp2(ctx, B.pk, EB, B.w, nullptr, 0, nullptr, 0, n, B.A2, nullptr, B.st + n));
+    ec::FrameArgs FA{B.X, B.Y, B.A1, B.A2, B.frames, (uint32_t)n, (uint32_t)EB};
+    MPVSS_CUDA(ctx, ec::launch_frames(FA, ctx->stream));
+    timing_launch(ctx);
+    return MPVSS_OK;
+  }
+  // r_i = w_i - p_i * c for n instances, p and w as 8-limb rows (participant.rs:1221-1231 / 1679-1688)
+  static void responses(const mpvss_ctx* ctx, const uint32_t* p, const uint32_t* w, const big::Int& c, size_t n,
+                        uint8_t* out) {
+    const big::Int& ord = ctx->ec_order;
+    for (size_t j = 0; j < n; ++j) {
+      big::Int pi(p + j * 8, p + j * 8 + 8), wi(w + j * 8, w + j * 8 + 8);
+      big::trim(pi);
+      big::trim(wi);
+      scalar_out(big::submod(wi, big::mulmod(pi, c, ord), ord), out + j * SB);
+    }
+  }
+  // U = secret XOR mask(a_0 * G) as element-size big-endian bytes (participant.rs:1234-1260 / 1691-1703); C_0 is
+  // that point.  False where the group rejects the mask.
+  static bool mask_secret(const mpvss_ctx* ctx, const uint8_t* c0, const uint8_t* secret, size_t len, uint8_t* u_out) {
+    big::Int mask;
+    if (!T::mask_of(c0, ctx->ec_order, &mask)) return false;
+    big::to_be(big::bxor(big::from_be(secret, len), mask), u_out, EB);
+    return true;
+  }
+
   // With a communicator the call is collective: rank r deals participants r, r + N, ... (commitments are
   // computed by every rank), one all-gather carries the framed transcript rows, a second one the shares,
   // responses and X of all ranks.
@@ -779,25 +829,11 @@ struct Ec {
     MPVSS_CUDA(ctx, cudaMemsetAsync(ctx->v_frames.p, 0, rpr * g.row(), ctx->stream));
     if (ctx->nranks > 1) MPVSS_CUDA(ctx, ctx->v_gather.ensure(N * rpr * g.row()));
     timing_begin(ctx);
-    // C_j = a_j * g (participant.rs:1130-1146 / 1603-1610), fixed-base table; every rank computes all of them
-    MPVSS_TRY(dev_fixed(ctx, dco.as<uint32_t>(), t, dC.as<uint8_t>()));
-    if (n) {
-      // p_i = P(i) mod order (participant.rs:1155-1157 / 1619-1621)
-      ec::PolyArgs PA{KN(ctx), dco.as<uint32_t>(), dpos.as<uint32_t>(), dp.as<uint32_t>(), (uint32_t)t, (uint32_t)n};
-      MPVSS_CUDA(ctx, ec::launch_poly(PA, ctx->stream));
-      timing_launch(ctx);
-      // X_i = p_i * g (dealer shortcut: same element as sum_j i^j C_j) ; Y_i = p_i * y_i ; a1 = w * g ; a2 = w * y_i
-      MPVSS_TRY(dev_fixed(ctx, dp.as<uint32_t>(), n, dX.as<uint8_t>()));
-      MPVSS_TRY(dev_exp2(ctx, dpk.as<uint8_t>(), EB, dp.as<uint32_t>(), nullptr, 0, nullptr, 0, n, dY.as<uint8_t>(),
-                         nullptr, dst.as<uint32_t>()));
-      MPVSS_TRY(dev_fixed(ctx, dw.as<uint32_t>(), n, dA1.as<uint8_t>()));
-      MPVSS_TRY(dev_exp2(ctx, dpk.as<uint8_t>(), EB, dw.as<uint32_t>(), nullptr, 0, nullptr, 0, n, dA2.as<uint8_t>(),
-                         nullptr, dst.as<uint32_t>() + n));
-      ec::FrameArgs FA{dX.as<uint8_t>(), dY.as<uint8_t>(), dA1.as<uint8_t>(), dA2.as<uint8_t>(),
-                       ctx->v_frames.as<uint8_t>(), (uint32_t)n, (uint32_t)EB};
-      MPVSS_CUDA(ctx, ec::launch_frames(FA, ctx->stream));
-      timing_launch(ctx);
-    }
+    const DealBufs B{dco.as<uint32_t>(), dw.as<uint32_t>(), dpk.as<uint8_t>(), dp.as<uint32_t>(), dC.as<uint8_t>(),
+                     dX.as<uint8_t>(), dY.as<uint8_t>(), dA1.as<uint8_t>(), dA2.as<uint8_t>(), dst.as<uint32_t>(),
+                     ctx->v_frames.as<uint8_t>()};
+    ec::PolyArgs PA{KN(ctx), dco.as<uint32_t>(), dpos.as<uint32_t>(), dp.as<uint32_t>(), (uint32_t)t, (uint32_t)n};
+    MPVSS_TRY(deal_kernels(ctx, B, t, n, [&] { return ec::launch_poly(PA, ctx->stream); }));
     MPVSS_TRY(timing_end(ctx));
     // an undecodable public key: mark the rows (the collectives below must still run on every rank)
     int bad_pk = n ? check_status(ctx, dst, 2 * n, "distribute (public keys)") : MPVSS_OK;
@@ -820,17 +856,11 @@ struct Ec {
         return mpvss_fail(ctx, MPVSS_ERR_ENCODING, "distribute: invalid public key encoding");
     big::Int c = challenge_of(ctx, h, nullptr);
     scalar_out(c, challenge_out);
-    const big::Int& ord = ctx->ec_order;
     std::vector<uint32_t> p(nn * 8);
     std::vector<uint8_t> resp(nn * SB);
     MPVSS_TRY(d2h(ctx, p.data(), dp, nn * 32));
     MPVSS_TRY(sync(ctx));
-    for (size_t j = 0; j < n; ++j) {  // r = w - p*c (participant.rs:1221-1231 / 1679-1688)
-      big::Int pi(p.begin() + j * 8, p.begin() + j * 8 + 8), wi(wl.begin() + j * 8, wl.begin() + j * 8 + 8);
-      big::trim(pi);
-      big::trim(wi);
-      scalar_out(big::submod(wi, big::mulmod(pi, c, ord), ord), resp.data() + j * SB);
-    }
+    responses(ctx, p.data(), wl.data(), c, n, resp.data());
     MPVSS_TRY(h2d(ctx, dR, resp.data(), nn * SB));
     const void* dev_rows[3] = {dY.p, dR.p, dX.p};
     uint8_t* host_rows[3] = {shares_out, responses_out, x_out};
@@ -838,11 +868,107 @@ struct Ec {
     MPVSS_TRY(transcript::gather_rows(ctx, dev_rows, host_rows, widths, x_out ? 3 : 2, n, n_total));
     MPVSS_TRY(d2h(ctx, commitments_out, dC, t * EB));
     MPVSS_TRY(sync(ctx));
-    // U = secret XOR mask(a_0 * G)  (participant.rs:1234-1260 / 1691-1703); C_0 is that point
-    big::Int mask;
-    if (!T::mask_of(commitments_out, ord, &mask))
+    if (!mask_secret(ctx, commitments_out, secret, secret_len, u_out))
       return mpvss_fail(ctx, MPVSS_ERR_ENCODING, "distribute: SHA-256(G^s) is not a canonical scalar");
-    big::to_be(big::bxor(big::from_be(secret, secret_len), mask), u_out, EB);
+    // the scratch buffers held secrets (coefficients, P(i), witnesses)
+    for (DevBuf* b : {&dco, &dp, &dw}) MPVSS_CUDA(ctx, cudaMemsetAsync(b->p, 0, b->cap, ctx->stream));
+    return sync(ctx);
+  }
+
+  // ---- mpvss_distribute_secrets: many dealings, one launch per kernel ---------------------------------
+  // The launches of distribute run once over every box (C over all coefficients, P(i) of every instance by the
+  // multi-box poly_boxes kernel, X / Y / a1 / a2 and the frames over all instances); the rows come to the host in
+  // one copy, each box's row range is hashed into its own challenge and the responses are computed on the host.  A
+  // box with a non-canonical coefficient or witness, an undecodable public key or a rejected mask gets
+  // MPVSS_ERR_ENCODING and zero rows, records no context error and leaves the other boxes alone.  Only scratch
+  // buffers are used, so the staged single-box verify state stays valid.
+  static int distribute_batch(mpvss_ctx* ctx, size_t nb, const size_t* nv, const size_t* tv, const uint8_t* secrets,
+                              const uint8_t* coeffs, const uint8_t* witnesses, const uint8_t* publickeys,
+                              uint8_t* commitments_out, uint8_t* shares_out, uint8_t* challenges_out,
+                              uint8_t* responses_out, uint8_t* u_out, uint8_t* x_out, int* status_out) {
+    std::vector<size_t> noff(nb + 1, 0), toff(nb + 1, 0);
+    for (size_t b = 0; b < nb; ++b) {
+      noff[b + 1] = noff[b] + nv[b];
+      toff[b + 1] = toff[b] + tv[b];
+    }
+    const size_t N = noff[nb], Tt = toff[nb];
+    // per instance: its position, then its box's first coefficient row, t_b and first instance row (poly_boxes_body);
+    // a box with a scalar the group rejects keeps zero limbs
+    std::vector<uint32_t> idx(4 * N), co(Tt * 8, 0), wl(N * 8, 0), bc, bw;
+    for (size_t b = 0; b < nb; ++b) {
+      status_out[b] = scalars_in(ctx, coeffs + toff[b] * SB, tv[b], bc, false) == MPVSS_OK &&
+                              scalars_in(ctx, witnesses + noff[b] * SB, nv[b], bw, false) == MPVSS_OK
+                          ? MPVSS_OK
+                          : MPVSS_ERR_ENCODING;
+      if (status_out[b] == MPVSS_OK) {
+        memcpy(&co[toff[b] * 8], bc.data(), tv[b] * 32);
+        memcpy(&wl[noff[b] * 8], bw.data(), nv[b] * 32);
+      }
+      for (size_t i = noff[b]; i < noff[b + 1]; ++i) {
+        idx[i] = (uint32_t)(i - noff[b] + 1);
+        idx[N + i] = (uint32_t)toff[b];
+        idx[2 * N + i] = (uint32_t)tv[b];
+        idx[3 * N + i] = (uint32_t)noff[b];
+      }
+    }
+    DevBuf &dco = ctx->buf(0), &dp = ctx->buf(1), &dw = ctx->buf(2), &dpk = ctx->buf(3), &dC = ctx->buf(4),
+           &dX = ctx->buf(5), &dY = ctx->buf(6), &dA1 = ctx->buf(7), &dA2 = ctx->buf(8), &didx = ctx->buf(9),
+           &dst = ctx->buf(10), &dfr = ctx->buf(11);
+    MPVSS_TRY(h2d(ctx, dco, co.data(), Tt * 32));
+    MPVSS_TRY(h2d(ctx, dw, wl.data(), N * 32));
+    MPVSS_TRY(h2d(ctx, dpk, publickeys, N * EB));
+    MPVSS_TRY(h2d(ctx, didx, idx.data(), idx.size() * 4));
+    MPVSS_CUDA(ctx, dp.ensure(N * 32));
+    MPVSS_CUDA(ctx, dC.ensure(Tt * EB));
+    for (DevBuf* b : {&dX, &dY, &dA1, &dA2}) MPVSS_CUDA(ctx, b->ensure(N * EB));
+    MPVSS_CUDA(ctx, dst.ensure(2 * N * 4));
+    const transcript::Geom g = geom();
+    const size_t row = g.row();
+    MPVSS_CUDA(ctx, dfr.ensure(N * row));
+    timing_begin(ctx);
+    const DealBufs B{dco.as<uint32_t>(), dw.as<uint32_t>(), dpk.as<uint8_t>(), dp.as<uint32_t>(), dC.as<uint8_t>(),
+                     dX.as<uint8_t>(), dY.as<uint8_t>(), dA1.as<uint8_t>(), dA2.as<uint8_t>(), dst.as<uint32_t>(),
+                     dfr.as<uint8_t>()};
+    const uint32_t* di = didx.as<uint32_t>();
+    ec::PolyBoxesArgs PA{KN(ctx), dco.as<uint32_t>(), di, di + N, di + 2 * N, di + 3 * N, dp.as<uint32_t>(),
+                         (uint32_t)N};
+    MPVSS_TRY(deal_kernels(ctx, B, Tt, N, [&] { return ec::launch_poly_boxes(PA, ctx->stream); }));
+    MPVSS_TRY(timing_end(ctx));
+    // rows, then the decode status of Y / a2, then P(i), in one pinned buffer
+    PinBuf& host = ctx->pin(0);
+    MPVSS_CUDA(ctx, host.ensure(N * row + 2 * N * 4 + N * 32));
+    uint8_t* rows = host.as<uint8_t>();
+    uint32_t* hst = reinterpret_cast<uint32_t*>(rows + N * row);
+    uint32_t* hp = hst + 2 * N;
+    MPVSS_TRY(d2h(ctx, rows, dfr, N * row));
+    MPVSS_TRY(d2h(ctx, hst, dst, 2 * N * 4));
+    MPVSS_TRY(d2h(ctx, hp, dp, N * 32));
+    MPVSS_TRY(d2h(ctx, shares_out, dY, N * EB));
+    if (x_out) MPVSS_TRY(d2h(ctx, x_out, dX, N * EB));
+    MPVSS_TRY(d2h(ctx, commitments_out, dC, Tt * EB));
+    MPVSS_TRY(sync(ctx));
+    for (size_t b = 0; b < nb; ++b) {
+      for (size_t i = noff[b]; i < noff[b + 1] && status_out[b] == MPVSS_OK; ++i)
+        if (hst[i] == 1 || hst[N + i] == 1) status_out[b] = MPVSS_ERR_ENCODING;
+      if (status_out[b] == MPVSS_OK) {
+        sha2::Sha256 h;  // participant.rs:1205-1212: (X, Y, a1, a2) in publickeys order
+        transcript::hash_ordered(h, rows, noff[b], noff[b + 1], g);
+        const big::Int c = challenge_of(ctx, h, nullptr);
+        scalar_out(c, challenges_out + b * SB);
+        responses(ctx, hp + noff[b] * 8, wl.data() + noff[b] * 8, c, nv[b], responses_out + noff[b] * SB);
+        if (!mask_secret(ctx, commitments_out + toff[b] * EB, secrets + b * EB, EB, u_out + b * EB))
+          status_out[b] = MPVSS_ERR_ENCODING;
+      }
+      if (status_out[b] != MPVSS_OK) {  // a rejected box has zero rows
+        memset(commitments_out + toff[b] * EB, 0, tv[b] * EB);
+        memset(shares_out + noff[b] * EB, 0, nv[b] * EB);
+        memset(challenges_out + b * SB, 0, SB);
+        memset(responses_out + noff[b] * SB, 0, nv[b] * SB);
+        memset(u_out + b * EB, 0, EB);
+        if (x_out) memset(x_out + noff[b] * EB, 0, nv[b] * EB);
+      }
+    }
+    memset(hp, 0, N * 32);  // P(i) is secret
     // the scratch buffers held secrets (coefficients, P(i), witnesses)
     for (DevBuf* b : {&dco, &dp, &dw}) MPVSS_CUDA(ctx, cudaMemsetAsync(b->p, 0, b->cap, ctx->stream));
     return sync(ctx);
@@ -1087,6 +1213,7 @@ GroupOps ec_ops() {
   o.verify_batch = E::verify_batch;
   o.scalar_poly_eval = E::scalar_poly_eval;
   o.distribute = E::distribute;
+  o.distribute_batch = E::distribute_batch;
   o.extract_shares = E::extract_shares;
   o.verify_shares = E::verify_shares;
   o.reconstruct = E::reconstruct;

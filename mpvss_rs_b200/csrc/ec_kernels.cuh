@@ -453,6 +453,26 @@ MP_DEV void poly_body(const PolyArgs& A, uint32_t tid) {
   store(A.out + (size_t)tid * 8, from_mont(acc, N));
 }
 
+// Several boxes at once (mpvss_distribute_secrets): the coefficients and the instances of the boxes are
+// concatenated, and instance i evaluates the polynomial of its own box: t_b = bt[i] coefficients from row coff[i],
+// the box's instances starting at row ioff[i].
+struct PolyBoxesArgs {
+  const Modulus* N;
+  const uint32_t* coeffs;  // sum t_b x 8 limbs, concatenated over the boxes
+  const uint32_t* pos;     // n positions, concatenated over the boxes
+  const uint32_t* coff;    // per instance: first coefficient row of its box
+  const uint32_t* bt;      // per instance: coefficients t_b of its box
+  const uint32_t* ioff;    // per instance: first instance row of its box
+  uint32_t* out;           // n x 8 limbs
+  uint32_t n;
+};
+MP_DEV void poly_boxes_body(const PolyBoxesArgs& A, uint32_t tid) {
+  if (tid >= A.n) return;
+  const uint32_t off = A.ioff[tid];
+  poly_body(PolyArgs{A.N, A.coeffs + (size_t)A.coff[tid] * 8, A.pos + off, A.out + (size_t)off * 8, A.bt[tid], A.n - off},
+            tid - off);
+}
+
 // Lagrange coefficients at 0 for the given positions, in the scalar field, with the sign of
 // the reference folded in:  lambda_i = prod_{j != i} x_j / (x_j - x_i)  (participant.rs:1518-1557
 // computes |x_j - x_i| and a separate sign, then negates the point; negating the scalar gives

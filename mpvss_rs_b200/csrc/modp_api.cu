@@ -65,6 +65,11 @@ big::Int u_mask(const mpvss_ctx* ctx, const uint8_t* gs) {
   sha2::sha256(tmp, min_be(gs, tmp), hs);
   return big::mod(big::from_be(hs, 32), ctx->q);
 }
+// U = secret XOR (int(SHA-256(bytes(G^s))) mod q) as element-size big-endian bytes; `secret` is a big-endian
+// integer of len bytes (participant.rs:267-272)
+void mask_secret(const mpvss_ctx* ctx, const uint8_t* secret, size_t len, const uint8_t* gs, uint8_t* u_out) {
+  big::to_be(big::bxor(big::from_be(secret, len), u_mask(ctx, gs)), u_out, EB);
+}
 // the order q-1 as EW little-endian limbs (the scalar kernels' modulus)
 std::vector<uint32_t> order_limbs(const mpvss_ctx* ctx) {
   std::vector<uint32_t> order(EW, 0);
@@ -935,6 +940,44 @@ int verify_batch(mpvss_ctx* ctx, size_t nb, const size_t* nv, const size_t* tv, 
 }
 
 // --------------------------------------------------------------- distribute ----
+// Device buffers of one dealing launch sequence: coefficients, secret exponents s = a_0 mod (q-1), witnesses and
+// public keys in; P(i), C, G^s, X, Y, a1, a2 and the framed transcript rows out; the two fixed-base tables.
+struct DealBufs {
+  const uint32_t *co, *s, *w, *pk;
+  uint32_t *p, *C, *Gs, *X, *Y, *A1, *A2;
+  uint8_t* frames;
+  const uint32_t *combG, *combg;
+};
+// The dealer's launches: C over t coefficients, G^s over ns secret exponents, then, for n instances, P(i) mod (q-1)
+// (`poly` enqueues that one launch), X, Y, a1, a2 and the frames.  Secret exponents (coefficients, P(i), witnesses)
+// always run the full window count: the schedule must not depend on their size.
+template <class Poly>
+static int deal_kernels(mpvss_ctx* ctx, const DealBufs& B, size_t t, size_t ns, size_t n, Poly poly) {
+  const uint32_t* K = ctx->consts_q.as<uint32_t>();
+  const uint32_t* G = ctx->gens.as<uint32_t>();
+  const uint32_t FW = 512;
+  // C_j = g^a_j (participant.rs:189-193); every rank computes all t of them (replicated, fixed-base table)
+  MPVSS_TRY(dev_exp2(ctx, K, G + 64, 0, B.co, EW, FW, nullptr, 0, nullptr, 0, 0, t, B.C, nullptr, B.combg));
+  // G^s (participant.rs:268)
+  MPVSS_TRY(dev_exp2(ctx, K, G, 0, B.s, EW, FW, nullptr, 0, nullptr, 0, 0, ns, B.Gs, nullptr, B.combG));
+  if (!n) return MPVSS_OK;
+  // p_i = P(i) mod (q-1) (participant.rs:202), one position per thread
+  MPVSS_CUDA(ctx, poly());
+  timing_launch(ctx);
+  // X_i = prod_j C_j^(i^j) = g^P(i): the dealer knows P, one fixed-base exponentiation
+  // gives the same group element as the reference's t-term product (participant.rs:207-215)
+  MPVSS_TRY(dev_exp2(ctx, K, G + 64, 0, B.p, EW, FW, nullptr, 0, nullptr, 0, 0, n, B.X, nullptr, B.combg));
+  // Y_i = y_i^P(i) (participant.rs:219)
+  MPVSS_TRY(dev_exp2(ctx, K, B.pk, EW, B.p, EW, FW, nullptr, 0, nullptr, 0, 0, n, B.Y));
+  // a1 = g^w, a2 = y^w (participant.rs:236-237)
+  MPVSS_TRY(dev_exp2(ctx, K, G + 64, 0, B.w, EW, FW, nullptr, 0, nullptr, 0, 0, n, B.A1, nullptr, B.combg));
+  MPVSS_TRY(dev_exp2(ctx, K, B.pk, EW, B.w, EW, FW, nullptr, 0, nullptr, 0, 0, n, B.A2));
+  modp::FrameArgs FA{B.X, B.Y, B.A1, B.A2, B.frames, (uint32_t)n};
+  MPVSS_CUDA(ctx, modp::launch_frames(FA, ctx->stream));
+  timing_launch(ctx);
+  return MPVSS_OK;
+}
+
 int distribute(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* secret, size_t secret_len,
                const uint8_t* coeffs, const uint8_t* witnesses, const uint8_t* publickeys, uint8_t* commitments_out,
                uint8_t* shares_out, uint8_t* challenge_out, uint8_t* responses_out, uint8_t* u_out, uint8_t* x_out) {
@@ -952,8 +995,6 @@ int distribute(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* secret, 
   std::vector<uint8_t> tw, tpk;
   const uint8_t* w = slice_rows(ctx, witnesses, n_total, EB, tw);
   const uint8_t* pk = slice_rows(ctx, publickeys, n_total, EB, tpk);
-  const uint32_t* K = ctx->consts_q.as<uint32_t>();
-  const uint32_t* G = ctx->gens.as<uint32_t>();
   DevBuf &dco = ctx->buf(0), &dp = ctx->buf(1), &dw = ctx->buf(2), &dpk = ctx->buf(3), &dC = ctx->buf(4),
          &dX = ctx->buf(5), &dY = ctx->buf(6), &dA1 = ctx->buf(7), &dA2 = ctx->buf(8), &dGs = ctx->buf(9),
          &ds = ctx->buf(10), &dord = ctx->buf(11), &dpos = ctx->buf(12), &dR = ctx->buf(13), &dc = ctx->buf(14);
@@ -973,9 +1014,6 @@ int distribute(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* secret, 
   MPVSS_CUDA(ctx, dC.ensure(t * EB));
   MPVSS_CUDA(ctx, dGs.ensure(EB));
   MPVSS_CUDA(ctx, dc.ensure(EB));
-  // secret exponents (coefficients, P(i), witnesses) always run the full window count: the schedule must
-  // not depend on their size
-  const uint32_t FW = 512;
   const uint32_t *combG, *combg;
   MPVSS_TRY(comb_table(ctx, 0, &combG));
   MPVSS_TRY(comb_table(ctx, 1, &combg));
@@ -984,35 +1022,12 @@ int distribute(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* secret, 
   MPVSS_CUDA(ctx, cudaMemsetAsync(ctx->v_frames.p, 0, rpr * GEOM.row(), ctx->stream));
   if (ctx->nranks > 1) MPVSS_CUDA(ctx, ctx->v_gather.ensure((size_t)ctx->nranks * rpr * GEOM.row()));
   timing_begin(ctx);
-  // C_j = g^a_j (participant.rs:189-193); every rank computes all t of them (replicated, fixed-base table)
-  MPVSS_TRY(dev_exp2(ctx, K, G + 64, 0, dco.as<uint32_t>(), EW, FW, nullptr, 0, nullptr, 0, 0, t, dC.as<uint32_t>(),
-                     nullptr, combg));
-  // G^s (participant.rs:268)
-  MPVSS_TRY(dev_exp2(ctx, K, G, 0, ds.as<uint32_t>(), EW, FW, nullptr, 0, nullptr, 0, 0, 1, dGs.as<uint32_t>(), nullptr,
-                     combG));
-  if (n) {
-    // p_i = P(i) mod (q-1) (participant.rs:202), one position per thread
-    modp::PolyArgs PA{dco.as<uint32_t>(), dord.as<uint32_t>(), dpos.as<uint32_t>(), dp.as<uint32_t>(), (uint32_t)t,
-                      (uint32_t)n};
-    MPVSS_CUDA(ctx, modp::launch_poly(PA, ctx->stream));
-    timing_launch(ctx);
-    // X_i = prod_j C_j^(i^j) = g^P(i): the dealer knows P, one fixed-base exponentiation
-    // gives the same group element as the reference's t-term product (participant.rs:207-215)
-    MPVSS_TRY(dev_exp2(ctx, K, G + 64, 0, dp.as<uint32_t>(), EW, FW, nullptr, 0, nullptr, 0, 0, n, dX.as<uint32_t>(),
-                       nullptr, combg));
-    // Y_i = y_i^P(i) (participant.rs:219)
-    MPVSS_TRY(dev_exp2(ctx, K, dpk.as<uint32_t>(), EW, dp.as<uint32_t>(), EW, FW, nullptr, 0, nullptr, 0, 0, n,
-                       dY.as<uint32_t>()));
-    // a1 = g^w, a2 = y^w (participant.rs:236-237)
-    MPVSS_TRY(dev_exp2(ctx, K, G + 64, 0, dw.as<uint32_t>(), EW, FW, nullptr, 0, nullptr, 0, 0, n, dA1.as<uint32_t>(),
-                       nullptr, combg));
-    MPVSS_TRY(dev_exp2(ctx, K, dpk.as<uint32_t>(), EW, dw.as<uint32_t>(), EW, FW, nullptr, 0, nullptr, 0, 0, n,
-                       dA2.as<uint32_t>()));
-    modp::FrameArgs FA{dX.as<uint32_t>(), dY.as<uint32_t>(), dA1.as<uint32_t>(), dA2.as<uint32_t>(),
-                       ctx->v_frames.as<uint8_t>(), (uint32_t)n};
-    MPVSS_CUDA(ctx, modp::launch_frames(FA, ctx->stream));
-    timing_launch(ctx);
-  }
+  const DealBufs B{dco.as<uint32_t>(), ds.as<uint32_t>(), dw.as<uint32_t>(), dpk.as<uint32_t>(), dp.as<uint32_t>(),
+                   dC.as<uint32_t>(), dGs.as<uint32_t>(), dX.as<uint32_t>(), dY.as<uint32_t>(), dA1.as<uint32_t>(),
+                   dA2.as<uint32_t>(), ctx->v_frames.as<uint8_t>(), combG, combg};
+  modp::PolyArgs PA{dco.as<uint32_t>(), dord.as<uint32_t>(), dpos.as<uint32_t>(), dp.as<uint32_t>(), (uint32_t)t,
+                    (uint32_t)n};
+  MPVSS_TRY(deal_kernels(ctx, B, t, 1, n, [&] { return modp::launch_poly(PA, ctx->stream); }));
   MPVSS_TRY(timing_end(ctx));
   // transcript (participant.rs:238-252): one all-gather of the framed rows, one hash pass, on every rank
   const uint8_t* rows = ctx->v_frames.as<uint8_t>();
@@ -1043,9 +1058,103 @@ int distribute(mpvss_ctx* ctx, size_t n_total, size_t t, const uint8_t* secret, 
   MPVSS_TRY(d2h(ctx, commitments_out, dC, t * EB));
   MPVSS_TRY(d2h(ctx, gs, dGs, EB));
   MPVSS_TRY(sync(ctx));
-  // U = secret XOR (int(SHA-256(bytes(G^s))) mod q)
-  big::Int u = big::bxor(big::from_be(secret, secret_len), u_mask(ctx, gs));
-  big::to_be(u, u_out, EB);
+  mask_secret(ctx, secret, secret_len, gs, u_out);
+  // the scratch buffers held secrets (coefficients, P(i), witnesses)
+  for (DevBuf* b : {&dco, &dp, &dw, &ds}) MPVSS_CUDA(ctx, cudaMemsetAsync(b->p, 0, b->cap, ctx->stream));
+  return sync(ctx);
+}
+
+// ------------------------------------------------------- distribute_secrets ----
+// Many dealings in one pass: the launches of distribute run once over every box (C over all coefficients, G^s over
+// the boxes' a_0, P(i) of every instance by the multi-box poly_boxes kernel, X / Y / a1 / a2 and the frames over all
+// instances), the rows come to the host in one copy and each box's row range is hashed into its own challenge, and
+// one response launch takes one challenge per instance.  ModpGroup rejects no box.  Only scratch buffers are used,
+// so the staged single-box verify state stays valid.
+int distribute_batch(mpvss_ctx* ctx, size_t nb, const size_t* nv, const size_t* tv, const uint8_t* secrets,
+                     const uint8_t* coeffs, const uint8_t* witnesses, const uint8_t* publickeys,
+                     uint8_t* commitments_out, uint8_t* shares_out, uint8_t* challenges_out, uint8_t* responses_out,
+                     uint8_t* u_out, uint8_t* x_out, int* status_out) {
+  const std::vector<uint32_t> order = order_limbs(ctx);
+  if (order[EW - 1] != 0xffffffffu || order[EW - 2] != 0xffffffffu)
+    return mpvss_fail(ctx, MPVSS_ERR_UNSUPPORTED,
+                      "distribute_secrets: scalar kernels need an order with all-ones top limbs");
+  std::vector<size_t> noff(nb + 1, 0), toff(nb + 1, 0);
+  for (size_t b = 0; b < nb; ++b) {
+    noff[b + 1] = noff[b] + nv[b];
+    toff[b + 1] = toff[b] + tv[b];
+  }
+  const size_t N = noff[nb], Tt = toff[nb];
+  // per instance: its position, then its box's first coefficient row, t_b and first instance row (poly_boxes_body)
+  std::vector<uint32_t> idx(4 * N);
+  std::vector<uint8_t> s_le(nb * EB);
+  for (size_t b = 0; b < nb; ++b) {
+    // s = a_0 mod (q-1)  (participant.rs:267)
+    big::to_le(big::mod(big::from_le(coeffs + toff[b] * EB, EB), ctx->qm1), s_le.data() + b * EB, EB);
+    for (size_t i = noff[b]; i < noff[b + 1]; ++i) {
+      idx[i] = (uint32_t)(i - noff[b] + 1);
+      idx[N + i] = (uint32_t)toff[b];
+      idx[2 * N + i] = (uint32_t)tv[b];
+      idx[3 * N + i] = (uint32_t)noff[b];
+    }
+  }
+  DevBuf &dco = ctx->buf(0), &dp = ctx->buf(1), &dw = ctx->buf(2), &dpk = ctx->buf(3), &dC = ctx->buf(4),
+         &dX = ctx->buf(5), &dY = ctx->buf(6), &dA1 = ctx->buf(7), &dA2 = ctx->buf(8), &dGs = ctx->buf(9),
+         &ds = ctx->buf(10), &dord = ctx->buf(11), &didx = ctx->buf(12), &dR = ctx->buf(13), &dc = ctx->buf(14),
+         &dfr = ctx->buf(15);
+  MPVSS_TRY(h2d(ctx, dco, coeffs, Tt * EB));
+  MPVSS_TRY(h2d(ctx, dord, order.data(), EB));
+  MPVSS_TRY(h2d(ctx, didx, idx.data(), idx.size() * 4));
+  MPVSS_TRY(h2d(ctx, ds, s_le.data(), nb * EB));
+  MPVSS_TRY(h2d(ctx, dw, witnesses, N * EB));
+  MPVSS_TRY(h2d(ctx, dpk, publickeys, N * EB));
+  for (DevBuf* b : {&dp, &dX, &dY, &dA1, &dA2, &dR, &dc}) MPVSS_CUDA(ctx, b->ensure(N * EB));
+  MPVSS_CUDA(ctx, dC.ensure(Tt * EB));
+  MPVSS_CUDA(ctx, dGs.ensure(nb * EB));
+  MPVSS_CUDA(ctx, dfr.ensure(N * GEOM.row()));
+  const uint32_t *combG, *combg;
+  MPVSS_TRY(comb_table(ctx, 0, &combG));
+  MPVSS_TRY(comb_table(ctx, 1, &combg));
+  timing_begin(ctx);
+  const DealBufs B{dco.as<uint32_t>(), ds.as<uint32_t>(), dw.as<uint32_t>(), dpk.as<uint32_t>(), dp.as<uint32_t>(),
+                   dC.as<uint32_t>(), dGs.as<uint32_t>(), dX.as<uint32_t>(), dY.as<uint32_t>(), dA1.as<uint32_t>(),
+                   dA2.as<uint32_t>(), dfr.as<uint8_t>(), combG, combg};
+  const uint32_t* di = didx.as<uint32_t>();
+  modp::PolyBoxesArgs PA{dco.as<uint32_t>(), dord.as<uint32_t>(), di, di + N, di + 2 * N, di + 3 * N, dp.as<uint32_t>(),
+                         (uint32_t)N};
+  MPVSS_TRY(deal_kernels(ctx, B, Tt, nb, N, [&] { return modp::launch_poly_boxes(PA, ctx->stream); }));
+  MPVSS_TRY(timing_end(ctx));
+  PinBuf& host = ctx->pin(0);
+  MPVSS_CUDA(ctx, host.ensure(N * GEOM.row()));
+  uint8_t* rows = host.as<uint8_t>();
+  MPVSS_TRY(d2h(ctx, rows, dfr, N * GEOM.row()));
+  MPVSS_TRY(sync(ctx));
+  // transcript per box (participant.rs:238-252), its challenge repeated for every instance of the box
+  std::vector<uint8_t> cexp(N * EB);
+  for (size_t b = 0; b < nb; ++b) {
+    sha2::Sha256 h;
+    transcript::hash_ordered(h, rows, noff[b], noff[b + 1], GEOM);
+    uint8_t digest[32];
+    h.finalize(digest);
+    challenge_from_digest(ctx, digest, challenges_out + b * EB);
+    for (size_t i = noff[b]; i < noff[b + 1]; ++i) memcpy(cexp.data() + i * EB, challenges_out + b * EB, EB);
+  }
+  // responses r_i = (w_i - p_i * c_b) mod (q-1) on the device (participant.rs:255-264, modp.rs:180-192)
+  MPVSS_TRY(h2d(ctx, dc, cexp.data(), N * EB));
+  modp::RespArgs RA{dord.as<uint32_t>(), dp.as<uint32_t>(), dw.as<uint32_t>(), dc.as<uint32_t>(), dR.as<uint32_t>(),
+                    (uint32_t)N, EW, EW};
+  MPVSS_CUDA(ctx, modp::launch_resp(RA, ctx->stream));
+  ctx->last_launches += 1;
+  std::vector<uint8_t> gs(nb * EB);
+  MPVSS_TRY(d2h(ctx, shares_out, dY, N * EB));
+  MPVSS_TRY(d2h(ctx, responses_out, dR, N * EB));
+  if (x_out) MPVSS_TRY(d2h(ctx, x_out, dX, N * EB));
+  MPVSS_TRY(d2h(ctx, commitments_out, dC, Tt * EB));
+  MPVSS_TRY(d2h(ctx, gs.data(), dGs, nb * EB));
+  MPVSS_TRY(sync(ctx));
+  for (size_t b = 0; b < nb; ++b) {
+    mask_secret(ctx, secrets + b * EB, EB, gs.data() + b * EB, u_out + b * EB);
+    status_out[b] = MPVSS_OK;
+  }
   // the scratch buffers held secrets (coefficients, P(i), witnesses)
   for (DevBuf* b : {&dco, &dp, &dw, &ds}) MPVSS_CUDA(ctx, cudaMemsetAsync(b->p, 0, b->cap, ctx->stream));
   return sync(ctx);
@@ -1431,6 +1540,7 @@ const GroupOps modp_ops = [] {
   o.verify_batch = modp_api::verify_batch;
   o.scalar_poly_eval = modp_api::scalar_poly_eval;
   o.distribute = modp_api::distribute;
+  o.distribute_batch = modp_api::distribute_batch;
   o.extract_shares = modp_api::extract_shares;
   o.verify_shares = modp_api::verify_shares;
   o.reconstruct = modp_api::reconstruct;

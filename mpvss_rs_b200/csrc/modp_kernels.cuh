@@ -462,6 +462,27 @@ MP_DEV void poly_body(const PolyArgs& A, uint32_t tid) {
   for (int i = 0; i < 64; ++i) A.out[(size_t)tid * 64 + i] = br ? acc[i] : r[i];
 }
 
+// Several boxes at once (mpvss_distribute_secrets): the coefficients and the instances of the boxes are
+// concatenated, and instance i evaluates the polynomial of its own box: t_b = bt[i] coefficients from row coff[i],
+// the box's instances starting at row ioff[i].
+struct PolyBoxesArgs {
+  const uint32_t* coeffs;  // sum t_b x 64 limbs, concatenated over the boxes
+  const uint32_t* order;   // 64 limbs
+  const uint32_t* pos;     // n positions (< 2^31), concatenated over the boxes
+  const uint32_t* coff;    // per instance: first coefficient row of its box
+  const uint32_t* bt;      // per instance: coefficients t_b of its box
+  const uint32_t* ioff;    // per instance: first instance row of its box
+  uint32_t* out;           // n x 64 limbs
+  uint32_t n;
+};
+MP_DEV void poly_boxes_body(const PolyBoxesArgs& A, uint32_t tid) {
+  if (tid >= A.n) return;
+  const uint32_t off = A.ioff[tid];
+  poly_body(PolyArgs{A.coeffs + (size_t)A.coff[tid] * 64, A.order, A.pos + off, A.out + (size_t)off * 64, A.bt[tid],
+                     A.n - off},
+            tid - off);
+}
+
 // ------------------------------------------------- DLEQ responses (scalars) ----
 // r_i = (w_i - (alpha_i * c mod order)) mod order  (dleq.rs:42-50 through modp.rs:180-192; call sites
 // participant.rs:255-264, 342-347): alpha_i < order, the challenge c < 2^256, w_i < 2^2048.  One instance

@@ -51,6 +51,8 @@ SIGNATURES = {
                                                   _u8p, _u8p, _u8p, _u8p, _intp, _u8p]),
     "mpvss_distribute": (ctypes.c_int, [_ctxp, _sz, _sz, _u8p, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p,
                                         _u8p, _u8p]),
+    "mpvss_distribute_secrets": (ctypes.c_int, [_ctxp, _sz, ctypes.POINTER(_sz), ctypes.POINTER(_sz), _u8p, _u8p, _u8p,
+                                                _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _intp]),
     "mpvss_extract_shares": (ctypes.c_int, [_ctxp, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, _intp]),
     "mpvss_verify_shares": (ctypes.c_int, [_ctxp, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _intp]),
     "mpvss_reconstruct": (ctypes.c_int, [_ctxp, _sz, _i64p, _u8p, _u8p, _u8p, _u8p]),

@@ -6,8 +6,8 @@ tests read like the reference's own tests; every group operation goes through
 libmpvss_b200.so (CUDA).  The only additions are the randomness-injection
 arguments (`coeffs`, `witnesses`, `private_key`) -- the reference draws those from
 `thread_rng` internally (polynomial.rs:34-47, participant.rs:223, 139-146) -- and
-the batch forms `extract_secret_shares` / `verify_shares` / `verify_distributions` /
-`reconstruct_secrets`.
+the batch forms `distribute_secrets` / `extract_secret_shares` / `verify_shares` /
+`verify_distributions` / `reconstruct_secrets`.
 
 Value representation at this level: MODP elements and all scalars are Python
 ints (the reference uses BigInt); secp256k1 / ristretto255 elements are their
@@ -221,7 +221,8 @@ class Participant:
         self.publickey = self.group.generate_public_key(self.privatekey)
 
     # -- distribute_secret: participant.rs:160-286 / 1094-1274 / 1573-1717 --
-    def distribute_secret(self, secret: int, publickeys, threshold: int, coeffs=None, witnesses=None):
+    def _deal_inputs(self, secret, publickeys, threshold, coeffs, witnesses):
+        """the host checks and the randomness of one dealing: (secret bytes, coefficients, witnesses)"""
         g, c = self.group, self.group.codec
         n = len(publickeys)
         assert threshold <= n                                   # participant.rs:166
@@ -230,15 +231,14 @@ class Participant:
         if witnesses is None:                                   # participant.rs:223
             witnesses = [g.generate_private_key() for _ in range(n)]
         assert len(coeffs) == threshold and len(witnesses) == n
-        sbytes = secret.to_bytes(max(1, (secret.bit_length() + 7) // 8), "big")
-        comm, shares = buf(size=threshold * c.eb), buf(size=n * c.eb)
-        chal, resp, u = buf(size=c.sb), buf(size=n * c.sb), buf(size=c.eb)
-        g.ctx.check(g.ctx.lib.mpvss_distribute(
-            g.ctx.h, n, threshold, ptr(buf(sbytes)), len(sbytes), ptr(buf(c.enc_scalars(coeffs))),
-            ptr(buf(c.enc_scalars(witnesses))), ptr(buf(c.enc_elems(publickeys))), ptr(comm), ptr(shares),
-            ptr(chal), ptr(resp), ptr(u), None))
+        return secret.to_bytes(max(1, (secret.bit_length() + 7) // 8), "big"), coeffs, witnesses
+
+    def _box(self, publickeys, comm, shares, chal, resp, u):
+        """DistributionSharesBox from one box's output rows"""
+        c = self.group.codec
+        n = len(publickeys)
         box = DistributionSharesBox()
-        box.commitments = c.dec_elems(comm, threshold)
+        box.commitments = c.dec_elems(comm, len(comm) // c.eb)
         ys, rs = c.dec_elems(shares, n), c.dec_scalars(resp, n)
         for i, pk in enumerate(publickeys):
             k = c.key(pk)
@@ -249,6 +249,53 @@ class Participant:
         box.challenge = c.dec_scalar(bytes(chal))
         box.U = int.from_bytes(bytes(u), "big")
         return box
+
+    def distribute_secret(self, secret: int, publickeys, threshold: int, coeffs=None, witnesses=None):
+        g, c = self.group, self.group.codec
+        n = len(publickeys)
+        sbytes, coeffs, witnesses = self._deal_inputs(secret, publickeys, threshold, coeffs, witnesses)
+        comm, shares = buf(size=threshold * c.eb), buf(size=n * c.eb)
+        chal, resp, u = buf(size=c.sb), buf(size=n * c.sb), buf(size=c.eb)
+        g.ctx.check(g.ctx.lib.mpvss_distribute(
+            g.ctx.h, n, threshold, ptr(buf(sbytes)), len(sbytes), ptr(buf(c.enc_scalars(coeffs))),
+            ptr(buf(c.enc_scalars(witnesses))), ptr(buf(c.enc_elems(publickeys))), ptr(comm), ptr(shares),
+            ptr(chal), ptr(resp), ptr(u), None))
+        return self._box(publickeys, bytes(comm), bytes(shares), bytes(chal), bytes(resp), bytes(u))
+
+    def distribute_secrets(self, jobs) -> list:
+        """Batch form of distribute_secret: one DistributionSharesBox per (secret, publickeys, threshold[, coeffs[,
+        witnesses]]) job, all jobs in one library call (mpvss_distribute_secrets).  A job whose box the library
+        rejects (where distribute_secret would raise) is None without disturbing the others."""
+        g, c = self.group, self.group.codec
+        if not jobs:
+            return []
+        deals = []
+        for job in jobs:
+            secret, publickeys, threshold, coeffs, witnesses = (tuple(job) + (None, None))[:5]
+            sbytes, coeffs, witnesses = self._deal_inputs(secret, publickeys, threshold, coeffs, witnesses)
+            if len(sbytes) > c.eb:                              # what mpvss_distribute rejects for this secret
+                raise _lib.MpvssError(_lib.ERR_ARG, "distribute_secrets: a secret is longer than one element")
+            deals.append((sbytes.rjust(c.eb, b"\0"), list(publickeys), threshold, coeffs, witnesses))
+        m = len(deals)
+        ns, ts = [len(d[1]) for d in deals], [d[2] for d in deals]
+        N, T = sum(ns), sum(ts)
+        comm, shares, resp = buf(size=T * c.eb), buf(size=N * c.eb), buf(size=N * c.sb)
+        chal, u, st = buf(size=m * c.sb), buf(size=m * c.eb), (ctypes.c_int * m)()
+        g.ctx.check(g.ctx.lib.mpvss_distribute_secrets(
+            g.ctx.h, m, (ctypes.c_size_t * m)(*ns), (ctypes.c_size_t * m)(*ts), ptr(buf(b"".join(d[0] for d in deals))),
+            ptr(buf(b"".join(c.enc_scalars(d[3]) for d in deals))),
+            ptr(buf(b"".join(c.enc_scalars(d[4]) for d in deals))),
+            ptr(buf(b"".join(c.enc_elems(d[1]) for d in deals))), ptr(comm), ptr(shares), ptr(chal), ptr(resp), ptr(u),
+            None, st))
+        comm, shares, resp, chal, u = bytes(comm), bytes(shares), bytes(resp), bytes(chal), bytes(u)
+        out, n0, t0 = [], 0, 0
+        for b, (_, publickeys, threshold, _, _) in enumerate(deals):
+            n = len(publickeys)
+            out.append(None if st[b] != _lib.OK else self._box(
+                publickeys, comm[t0 * c.eb:(t0 + threshold) * c.eb], shares[n0 * c.eb:(n0 + n) * c.eb],
+                chal[b * c.sb:(b + 1) * c.sb], resp[n0 * c.sb:(n0 + n) * c.sb], u[b * c.eb:(b + 1) * c.eb]))
+            n0, t0 = n0 + n, t0 + threshold
+        return out
 
     # -- verify_distribution_shares: participant.rs:399-455 / 1384-1442 / 1827-1885 --
     def _flatten(self, box):
