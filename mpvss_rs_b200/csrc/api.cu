@@ -324,9 +324,27 @@ int mpvss_verify_shares(mpvss_ctx* ctx, size_t n, const uint8_t* publickeys, con
                         const uint8_t* enc_shares, const uint8_t* challenges, const uint8_t* responses, int* ok_out) {
   DISPATCH(ctx, verify_shares, n, publickeys, shares, enc_shares, challenges, responses, ok_out);
 }
+// A batch of one box.  The batch zeroes a rejected box's rows and records no error; this call leaves its outputs
+// alone and records one, so the box's rows land in local buffers first.
 int mpvss_reconstruct(mpvss_ctx* ctx, size_t k, const int64_t* positions, const uint8_t* shares, const uint8_t* u,
                       uint8_t* secret_out, uint8_t* gs_out) {
-  DISPATCH(ctx, reconstruct, k, positions, shares, u, secret_out, gs_out);
+  if (!ctx) return MPVSS_ERR_ARG;
+  Guard hold(ctx);
+  if (k == 0 || k > 0x7fffffff || !positions || !shares || !u || !secret_out)  // the kernels count shares in 32 bits
+    return mpvss_fail(ctx, MPVSS_ERR_ARG, "reconstruct: bad arguments");
+  uint8_t secret[256], gs[256];  // one element (256 / 33 / 32 bytes)
+  int status = MPVSS_OK;
+  MPVSS_TRY(ctx->ops->reconstruct_batch(ctx, 1, &k, positions, shares, u, secret, gs, &status));
+  if (status == MPVSS_ERR_ARG)  // the curves accept a repeated position (lambda = 0)
+    return mpvss_fail(ctx, status, ctx->group == MPVSS_GROUP_MODP
+                                       ? "reconstruct: position out of range [1, 2^31) or repeated"
+                                       : "reconstruct: position out of range [1, 2^31)");
+  if (status != MPVSS_OK)
+    return mpvss_fail(ctx, status, "reconstruct: a share is not a valid element encoding, or SHA-256(G^s) is not a "
+                                   "canonical scalar");
+  memcpy(secret_out, secret, mpvss_element_bytes(ctx));
+  if (gs_out) memcpy(gs_out, gs, mpvss_element_bytes(ctx));
+  return MPVSS_OK;
 }
 int mpvss_reconstruct_secrets(mpvss_ctx* ctx, size_t n_boxes, const size_t* k, const int64_t* positions,
                               const uint8_t* shares, const uint8_t* u, uint8_t* secrets_out, uint8_t* gs_out,

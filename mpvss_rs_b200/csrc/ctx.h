@@ -182,7 +182,6 @@ struct GroupOps {
                         uint8_t*, uint8_t*, int*);
   int (*verify_shares)(mpvss_ctx*, size_t, const uint8_t*, const uint8_t*, const uint8_t*, const uint8_t*,
                        const uint8_t*, int*);
-  int (*reconstruct)(mpvss_ctx*, size_t, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*, uint8_t*);
   int (*reconstruct_batch)(mpvss_ctx*, size_t, const size_t*, const int64_t*, const uint8_t*, const uint8_t*, uint8_t*,
                            uint8_t*, int*);
 };

@@ -38,7 +38,6 @@ template <class Cv> __global__ void __launch_bounds__(TPB) add_kernel(AddArgs<Cv
 __global__ void __launch_bounds__(TPB) frame_kernel(FrameArgs A) { frame_body(A, TID); }
 __global__ void __launch_bounds__(TPB) poly_kernel(PolyArgs A) { poly_body(A, TID); }
 __global__ void __launch_bounds__(TPB) poly_boxes_kernel(PolyBoxesArgs A) { poly_boxes_body(A, TID); }
-__global__ void __launch_bounds__(TPB) lagrange_kernel(LagrangeArgs A) { lagrange_body(A, TID); }
 __global__ void __launch_bounds__(TPB) lagrange_boxes_kernel(LagrangeBoxesArgs A) { lagrange_boxes_body(A, TID); }
 __global__ void __launch_bounds__(TPB) inv_kernel(InvArgs A) { inv_body(A, TID); }
 __global__ void __launch_bounds__(TPB) proof_kernel(ProofArgs A) { proof_body(A, TID); }
@@ -108,11 +107,6 @@ cudaError_t launch_poly(const PolyArgs& A, cudaStream_t s) {
 cudaError_t launch_poly_boxes(const PolyBoxesArgs& A, cudaStream_t s) {
   if (A.n == 0) return cudaErrorInvalidValue;
   poly_boxes_kernel<<<blocks(A.n), TPB, 0, s>>>(A);
-  return cudaGetLastError();
-}
-cudaError_t launch_lagrange(const LagrangeArgs& A, cudaStream_t s) {
-  if (A.k == 0) return cudaErrorInvalidValue;
-  lagrange_kernel<<<blocks(A.k), TPB, 0, s>>>(A);
   return cudaGetLastError();
 }
 cudaError_t launch_lagrange_boxes(const LagrangeBoxesArgs& A, cudaStream_t s) {

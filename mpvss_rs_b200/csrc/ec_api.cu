@@ -214,24 +214,46 @@ struct Ec {
     timing_launch(ctx);
     return MPVSS_OK;
   }
-  // sum `count` points per group down to one, encode the result(s) into out
-  static int dev_sum_all(mpvss_ctx* ctx, Point* pts, size_t total, DevBuf& tmp, uint8_t* out) {
-    // repeated 64-way partial sums until one point is left
-    Point* cur = pts;
-    MPVSS_CUDA(ctx, tmp.ensure(((total + 63) / 64) * sizeof(Point) * 2));
-    Point* nxt = tmp.as<Point>();
-    Point* alt = nxt + (total + 63) / 64;
-    while (true) {
-      size_t groups = (total + 63) / 64;
-      bool last = groups == 1;
-      ec::SumArgs<Cv> S{K(ctx), cur, last ? nullptr : nxt, last ? out : nullptr, (uint32_t)groups, 64, 64, 1,
-                        (uint32_t)total};
-      MPVSS_CUDA(ctx, ec::launch_sum<Cv>(S, ctx->stream));
+  // The 64-way segmented sums that add box j's cnt[j] points from row start[j] without crossing a box boundary:
+  // every level planned on the host and uploaded to dseg at once, and the point buffers sized, before the caller
+  // opens its timing bracket.  level_end[l] is the number of groups of levels 0..l.
+  static int plan_sums(mpvss_ctx* ctx, const uint32_t* start, const uint32_t* cnt, size_t L, DevBuf& dseg, DevBuf& dj,
+                       DevBuf& dtmp, std::vector<uint32_t>& level_end) {
+    std::vector<uint32_t> seg, s(start, start + L), c(cnt, cnt + L);
+    level_end.clear();
+    for (bool last = false; !last;) {
+      last = *std::max_element(c.begin(), c.end()) <= 64;
+      size_t groups = 0;
+      for (uint32_t x : c) groups += (x + 63) / 64;
+      const size_t lo = seg.size() / 2;
+      seg.resize(2 * (lo + groups));
+      ec::sum_boxes_level(s.data(), c.data(), (uint32_t)L, seg.data() + 2 * lo);
+      level_end.push_back((uint32_t)(lo + groups));
+    }
+    MPVSS_TRY(h2d(ctx, dseg, seg.data(), seg.size() * 4));
+    MPVSS_CUDA(ctx, dj.ensure(((size_t)start[L - 1] + cnt[L - 1]) * sizeof(Point)));
+    MPVSS_CUDA(ctx, dtmp.ensure(2 * (size_t)level_end[0] * sizeof(Point)));  // the first level has the most groups
+    return MPVSS_OK;
+  }
+  // sum_r e[r] * bases[r] per box: one exponentiation launch over rows [0, n) into projective points (per-row
+  // decode status into `status`), then one launch per level of plan_sums' plan; the last level encodes box j's
+  // sum into out + j * EB
+  static int multi_exp_boxes(mpvss_ctx* ctx, const uint8_t* bases, const uint32_t* e, size_t n, uint32_t* status,
+                             uint8_t* out, const std::vector<uint32_t>& level_end, const DevBuf& dj, const DevBuf& dseg,
+                             const DevBuf& dtmp) {
+    MPVSS_TRY(dev_exp2(ctx, bases, EB, e, nullptr, 0, nullptr, 0, n, nullptr, dj.as<Point>(), status));
+    const Point* cur = dj.as<Point>();
+    Point* nxt = dtmp.as<Point>();
+    Point* alt = nxt + level_end[0];
+    for (size_t l = 0; l < level_end.size(); ++l) {
+      const uint32_t lo = l ? level_end[l - 1] : 0;
+      const bool last = l + 1 == level_end.size();
+      ec::SumBoxesArgs<Cv> S{K(ctx), cur, dseg.as<uint32_t>() + 2 * lo, last ? nullptr : nxt, last ? out : nullptr,
+                             level_end[l] - lo};
+      MPVSS_CUDA(ctx, ec::launch_sum_boxes<Cv>(S, ctx->stream));
       timing_launch(ctx);
-      if (last) break;
       cur = nxt;
       std::swap(nxt, alt);
-      total = groups;
     }
     return MPVSS_OK;
   }
@@ -431,30 +453,26 @@ struct Ec {
     ctx->last_launches += l;
     return MPVSS_OK;
   }
-  static int multi_exp_limbs(mpvss_ctx* ctx, const uint8_t* bases, const uint32_t* scalar_limbs_dev,
-                             const uint32_t* scalar_limbs_host, size_t n, uint8_t* out) {
-    DevBuf &db = ctx->buf(0), &de = ctx->buf(1), &dj = ctx->buf(2), &dst = ctx->buf(3), &dout = ctx->buf(4),
-           &tmp = ctx->buf(5);
-    MPVSS_TRY(h2d(ctx, db, bases, n * EB));
-    if (scalar_limbs_host) MPVSS_TRY(h2d(ctx, de, scalar_limbs_host, n * 32));
-    const uint32_t* e = scalar_limbs_host ? de.as<uint32_t>() : scalar_limbs_dev;
-    MPVSS_CUDA(ctx, dj.ensure(n * sizeof(Point)));
-    MPVSS_CUDA(ctx, dst.ensure(n * 4));
-    MPVSS_CUDA(ctx, dout.ensure(EB));
-    timing_begin(ctx);
-    MPVSS_TRY(dev_exp2(ctx, db.as<uint8_t>(), EB, e, nullptr, 0, nullptr, 0, n, nullptr, dj.as<Point>(),
-                       dst.as<uint32_t>()));
-    MPVSS_TRY(dev_sum_all(ctx, dj.as<Point>(), n, tmp, dout.as<uint8_t>()));
-    MPVSS_TRY(timing_end(ctx));
-    MPVSS_TRY(check_status(ctx, dst, n, "multi_exp"));
-    MPVSS_TRY(d2h(ctx, out, dout, EB));
-    return sync(ctx);
-  }
   static int multi_exp(mpvss_ctx* ctx, const uint8_t* bases, const uint8_t* scalars, size_t n, uint8_t* out) {
     MPVSS_TRY(check_args(ctx, bases && scalars && out && n > 0, "multi_exp: bad arguments"));
     std::vector<uint32_t> e;
     MPVSS_TRY(scalars_in(ctx, scalars, n, e));
-    return multi_exp_limbs(ctx, bases, nullptr, e.data(), n, out);
+    DevBuf &db = ctx->buf(0), &de = ctx->buf(1), &dst = ctx->buf(3), &dout = ctx->buf(4);
+    MPVSS_TRY(h2d(ctx, db, bases, n * EB));
+    MPVSS_TRY(h2d(ctx, de, e.data(), n * 32));
+    MPVSS_CUDA(ctx, dst.ensure(n * 4));
+    MPVSS_CUDA(ctx, dout.ensure(EB));
+    const uint32_t start = 0, cnt = (uint32_t)n;
+    DevBuf &dj = ctx->buf(2), &dseg = ctx->buf(5), &dtmp = ctx->buf(6);
+    std::vector<uint32_t> level_end;
+    MPVSS_TRY(plan_sums(ctx, &start, &cnt, 1, dseg, dj, dtmp, level_end));
+    timing_begin(ctx);
+    MPVSS_TRY(multi_exp_boxes(ctx, db.as<uint8_t>(), de.as<uint32_t>(), n, dst.as<uint32_t>(), dout.as<uint8_t>(),
+                              level_end, dj, dseg, dtmp));
+    MPVSS_TRY(timing_end(ctx));
+    MPVSS_TRY(check_status(ctx, dst, n, "multi_exp"));
+    MPVSS_TRY(d2h(ctx, out, dout, EB));
+    return sync(ctx);
   }
 
   // ---- verify_distribution_shares --------------------------------------------------------------
@@ -1081,35 +1099,9 @@ struct Ec {
     return MPVSS_OK;
   }
 
-  static int reconstruct(mpvss_ctx* ctx, size_t k, const int64_t* positions, const uint8_t* shares, const uint8_t* u,
-                         uint8_t* secret_out, uint8_t* gs_out) {
-    MPVSS_TRY(check_args(ctx, k > 0 && positions && shares && u && secret_out, "reconstruct: bad arguments"));
-    std::vector<uint32_t> pos;
-    if (positions_u32(positions, k, pos) != k) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range [1, 2^31)");
-    DevBuf &dpos = ctx->buf(10), &dlam = ctx->buf(11);
-    MPVSS_TRY(h2d(ctx, dpos, pos.data(), k * 4));
-    MPVSS_CUDA(ctx, dlam.ensure(k * 32));
-    ec::LagrangeArgs LA{KN(ctx), dpos.as<uint32_t>(), dlam.as<uint32_t>(), (uint32_t)k};
-    timing_begin(ctx);  // the Lagrange kernel counts towards the kernel time of the call
-    MPVSS_CUDA(ctx, ec::launch_lagrange(LA, ctx->stream));
-    MPVSS_TRY(timing_end(ctx));
-    const float ms_lambda = ctx->last_ms;
-    uint8_t gs[EB];
-    MPVSS_TRY(multi_exp_limbs(ctx, shares, dlam.as<uint32_t>(), nullptr, k, gs));
-    ctx->last_launches += 1;
-    ctx->last_ms += ms_lambda;
-    big::Int mask;
-    if (!T::mask_of(gs, ctx->ec_order, &mask))
-      return mpvss_fail(ctx, MPVSS_ERR_ENCODING, "reconstruct: SHA-256(G^s) is not a canonical scalar");
-    big::to_be(big::bxor(mask, big::from_be(u, EB)), secret_out, EB);
-    if (gs_out) memcpy(gs_out, gs, EB);
-    return MPVSS_OK;
-  }
-
-  // Many reconstruct calls in one (mpvss_reconstruct_secrets): the live boxes' positions and shares are
-  // concatenated; one box-aware Lagrange launch, one dev_exp2 launch over every share into projective points
-  // (its per-share status gives a box's ERR_ENCODING), then segmented 64-way sums that never cross a box
-  // boundary until each box has one point, which the last level encodes.
+  // Many reconstruct calls in one (mpvss_reconstruct_secrets; mpvss_reconstruct is a batch of one box): the live
+  // boxes' positions and shares are concatenated; one box-aware Lagrange launch, then multi_exp_boxes (its
+  // per-share status gives a box's ERR_ENCODING).  A repeated position gets lambda = 0 in its box.
   static int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t* positions,
                                const uint8_t* shares, const uint8_t* u, uint8_t* secrets_out, uint8_t* gs_out,
                                int* status_out) {
@@ -1127,51 +1119,22 @@ struct Ec {
     const LiveBoxes B = pack_live_boxes(nb, kv, positions, shares, EB, live);
     const size_t L = live.size(), n = B.n;
     const std::vector<uint32_t> &start = B.start, &cnt = B.cnt;
-    // every level of the segmented sum, planned here and uploaded at once
-    std::vector<uint32_t> seg, level_end;
-    {
-      std::vector<uint32_t> s(start), c(cnt);
-      for (bool last = false; !last;) {
-        last = *std::max_element(c.begin(), c.end()) <= 64;
-        size_t groups = 0;
-        for (uint32_t x : c) groups += (x + 63) / 64;
-        const size_t lo = seg.size() / 2;
-        seg.resize(2 * (lo + groups));
-        ec::sum_boxes_level(s.data(), c.data(), (uint32_t)L, seg.data() + 2 * lo);
-        level_end.push_back((uint32_t)(lo + groups));
-      }
-    }
     DevBuf &dsh = ctx->buf(0), &didx = ctx->buf(1), &dlam = ctx->buf(2), &dj = ctx->buf(3), &dst = ctx->buf(4),
            &dseg = ctx->buf(5), &dtmp = ctx->buf(6), &dout = ctx->buf(7);
-    MPVSS_TRY(h2d(ctx, dsh, B.shares.data(), n * EB));
+    std::vector<uint32_t> level_end;
+    MPVSS_TRY(plan_sums(ctx, start.data(), cnt.data(), L, dseg, dj, dtmp, level_end));
+    MPVSS_TRY(h2d(ctx, dsh, B.rows(shares), n * EB));
     MPVSS_TRY(h2d(ctx, didx, B.idx.data(), 3 * n * 4));
-    MPVSS_TRY(h2d(ctx, dseg, seg.data(), seg.size() * 4));
-    const size_t g1 = level_end[0];  // the first level has the most groups
     MPVSS_CUDA(ctx, dlam.ensure(n * 32));
-    MPVSS_CUDA(ctx, dj.ensure(n * sizeof(Point)));
     MPVSS_CUDA(ctx, dst.ensure(n * 4));
-    MPVSS_CUDA(ctx, dtmp.ensure(2 * g1 * sizeof(Point)));
     MPVSS_CUDA(ctx, dout.ensure(L * EB));
     const uint32_t* di = didx.as<uint32_t>();
     ec::LagrangeBoxesArgs LA{KN(ctx), di, di + n, di + 2 * n, dlam.as<uint32_t>(), (uint32_t)n};
     timing_begin(ctx);
     MPVSS_CUDA(ctx, ec::launch_lagrange_boxes(LA, ctx->stream));
     timing_launch(ctx);
-    MPVSS_TRY(dev_exp2(ctx, dsh.as<uint8_t>(), EB, dlam.as<uint32_t>(), nullptr, 0, nullptr, 0, n, nullptr,
-                       dj.as<Point>(), dst.as<uint32_t>()));
-    const Point* cur = dj.as<Point>();
-    Point* nxt = dtmp.as<Point>();
-    Point* alt = nxt + g1;
-    for (size_t l = 0; l < level_end.size(); ++l) {
-      const uint32_t lo = l ? level_end[l - 1] : 0;
-      const bool last = l + 1 == level_end.size();
-      ec::SumBoxesArgs<Cv> S{K(ctx), cur, dseg.as<uint32_t>() + 2 * lo, last ? nullptr : nxt,
-                             last ? dout.as<uint8_t>() : nullptr, level_end[l] - lo};
-      MPVSS_CUDA(ctx, ec::launch_sum_boxes<Cv>(S, ctx->stream));
-      timing_launch(ctx);
-      cur = nxt;
-      std::swap(nxt, alt);
-    }
+    MPVSS_TRY(multi_exp_boxes(ctx, dsh.as<uint8_t>(), dlam.as<uint32_t>(), n, dst.as<uint32_t>(), dout.as<uint8_t>(),
+                              level_end, dj, dseg, dtmp));
     MPVSS_TRY(timing_end(ctx));
     std::vector<uint32_t> st(n);
     std::vector<uint8_t> gs(L * EB);
@@ -1216,7 +1179,6 @@ GroupOps ec_ops() {
   o.distribute_batch = E::distribute_batch;
   o.extract_shares = E::extract_shares;
   o.verify_shares = E::verify_shares;
-  o.reconstruct = E::reconstruct;
   o.reconstruct_batch = E::reconstruct_batch;
   return o;
 }

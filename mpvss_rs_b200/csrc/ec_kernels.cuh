@@ -267,7 +267,10 @@ MP_DEV void horner_body(const HornerArgs<Cv>& A, uint32_t tid) {
 // position i belongs to a box whose t_b commitments start at cxy row coff[i].  Instance (k, i) evaluates
 // chunk k = [k B_b, min((k+1) B_b, t_b)), B_b = ceil(t_b / K), of that box's polynomial; a chunk that lies
 // past t_b (boxes with fewer than K coefficients) contributes the identity.  The body repeats horner_body
-// instead of sharing a helper with it so that the single-box kernel's code stays exactly as it is.
+// instead of sharing a helper with it so that the single-box kernel's code stays exactly as it is.  Running the
+// single-box calls through this kernel as one box was measured and not taken: at 128 registers it keeps 264
+// bytes of stack against horner_kernel's 256 (secp256k1), and the secp256k1 X_i phase of the n = 4096 verify
+// took 26.02-26.10 ms against 25.98-26.00 ms (NVIDIA B200, 1000 W, 3 alternating runs each).
 template <class Cv>
 struct HornerBoxesArgs {
   const typename Cv::Consts* C;

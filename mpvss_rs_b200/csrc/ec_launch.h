@@ -24,7 +24,6 @@ template <class Cv> cudaError_t launch_add(const AddArgs<Cv>& A, cudaStream_t s)
 cudaError_t launch_frames(const FrameArgs& A, cudaStream_t s);
 cudaError_t launch_poly(const PolyArgs& A, cudaStream_t s);
 cudaError_t launch_poly_boxes(const PolyBoxesArgs& A, cudaStream_t s);
-cudaError_t launch_lagrange(const LagrangeArgs& A, cudaStream_t s);
 cudaError_t launch_lagrange_boxes(const LagrangeBoxesArgs& A, cudaStream_t s);
 cudaError_t launch_inv(const InvArgs& A, cudaStream_t s);
 cudaError_t launch_proof(const ProofArgs& A, cudaStream_t s);

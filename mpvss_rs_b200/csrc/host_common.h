@@ -56,11 +56,13 @@ inline size_t positions_u32(const int64_t* positions, size_t n, std::vector<uint
 
 // The live boxes of a reconstruct batch packed in the order of `live`: box live[j] takes rows
 // [start[j], start[j] + cnt[j]) of the n rows.  idx holds the positions, then per row its box's first row, then
-// its box's share count (the box-aware Lagrange kernels' layout); shares are the rows' shares, eb bytes each.
+// its box's share count (the box-aware Lagrange kernels' layout).  rows(shares) are the rows' shares, eb bytes
+// each: the caller's array itself when every box is live in its own order (always so for a single box).
 struct LiveBoxes {
   size_t n = 0;
   std::vector<uint32_t> start, cnt, idx;
-  std::vector<uint8_t> shares;
+  std::vector<uint8_t> packed;  // the rows' shares when they are not the caller's array as it stands
+  const uint8_t* rows(const uint8_t* shares) const { return packed.empty() ? shares : packed.data(); }
 };
 inline LiveBoxes pack_live_boxes(size_t nb, const size_t* kv, const int64_t* positions, const uint8_t* shares,
                                  size_t eb, const std::vector<size_t>& live) {
@@ -77,7 +79,9 @@ inline LiveBoxes pack_live_boxes(size_t nb, const size_t* kv, const int64_t* pos
   }
   const size_t n = P.n;
   P.idx.resize(3 * n);
-  P.shares.resize(n * eb);
+  bool in_place = L == nb;
+  for (size_t j = 0; j < L && in_place; ++j) in_place = live[j] == j;
+  if (!in_place) P.packed.resize(n * eb);
   for (size_t j = 0; j < L; ++j) {
     const size_t b = live[j];
     for (uint32_t i = 0; i < P.cnt[j]; ++i) {
@@ -85,7 +89,7 @@ inline LiveBoxes pack_live_boxes(size_t nb, const size_t* kv, const int64_t* pos
       P.idx[n + P.start[j] + i] = P.start[j];
       P.idx[2 * n + P.start[j] + i] = P.cnt[j];
     }
-    memcpy(P.shares.data() + (size_t)P.start[j] * eb, shares + first[b] * eb, P.cnt[j] * eb);
+    if (!in_place) memcpy(P.packed.data() + (size_t)P.start[j] * eb, shares + first[b] * eb, P.cnt[j] * eb);
   }
   return P;
 }

@@ -55,7 +55,6 @@ __global__ void __launch_bounds__(128) frame_kernel(FrameArgs A) { frame_body(A,
 __global__ void __launch_bounds__(64) resp_kernel(RespArgs A) { resp_body(A, blockIdx.x * 64 + threadIdx.x); }
 __global__ void __launch_bounds__(64) poly_kernel(PolyArgs A) { poly_body(A, blockIdx.x * 64 + threadIdx.x); }
 __global__ void __launch_bounds__(64) poly_boxes_kernel(PolyBoxesArgs A) { poly_boxes_body(A, blockIdx.x * 64 + threadIdx.x); }
-__global__ void __launch_bounds__(64) lagrange_kernel(LagrangeArgs A) { lagrange_body(A, blockIdx.x * 64 + threadIdx.x); }
 __global__ void __launch_bounds__(64) lagrange_boxes_kernel(LagrangeBoxesArgs A) {
   lagrange_boxes_body(A, blockIdx.x * 64 + threadIdx.x);
 }
@@ -198,13 +197,6 @@ cudaError_t launch_poly(const PolyArgs& A, cudaStream_t s) {
 cudaError_t launch_poly_boxes(const PolyBoxesArgs& A, cudaStream_t s) {
   if (A.n == 0) return cudaErrorInvalidValue;
   poly_boxes_kernel<<<(A.n + 63) / 64, 64, 0, s>>>(A);
-  return cudaGetLastError();
-}
-
-cudaError_t launch_lagrange(const LagrangeArgs& A, cudaStream_t s) {
-  if (A.k == 0) return cudaErrorInvalidValue;
-  const uint32_t threads = 2u * (A.parts ? A.parts : 1u) * A.k;
-  lagrange_kernel<<<(threads + 63) / 64, 64, 0, s>>>(A);
   return cudaGetLastError();
 }
 

@@ -513,23 +513,6 @@ int dleq_prove_commit(mpvss_ctx* ctx, const uint8_t* g1, const uint8_t* g2, cons
   return sync(ctx);
 }
 
-// in-place pairwise product tree over `n` device elements; the result lands in slot 0
-static int dev_product_tree(mpvss_ctx* ctx, uint32_t* v, DevBuf& tmp, size_t n) {
-  const uint32_t* K = ctx->consts_q.as<uint32_t>();
-  MPVSS_CUDA(ctx, tmp.ensure(((n + 1) / 2) * EB));
-  while (n > 1) {
-    size_t half = n / 2;
-    // tmp[i] = v[i] * v[i + half]
-    MPVSS_TRY(dev_mul(ctx, K, v, EW, v + half * EW, EW, 0, half, tmp.as<uint32_t>()));
-    if (n & 1)
-      MPVSS_CUDA(ctx, cudaMemcpyAsync(tmp.as<uint32_t>() + half * EW, v + 2 * half * EW, EB, cudaMemcpyDeviceToDevice,
-                                      ctx->stream));
-    n = half + (n & 1);
-    MPVSS_CUDA(ctx, cudaMemcpyAsync(v, tmp.p, n * EB, cudaMemcpyDeviceToDevice, ctx->stream));
-  }
-  return MPVSS_OK;
-}
-
 // Bucket method (Pippenger, 8-bit windows) for prod_i bases[i]^scalars[i], all on the device: counting sort of
 // every window's exponent bytes, bucket products, per-window products, final fold (modp::launch_msm).
 // `db` holds the bases in normal form, `de` the exponents; the result lands in dout[0].
@@ -550,9 +533,41 @@ static int multi_exp_buckets(mpvss_ctx* ctx, DevBuf& db, DevBuf& de, uint32_t wi
   return MPVSS_OK;
 }
 
+// The segmented product tree that folds box j's cnt[j] rows from start[j] into row start[j]: every level planned
+// on the host and uploaded to dplan at once, before the caller opens its timing bracket.  level_end[l] is the
+// number of (a, b, out) triples of levels 0..l.
+static int plan_product_tree(mpvss_ctx* ctx, const uint32_t* start, const uint32_t* cnt, size_t L, DevBuf& dplan,
+                             std::vector<uint32_t>& level_end) {
+  std::vector<uint32_t> rows(3 * ((size_t)start[L - 1] + cnt[L - 1])), c(cnt, cnt + L);
+  level_end.clear();
+  for (size_t m = 0, total = 0;
+       (m = modp::product_tree_level(start, c.data(), (uint32_t)L, rows.data() + 3 * total)) > 0;) {
+    total += m;
+    level_end.push_back((uint32_t)total);
+  }
+  if (!level_end.empty()) MPVSS_TRY(h2d(ctx, dplan, rows.data(), (size_t)level_end.back() * 3 * 4));
+  return MPVSS_OK;
+}
+
+// prod_r db[r]^de[r] per box: one exponentiation launch over rows [0, n) into dpow, then one gather-multiply launch
+// per level of the tree plan_product_tree uploaded to dplan.  `windows` as dev_exp2 takes it.
+static int multi_exp_direct(mpvss_ctx* ctx, const DevBuf& db, const DevBuf& de, uint32_t windows, size_t n,
+                            const std::vector<uint32_t>& level_end, DevBuf& dpow, const DevBuf& dplan) {
+  const uint32_t* K = ctx->consts_q.as<uint32_t>();
+  MPVSS_TRY(dev_exp2(ctx, K, db.as<uint32_t>(), EW, de.as<uint32_t>(), EW, windows, nullptr, 0, nullptr, 0, 0, n,
+                     dpow.as<uint32_t>()));
+  for (size_t l = 0; l < level_end.size(); ++l) {
+    const uint32_t lo = l ? level_end[l - 1] : 0;
+    modp::MulRowsArgs MA{K, dpow.as<uint32_t>(), dplan.as<uint32_t>() + 3 * lo, level_end[l] - lo};
+    MPVSS_CUDA(ctx, modp::launch_mul_rows(ctx->modp_tpi, MA, ctx->stream));
+    timing_launch(ctx);
+  }
+  return MPVSS_OK;
+}
+
 int multi_exp(mpvss_ctx* ctx, const uint8_t* bases, const uint8_t* scalars, size_t n, uint8_t* out) {
   MPVSS_TRY(check_args(ctx, bases && scalars && out && n > 0, "multi_exp: bad arguments"));
-  DevBuf &db = ctx->buf(0), &de = ctx->buf(1), &dout = ctx->buf(2), &tmp = ctx->buf(3);
+  DevBuf &db = ctx->buf(0), &de = ctx->buf(1), &dout = ctx->buf(2);
   MPVSS_TRY(h2d(ctx, db, bases, n * EB));
   MPVSS_CUDA(ctx, dout.ensure(n * EB));
   // One exponentiation per base + product tree is ~2560 products deep whatever n is; the bucket method does
@@ -561,14 +576,15 @@ int multi_exp(mpvss_ctx* ctx, const uint8_t* bases, const uint8_t* scalars, size
   // runs in several waves ("modp_msm": 0 never, 1 always, 2 = from msm_threshold bases on).
   const bool buckets = ctx->modp_msm == 1 || (ctx->modp_msm == 2 && n >= (size_t)ctx->msm_threshold);
   MPVSS_TRY(h2d(ctx, de, scalars, n * EB));
+  const uint32_t start = 0, cnt = (uint32_t)n;
+  DevBuf& dplan = ctx->buf(4);
+  std::vector<uint32_t> level_end;
+  if (!buckets) MPVSS_TRY(plan_product_tree(ctx, &start, &cnt, 1, dplan, level_end));
   timing_begin(ctx);
-  if (buckets) {
+  if (buckets)
     MPVSS_TRY(multi_exp_buckets(ctx, db, de, (windows_for(scalars, EB, n) + 1) / 2, n, dout));
-  } else {
-    MPVSS_TRY(dev_exp2(ctx, ctx->consts_q.as<uint32_t>(), db.as<uint32_t>(), EW, de.as<uint32_t>(), EW,
-                       windows_for(scalars, EB, n), nullptr, 0, nullptr, 0, 0, n, dout.as<uint32_t>()));
-    MPVSS_TRY(dev_product_tree(ctx, dout.as<uint32_t>(), tmp, n));
-  }
+  else
+    MPVSS_TRY(multi_exp_direct(ctx, db, de, windows_for(scalars, EB, n), n, level_end, dout, dplan));
   MPVSS_TRY(timing_end(ctx));
   MPVSS_TRY(d2h(ctx, out, dout, EB));
   return sync(ctx);
@@ -1376,61 +1392,19 @@ static int lagrange_lambdas(mpvss_ctx* ctx, DevBuf& dnum, DevBuf& dden, DevBuf& 
   return MPVSS_OK;
 }
 
-int reconstruct(mpvss_ctx* ctx, size_t k, const int64_t* positions, const uint8_t* shares, const uint8_t* u,
-                uint8_t* secret_out, uint8_t* gs_out) {
-  MPVSS_TRY(check_args(ctx, k > 0 && positions && shares && u && secret_out, "reconstruct: bad arguments"));
-  std::vector<uint32_t> pos;
-  if (positions_u32(positions, k, pos) != k) return mpvss_fail(ctx, MPVSS_ERR_ARG, "position out of range");
-  // lambda_i = prod_{j != i} j / (j - i) mod g with the sign folded into the exponent:
-  // S^(-lambda) = S^((q-1) - lambda)  (participant.rs:535-558, element_inverse modp.rs:138-140).
-  // Numerators / denominators mod q-1 on the device (one position per thread), then
-  // den^-1 mod g and lambda = num * den^-1 mod g with the kernels of modulus g (lagrange_lambdas).
-  {
-    std::vector<uint32_t> sorted(pos);
-    std::sort(sorted.begin(), sorted.end());
-    if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
-      return mpvss_fail(ctx, MPVSS_ERR_ARG, "duplicate position");
-  }
-  const std::vector<uint32_t> order = order_limbs(ctx);
-  std::vector<uint8_t> lam;
-  DevBuf &dpos = ctx->buf(12), &dord = ctx->buf(13), &dnum = ctx->buf(14), &dden = ctx->buf(15), &dneg = ctx->buf(16),
-         &dinv = ctx->buf(18), &dlam = ctx->buf(19);
-  MPVSS_TRY(h2d(ctx, dpos, pos.data(), k * 4));
-  MPVSS_TRY(h2d(ctx, dord, order.data(), EB));
-  // the k-term products are cut into `parts` ranges (more, shorter threads), multiplied together mod g afterwards
-  const size_t parts = k >= 64 ? 8 : 1;
-  for (DevBuf* b : {&dnum, &dden}) MPVSS_CUDA(ctx, b->ensure(parts * k * EB));
-  for (DevBuf* b : {&dinv, &dlam}) MPVSS_CUDA(ctx, b->ensure(k * EB));
-  MPVSS_CUDA(ctx, dneg.ensure(parts * k * 4));
-  modp::LagrangeArgs LA{dord.as<uint32_t>(), dpos.as<uint32_t>(), dnum.as<uint32_t>(), dden.as<uint32_t>(),
-                        dneg.as<uint32_t>(), (uint32_t)k, (uint32_t)parts};
-  timing_begin(ctx);  // the Lagrange part counts towards the kernel time of the call
-  MPVSS_CUDA(ctx, modp::launch_lagrange(LA, ctx->stream));
-  timing_launch(ctx);
-  MPVSS_TRY(lagrange_lambdas(ctx, dnum, dden, dneg, dinv, dlam, k, parts, lam));
-  const float ms_lambda = ctx->last_ms;
-  const int launches_lambda = ctx->last_launches;
-  uint8_t gs[EB];
-  MPVSS_TRY(multi_exp(ctx, shares, lam.data(), k, gs));
-  ctx->last_ms += ms_lambda;
-  ctx->last_launches += launches_lambda;
-  big::to_be(big::bxor(u_mask(ctx, gs), big::from_be(u, EB)), secret_out, EB);
-  if (gs_out) memcpy(gs_out, gs, EB);
-  return MPVSS_OK;
-}
-
-// Many reconstruct calls in one (mpvss_reconstruct_secrets).  The live boxes' positions and shares are
-// concatenated, the boxes that take the direct method first.  One box-aware Lagrange launch, the part products,
-// ONE batch inversion mod g over every box's denominators, and the signs folded on the host as reconstruct
-// does; then one dev_exp2 launch over every direct box's shares, reduced by a segmented product tree (one
-// gather-multiply launch per level), and the bucket method box after box for the others.
+// Many reconstruct calls in one (mpvss_reconstruct_secrets; mpvss_reconstruct is a batch of one box).  The live
+// boxes' positions and shares are concatenated, the boxes that take the direct method first.  One box-aware
+// Lagrange launch, the part products, ONE batch inversion mod g over every box's denominators, and the signs
+// folded on the host: lambda_i = prod_{j != i} j / (j - i) mod g, S^(-lambda) = S^((q-1) - lambda)
+// (participant.rs:535-558, element_inverse modp.rs:138-140).  Then multi_exp_direct over every direct box's
+// shares, and the bucket method box after box for the others.
 int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t* positions, const uint8_t* shares,
                       const uint8_t* u, uint8_t* secrets_out, uint8_t* gs_out, int* status_out) {
   memset(secrets_out, 0, nb * EB);
   if (gs_out) memset(gs_out, 0, nb * EB);
   ctx->last_ms = 0.f;
   ctx->last_launches = 0;
-  std::vector<size_t> live;  // boxes that pass reconstruct's checks
+  std::vector<size_t> live;  // boxes whose positions are in range and distinct
   std::vector<uint32_t> sorted;
   for (size_t b = 0, off = 0; b < nb; off += kv[b], ++b) {
     bool ok = positions_u32(positions + off, kv[b], sorted) == kv[b];
@@ -1442,17 +1416,17 @@ int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t
     if (ok) live.push_back(b);
   }
   if (live.empty()) return MPVSS_OK;
-  // a lone box chooses as reconstruct does; in a batch a box joins the direct launch below msm_batch_threshold
+  // a lone box chooses as multi_exp does; in a batch a box joins the direct launch below msm_batch_threshold
   const size_t threshold = live.size() == 1 ? (size_t)ctx->msm_threshold : mpvss_ctx::msm_batch_threshold;
   auto buckets = [&](size_t b) { return ctx->modp_msm == 1 || (ctx->modp_msm == 2 && kv[b] >= threshold); };
   std::stable_partition(live.begin(), live.end(), [&](size_t b) { return !buckets(b); });
   LiveBoxes B = pack_live_boxes(nb, kv, positions, shares, EB, live);
   const size_t L = live.size(), n = B.n;
   const std::vector<uint32_t> &start = B.start, &cnt = B.cnt;
-  size_t n_direct = 0, L_direct = 0, kmax = 0;  // rows / boxes of the direct launch
+  size_t L_direct = 0, kmax = 0;  // boxes of the direct launch
   for (size_t j = 0; j < L; ++j) {
     kmax = std::max<size_t>(kmax, cnt[j]);
-    if (!buckets(live[j])) n_direct = start[j] + cnt[j], L_direct = j + 1;
+    if (!buckets(live[j])) L_direct = j + 1;
   }
   // multi_exp_buckets holds buf(15..19) and dev_batch_inverse_g buf(21..23)
   DevBuf &dshares = ctx->buf(0), &dexp = ctx->buf(1), &dpow = ctx->buf(2), &dplan = ctx->buf(4), &didx = ctx->buf(10),
@@ -1460,13 +1434,13 @@ int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t
   const std::vector<uint32_t> order = order_limbs(ctx);
   MPVSS_TRY(h2d(ctx, didx, B.idx.data(), 3 * n * 4));
   MPVSS_TRY(h2d(ctx, dord, order.data(), EB));
-  MPVSS_TRY(h2d(ctx, dshares, B.shares.data(), n * EB));
-  const size_t parts = kmax >= 64 ? 8 : 1;  // as reconstruct cuts a box of kmax positions
+  MPVSS_TRY(h2d(ctx, dshares, B.rows(shares), n * EB));
+  // the k-term products are cut into `parts` ranges (more, shorter threads), multiplied together mod g afterwards
+  const size_t parts = kmax >= 64 ? 8 : 1;
   for (DevBuf* b : {&dnum, &dden}) MPVSS_CUDA(ctx, b->ensure(parts * n * EB));
   MPVSS_CUDA(ctx, dinv.ensure(n * EB));
   MPVSS_CUDA(ctx, dneg.ensure(parts * n * 4));
   MPVSS_CUDA(ctx, dpow.ensure(n * EB));
-  const uint32_t* K = ctx->consts_q.as<uint32_t>();
   const uint32_t* di = didx.as<uint32_t>();
   modp::LagrangeBoxesArgs LA{dord.as<uint32_t>(), di, di + n, di + 2 * n, dnum.as<uint32_t>(), dden.as<uint32_t>(),
                              dneg.as<uint32_t>(), (uint32_t)n, (uint32_t)parts};
@@ -1478,28 +1452,13 @@ int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t
   const float ms_lambda = ctx->last_ms;
   const int launches_lambda = ctx->last_launches;
   MPVSS_TRY(h2d(ctx, dexp, lam.data(), n * EB));
-  // the direct boxes' product trees, every level planned here and uploaded at once
-  std::vector<uint32_t> rows(3 * n_direct), level_end;
-  {
-    std::vector<uint32_t> c(cnt.begin(), cnt.begin() + L_direct);
-    for (size_t m = 0, total = 0; (m = modp::product_tree_level(start.data(), c.data(), (uint32_t)L_direct,
-                                                                rows.data() + 3 * total)) > 0;) {
-      total += m;
-      level_end.push_back((uint32_t)total);
-    }
-  }
-  if (!level_end.empty()) MPVSS_TRY(h2d(ctx, dplan, rows.data(), (size_t)level_end.back() * 3 * 4));
+  const size_t n_direct = L_direct ? (size_t)start[L_direct - 1] + cnt[L_direct - 1] : 0;  // rows of the direct boxes
+  std::vector<uint32_t> level_end;
+  if (L_direct) MPVSS_TRY(plan_product_tree(ctx, start.data(), cnt.data(), L_direct, dplan, level_end));
   timing_begin(ctx);
-  if (n_direct) {
-    MPVSS_TRY(dev_exp2(ctx, K, dshares.as<uint32_t>(), EW, dexp.as<uint32_t>(), EW, windows_for(lam.data(), EB, n_direct),
-                       nullptr, 0, nullptr, 0, 0, n_direct, dpow.as<uint32_t>()));
-    for (size_t l = 0; l < level_end.size(); ++l) {
-      const uint32_t lo = l ? level_end[l - 1] : 0;
-      modp::MulRowsArgs MA{K, dpow.as<uint32_t>(), dplan.as<uint32_t>() + 3 * lo, level_end[l] - lo};
-      MPVSS_CUDA(ctx, modp::launch_mul_rows(ctx->modp_tpi, MA, ctx->stream));
-      timing_launch(ctx);
-    }
-  }
+  if (L_direct)
+    MPVSS_TRY(multi_exp_direct(ctx, dshares, dexp, windows_for(lam.data(), EB, n_direct), n_direct, level_end, dpow,
+                               dplan));
   for (size_t j = L_direct; j < L; ++j) {
     DevBuf vb, ve, vo;  // views of box j's rows (not owned)
     vb.p = dshares.as<uint32_t>() + (size_t)start[j] * EW;
@@ -1511,8 +1470,9 @@ int reconstruct_batch(mpvss_ctx* ctx, size_t nb, const size_t* kv, const int64_t
   MPVSS_TRY(timing_end(ctx));
   ctx->last_ms += ms_lambda;
   ctx->last_launches += launches_lambda;
-  std::vector<uint8_t>& host = B.shares;  // uploaded already: takes the results
-  MPVSS_TRY(d2h(ctx, host.data(), dpow, n * EB));
+  // each box's result is its first row; the rows up to the last box's hold them all (one row for one box)
+  std::vector<uint8_t> host(((size_t)start[L - 1] + 1) * EB);
+  MPVSS_TRY(d2h(ctx, host.data(), dpow, host.size()));
   MPVSS_TRY(sync(ctx));
   for (size_t j = 0; j < L; ++j) {
     const size_t b = live[j];
@@ -1543,7 +1503,6 @@ const GroupOps modp_ops = [] {
   o.distribute_batch = modp_api::distribute_batch;
   o.extract_shares = modp_api::extract_shares;
   o.verify_shares = modp_api::verify_shares;
-  o.reconstruct = modp_api::reconstruct;
   o.reconstruct_batch = modp_api::reconstruct_batch;
   return o;
 }();

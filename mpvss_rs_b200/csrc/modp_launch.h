@@ -17,7 +17,6 @@ cudaError_t launch_resp(const RespArgs& A, cudaStream_t s);
 cudaError_t launch_comb_build(int tpi, const CombArgs& A, cudaStream_t s);
 cudaError_t launch_poly(const PolyArgs& A, cudaStream_t s);
 cudaError_t launch_poly_boxes(const PolyBoxesArgs& A, cudaStream_t s);
-cudaError_t launch_lagrange(const LagrangeArgs& A, cudaStream_t s);
 cudaError_t launch_lagrange_boxes(const LagrangeBoxesArgs& A, cudaStream_t s);
 cudaError_t launch_mul(int tpi, const MulArgs& A, cudaStream_t s);
 cudaError_t launch_mul_rows(int tpi, const MulRowsArgs& A, cudaStream_t s);
